@@ -32,6 +32,7 @@ import numpy as np
 
 REPO = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, REPO)
+sys.dont_write_bytecode = True   # the benchmark leaves the tree it runs from as it found it (no __pycache__)
 
 FLOP_PER_STEP = {"open": 750.0, "lqr": 815.0}   # algorithmic FP64 flop per hifi aircraft-step (SURVEY.md 8d)
 BYTES_PER_AIRCRAFT_LAUNCH = 320.0               # read 18 + 4, write 18 doubles, independent of K
@@ -63,6 +64,22 @@ def perturbed_trim(n, x_trim, u_trim, seed, frac=0.05):
     x[0:2] = 0.0
     u = u_trim[:, None] * (1 + frac * ru)
     return np.ascontiguousarray(x), np.ascontiguousarray(u)
+
+
+DUMP_AIRCRAFT = 1 << 17   # aircraft kept by --dump-outputs over all ranks: 19 doubles each, 20 MB in all
+
+
+def dump_outputs(out_dir, x, status, rank=0, world=1):
+    """--dump-outputs: what the last timed step returned, the state [18][n] as DIR/x.npy and the status words [n] as
+    DIR/status.npy (float64, exact for the int32 bit masks); under several ranks every rank writes its own batch as
+    DIR/x.rank<k>.npy and DIR/status.rank<k>.npy.  A batch above its share of DUMP_AIRCRAFT keeps a fixed seeded sample of
+    aircraft in ascending order, the same columns in every run, so that two builds compare entry for entry."""
+    n, keep = x.shape[1], DUMP_AIRCRAFT // world
+    idx = np.arange(n) if n <= keep else np.sort(np.random.default_rng(0xD0).choice(n, keep, replace=False))
+    sfx = f".rank{rank}" if world > 1 else ""
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, f"x{sfx}.npy"), np.ascontiguousarray(x[:, idx], dtype=np.float64))
+    np.save(os.path.join(out_dir, f"status{sfx}.npy"), status[idx].astype(np.float64))
 
 
 class ClockSampler:
@@ -141,10 +158,10 @@ def cpu_reference_rate(aircraft, euler_steps, seed, repeats=1, lqr=None):
     best = None
     for _ in range(repeats):
         t0 = time.perf_counter()
-        _, st = o.step_batch(x, u, euler_steps, 0.001, 1, 0.25, lqr, be)
+        xf, st = o.step_batch(x, u, euler_steps, 0.001, 1, 0.25, lqr, be)
         dt = time.perf_counter() - t0
         best = dt if best is None else min(best, dt)
-    return aircraft * euler_steps / best, kind, o.max_threads(), float((st == 0).mean()), best
+    return aircraft * euler_steps / best, kind, o.max_threads(), float((st == 0).mean()), best, xf, st
 
 
 def run_reference(args):
@@ -156,8 +173,10 @@ def run_reference(args):
         cpu_reference_rate(aircraft, esteps, seed=1)
     t_total, kind, cores, alive = 0.0, "port", 1, 1.0
     for s in range(args.steps):
-        rate, kind, cores, alive, dt = cpu_reference_rate(aircraft, esteps, seed=0xF16 + s)
+        rate, kind, cores, alive, dt, xf, st = cpu_reference_rate(aircraft, esteps, seed=0xF16 + s)
         t_total += dt
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, xf, st)
     value = aircraft * esteps * args.steps / t_total
     sample = f"{aircraft} aircraft x {esteps} Euler steps per bench step (of 2^20 x 10000), hifi xcg 0.25"
     line = {
@@ -314,6 +333,8 @@ def run_ours(args):
     alive = float((st == 0).mean())
     xf = np.empty_like(x)
     ck(L.f16_memcpy_d2h(xf.ctypes.data, d_x, x.nbytes), "d2h")
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, xf, st, rank, world)
 
     # kernel-only duration of one launch (CUDA events on the launching stream), for the roofline
     reset_state()
@@ -400,7 +421,7 @@ def run_ours(args):
 
     cpu = None
     if rank == 0 and world == 1 and not args.no_cpu_baseline:
-        rate, kind, cores, cpu_alive, _ = cpu_reference_rate(args.ref_aircraft, args.ref_euler_steps, seed=0xF16)
+        rate, kind, cores, cpu_alive, _, _, _ = cpu_reference_rate(args.ref_aircraft, args.ref_euler_steps, seed=0xF16)
         cpu = {"value": rate, "unit": "aircraft-steps/s", "cores": cores, "kind": kind,
                "sample": f"{args.ref_aircraft} aircraft x {args.ref_euler_steps} Euler steps of the same workload",
                "alive_fraction": cpu_alive}
@@ -503,7 +524,13 @@ def main():
                          "aircraft, 2 strict CTA per 32 aircraft")
     ap.add_argument("--ref-aircraft", type=int, default=4096, help="aircraft in the CPU sample")
     ap.add_argument("--ref-euler-steps", type=int, default=200, help="Euler steps in the CPU sample")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the last step's final state and status words as DIR/x.npy and DIR/status.npy "
+                         f"(x.rank<k>.npy, status.rank<k>.npy per rank; a fixed sample of {DUMP_AIRCRAFT} aircraft over all ranks "
+                         "of a larger batch); bench_outputs/ in the repository is ignored by git")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
     return run_reference(args) if args.impl == "reference" else run_ours(args)
 
 
