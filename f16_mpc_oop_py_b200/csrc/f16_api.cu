@@ -7,6 +7,7 @@
 #include <string.h>
 
 #include <atomic>
+#include <cmath>
 #include <memory>
 #include <mutex>
 #include <thread>
@@ -1486,7 +1487,10 @@ int discretise_batch_dev(const double* A, const double* B, int n, int m, long lo
   std::lock_guard<std::mutex> lk(G_mu);
   int rc = ensure();
   if (rc != F16_OK) return rc;
-  if (N < 0 || !dims_ok(n, m) || (N > 0 && (!A || !B || !Ad || !Bd))) { set_err("discretise_batch_dev: bad argument"); return F16_ERR_ARG; }
+  if (N < 0 || !dims_ok(n, m) || !std::isfinite(dt) || (N > 0 && (!A || !B || !Ad || !Bd))) {
+    set_err("discretise_batch_dev: bad argument");
+    return F16_ERR_ARG;
+  }
   CK(f16::linalg::launch_zoh(cfg(false), A, B, n, m, N, dt, Ad, Bd));
   return F16_OK;
 }
@@ -1523,7 +1527,10 @@ int discretise_batch(const double* A, const double* B, int n, int m, long long N
   std::lock_guard<std::mutex> lk(G_mu);
   int rc = ensure();
   if (rc != F16_OK) return rc;
-  if (N < 0 || !dims_ok(n, m) || (N > 0 && (!A || !B || !Ad || !Bd))) { set_err("discretise_batch: bad argument"); return F16_ERR_ARG; }
+  if (N < 0 || !dims_ok(n, m) || !std::isfinite(dt) || (N > 0 && (!A || !B || !Ad || !Bd))) {
+    set_err("discretise_batch: bad argument");
+    return F16_ERR_ARG;
+  }
   if (N == 0) return F16_OK;
   const size_t na = (size_t)N * n * n * 8, nb = (size_t)N * n * m * 8;
   CK(D->b_l1.reserve(na));

@@ -7,233 +7,43 @@
 //   zoh               env.py:46,50  scipy.signal.cont2discrete(method='zoh'): expm([[A, B], [0, 0]] dt) -> Ad, Bd,
 //                     by scaling and squaring with a degree-14 Taylor polynomial (||M|| <= 1/2 after scaling).
 //   dlqr              utils.py:219-245  K = (B'PB + R)^-1 B'PA with P from the discrete algebraic Riccati equation,
-//                     solved by the structured doubling algorithm (quadratically convergent; ~21 doublings at dt = 1 ms).
+//                     solved by the structured doubling algorithm (quadratically convergent; ~21 doublings at dt = 1 ms);
+//                     a solution that does not stabilise A - BK is flagged (info -5), as are non-finite iterates (-3).
 //
 // These are tolerance-parity kernels (scipy uses Pade / QZ for the same quantities); FP64 throughout, no tensor cores:
 // the matrices are 9x9 .. 22x22 and there are a few thousand of them.
 #include <math.h>
 
 #include "f16_kernels.cuh"
+#include "f16_linalg.cuh"
 
 namespace f16 {
 namespace linalg {
 
-constexpr int MAXD = 22;  // 18 states + 4 inputs
-
-__device__ __forceinline__ void matmul(const double* X, const double* Y, double* Z, int n) {  // Z = X Y, n x n, ld MAXD
-  for (int i = 0; i < n; i++)
-    for (int j = 0; j < n; j++) {
-      double a = 0;
-      for (int k = 0; k < n; k++) a = fma(X[i * MAXD + k], Y[k * MAXD + j], a);
-      Z[i * MAXD + j] = a;
-    }
-}
-
-// exp(M) for an n x n matrix (ld MAXD), in place; T1, T2 scratch
-__device__ void expm(double* M, double* T1, double* T2, int n) {
-  double norm = 0;
-  for (int j = 0; j < n; j++) {
-    double c = 0;
-    for (int i = 0; i < n; i++) c += fabs(M[i * MAXD + j]);
-    norm = fmax(norm, c);
-  }
-  int s = 0;
-  if (norm > 0.5) {
-    frexp(norm, &s);  // norm = f 2^s, f in [0.5, 1)
-    s += 1;
-    if (s < 0) s = 0;
-    if (s > 60) s = 60;
-  }
-  const double sc = ldexp(1.0, -s);
-  for (int i = 0; i < n * MAXD; i++) M[i] *= sc;
-  // Horner form of sum_k M^k / k!, degree 14: T1 = I + M/14; T1 = I + (M/13) T1; ...
-  for (int i = 0; i < n; i++)
-    for (int j = 0; j < n; j++) T1[i * MAXD + j] = (i == j ? 1.0 : 0.0) + M[i * MAXD + j] * (1.0 / 14);
-  for (int k = 13; k >= 1; k--) {
-    matmul(M, T1, T2, n);
-    const double inv = 1.0 / k;
-    for (int i = 0; i < n; i++)
-      for (int j = 0; j < n; j++) T1[i * MAXD + j] = (i == j ? 1.0 : 0.0) + T2[i * MAXD + j] * inv;
-  }
-  for (int q = 0; q < s; q++) {
-    matmul(T1, T1, T2, n);
-    for (int i = 0; i < n * MAXD; i++) T1[i] = T2[i];
-  }
-  for (int i = 0; i < n * MAXD; i++) M[i] = T1[i];
-}
+// the per-system bodies (zoh_one, dlqr_one, reduce_one) live in f16_linalg.cuh, shared with the host build of the tests
 
 __global__ void __launch_bounds__(64)
 zoh_kernel(const double* __restrict__ A, const double* __restrict__ B, int n, int m, long long N, double dt,
            double* __restrict__ Ad, double* __restrict__ Bd) {
   double M[MAXD * MAXD], T1[MAXD * MAXD], T2[MAXD * MAXD];
-  for (long long p = (long long)blockIdx.x * blockDim.x + threadIdx.x; p < N; p += (long long)gridDim.x * blockDim.x) {
-    const int d = n + m;
-    for (int i = 0; i < d; i++)
-      for (int j = 0; j < d; j++) {
-        double v = 0;
-        if (i < n) v = (j < n ? A[p * n * n + i * n + j] : B[p * n * m + i * m + (j - n)]) * dt;
-        M[i * MAXD + j] = v;
-      }
-    expm(M, T1, T2, d);
-    for (int i = 0; i < n; i++) {
-      for (int j = 0; j < n; j++) Ad[p * n * n + i * n + j] = M[i * MAXD + j];
-      for (int j = 0; j < m; j++) Bd[p * n * m + i * m + j] = M[i * MAXD + n + j];
-    }
-  }
+  for (long long p = (long long)blockIdx.x * blockDim.x + threadIdx.x; p < N; p += (long long)gridDim.x * blockDim.x)
+    zoh_one(A, B, n, m, p, dt, Ad, Bd, M, T1, T2);
 }
 
-// Z = X^-1 by Gauss-Jordan with partial pivoting (n <= 18, ld MAXD); returns false when singular
-__device__ bool invert(const double* X, double* Z, double* W, int n) {
-  for (int i = 0; i < n; i++)
-    for (int j = 0; j < n; j++) {
-      W[i * MAXD + j] = X[i * MAXD + j];
-      Z[i * MAXD + j] = i == j ? 1.0 : 0.0;
-    }
-  for (int c = 0; c < n; c++) {
-    int piv = c;
-    double best = fabs(W[c * MAXD + c]);
-    for (int r = c + 1; r < n; r++)
-      if (fabs(W[r * MAXD + c]) > best) { best = fabs(W[r * MAXD + c]); piv = r; }
-    if (!(best > 0)) return false;
-    if (piv != c)
-      for (int j = 0; j < n; j++) {
-        double t = W[c * MAXD + j]; W[c * MAXD + j] = W[piv * MAXD + j]; W[piv * MAXD + j] = t;
-        t = Z[c * MAXD + j]; Z[c * MAXD + j] = Z[piv * MAXD + j]; Z[piv * MAXD + j] = t;
-      }
-    const double inv = 1.0 / W[c * MAXD + c];
-    for (int j = 0; j < n; j++) { W[c * MAXD + j] *= inv; Z[c * MAXD + j] *= inv; }
-    for (int r = 0; r < n; r++) {
-      if (r == c) continue;
-      const double f = W[r * MAXD + c];
-      if (f == 0) continue;
-      for (int j = 0; j < n; j++) {
-        W[r * MAXD + j] = fma(-f, W[c * MAXD + j], W[r * MAXD + j]);
-        Z[r * MAXD + j] = fma(-f, Z[c * MAXD + j], Z[r * MAXD + j]);
-      }
-    }
-  }
-  return true;
-}
-
-// Structured doubling for  P = A'PA - A'PB (R + B'PB)^-1 B'PA + Q:
-//   A0 = A, G0 = B R^-1 B', H0 = Q;  W = (I + G H)^-1;  A+ = A W A;  G+ = G + A W G A';  H+ = H + A' H W A;  H -> P
 __global__ void __launch_bounds__(64)
 dlqr_kernel(const double* __restrict__ Ad, const double* __restrict__ Bd, const double* __restrict__ Q, const double* __restrict__ R,
             int n, int m, long long N, int max_doublings, double tol, double* __restrict__ K, double* __restrict__ P_out,
             int* __restrict__ info) {
   double Ak[MAXD * MAXD], G[MAXD * MAXD], H[MAXD * MAXD], W[MAXD * MAXD], T1[MAXD * MAXD], T2[MAXD * MAXD], T3[MAXD * MAXD];
-  for (long long p = (long long)blockIdx.x * blockDim.x + threadIdx.x; p < N; p += (long long)gridDim.x * blockDim.x) {
-    const double* A0 = Ad + p * n * n;
-    const double* B0 = Bd + p * n * m;
-    int status = 0;
-    // R^-1 (m x m) -> T1;  G = B R^-1 B'
-    for (int i = 0; i < m; i++)
-      for (int j = 0; j < m; j++) T2[i * MAXD + j] = R[i * m + j];
-    if (!invert(T2, T1, T3, m)) status = -1;
-    for (int i = 0; i < n; i++)
-      for (int j = 0; j < m; j++) {  // T2 = B R^-1  (n x m)
-        double a = 0;
-        for (int k = 0; k < m; k++) a = fma(B0[i * m + k], T1[k * MAXD + j], a);
-        T2[i * MAXD + j] = a;
-      }
-    for (int i = 0; i < n; i++)
-      for (int j = 0; j < n; j++) {
-        double a = 0;
-        for (int k = 0; k < m; k++) a = fma(T2[i * MAXD + k], B0[j * m + k], a);
-        G[i * MAXD + j] = a;
-        Ak[i * MAXD + j] = A0[i * n + j];
-        H[i * MAXD + j] = Q[i * n + j];
-      }
-    int it = 0;
-    for (; it < max_doublings && status == 0; it++) {
-      matmul(G, H, T1, n);  // T1 = I + G H
-      for (int i = 0; i < n; i++) T1[i * MAXD + i] += 1.0;
-      if (!invert(T1, W, T2, n)) { status = -2; break; }
-      matmul(Ak, W, T1, n);                       // T1 = A W
-      matmul(T1, G, T2, n);                       // T2 = A W G
-      for (int i = 0; i < n; i++)                 // G += A W G A'
-        for (int j = 0; j < n; j++) {
-          double a = 0;
-          for (int k = 0; k < n; k++) a = fma(T2[i * MAXD + k], Ak[j * MAXD + k], a);
-          T3[i * MAXD + j] = a;
-        }
-      for (int i = 0; i < n; i++)
-        for (int j = 0; j < n; j++) G[i * MAXD + j] += T3[i * MAXD + j];
-      matmul(W, Ak, T2, n);                       // T2 = W A
-      matmul(H, T2, T3, n);                       // T3 = H W A
-      double dmax = 0, hmax = 0;
-      for (int i = 0; i < n; i++)                 // H += A' H W A
-        for (int j = 0; j < n; j++) {
-          double a = 0;
-          for (int k = 0; k < n; k++) a = fma(Ak[k * MAXD + i], T3[k * MAXD + j], a);
-          T2[i * MAXD + j] = a;
-        }
-      for (int i = 0; i < n; i++)
-        for (int j = 0; j < n; j++) {
-          H[i * MAXD + j] += T2[i * MAXD + j];
-          dmax = fmax(dmax, fabs(T2[i * MAXD + j]));
-          hmax = fmax(hmax, fabs(H[i * MAXD + j]));
-        }
-      matmul(T1, Ak, T2, n);                      // A <- A W A
-      for (int i = 0; i < n * MAXD; i++) Ak[i] = T2[i];
-      if (!(dmax == dmax)) { status = -3; break; }
-      if (dmax <= tol * hmax) { it++; break; }
-    }
-    if (status == 0 && it >= max_doublings) status = 1;  // not converged to tol
-    // symmetrise P, K = (R + B'PB)^-1 B'PA
-    for (int i = 0; i < n; i++)
-      for (int j = i + 1; j < n; j++) {
-        const double v = 0.5 * (H[i * MAXD + j] + H[j * MAXD + i]);
-        H[i * MAXD + j] = v;
-        H[j * MAXD + i] = v;
-      }
-    for (int i = 0; i < m; i++)                   // T1 = B'P  (m x n)
-      for (int j = 0; j < n; j++) {
-        double a = 0;
-        for (int k = 0; k < n; k++) a = fma(B0[k * m + i], H[k * MAXD + j], a);
-        T1[i * MAXD + j] = a;
-      }
-    for (int i = 0; i < m; i++)                   // T2 = R + B'PB (m x m)
-      for (int j = 0; j < m; j++) {
-        double a = R[i * m + j];
-        for (int k = 0; k < n; k++) a = fma(T1[i * MAXD + k], B0[k * m + j], a);
-        T2[i * MAXD + j] = a;
-      }
-    if (!invert(T2, W, T3, m) && status == 0) status = -4;
-    for (int i = 0; i < m; i++)                   // T3 = B'PA (m x n)
-      for (int j = 0; j < n; j++) {
-        double a = 0;
-        for (int k = 0; k < n; k++) a = fma(T1[i * MAXD + k], A0[k * n + j], a);
-        T3[i * MAXD + j] = a;
-      }
-    for (int i = 0; i < m; i++)
-      for (int j = 0; j < n; j++) {
-        double a = 0;
-        for (int k = 0; k < m; k++) a = fma(W[i * MAXD + k], T3[k * MAXD + j], a);
-        K[p * m * n + i * n + j] = status < 0 ? __longlong_as_double(0x7ff8000000000000LL) : a;
-      }
-    if (P_out)
-      for (int i = 0; i < n; i++)
-        for (int j = 0; j < n; j++) P_out[p * n * n + i * n + j] = H[i * MAXD + j];
-    if (info) {
-      info[2 * p] = status;
-      info[2 * p + 1] = it;
-    }
-  }
+  for (long long p = (long long)blockIdx.x * blockDim.x + threadIdx.x; p < N; p += (long long)gridDim.x * blockDim.x)
+    dlqr_one(Ad, Bd, Q, R, n, m, p, max_doublings, tol, K, P_out, info, Ak, G, H, W, T1, T2, T3);
 }
 
 __global__ void __launch_bounds__(256)
 reduce_jacobian_kernel(const double* __restrict__ A, long long N, double* __restrict__ A_na, double* __restrict__ B_na) {
-  // rows of the reduced model in full-state numbering (lf2dot, lf1dot swapped as env.py:184,189 does);
-  // columns: mpc_states = {phi, theta, alpha, beta, p, q, r, lf1, lf2} (parameters.py:135), inputs -> actuator states 13..15
-  const int rows[9] = {3, 4, 7, 8, 9, 10, 11, 16, 17};
-  const int cols[12] = {3, 4, 7, 8, 9, 10, 11, 17, 16, 13, 14, 15};
   for (long long e = (long long)blockIdx.x * blockDim.x + threadIdx.x; e < N * 108; e += (long long)gridDim.x * blockDim.x) {
     const long long p = e / 108;
-    const int k = (int)(e - p * 108), i = k / 12, j = k - i * 12;
-    const double v = A[p * 324 + rows[i] * 18 + cols[j]];
-    if (j < 9) A_na[p * 81 + i * 9 + j] = v;
-    else B_na[p * 27 + i * 3 + (j - 9)] = v;
+    reduce_one(A, p, (int)(e - p * 108), A_na, B_na);
   }
 }
 

@@ -186,9 +186,16 @@ int trim_batch(const double *h, const double *V, long long N, double tol, int ma
  * reduce_jacobian_batch: A [N][18][18] (forward linearise) -> the reference's 9-state / 3-input model (env.py:49,152-193):
  *   A_na [N][9][9] over mpc_states {phi,theta,alpha,beta,p,q,r,lf1,lf2}, B_na [N][9][3] over {dh,da,dr}.  An exact gather:
  *   _calc_xdot_na perturbs the same full-model evaluation (rows 3,4,7,8,9,10,11,16,17; the LEF derivatives swap, :184,189).
- * discretise_batch: scipy.signal.cont2discrete(method='zoh') of env.py:46,50 for N systems, A [N][n][n], B [N][n][m].
+ * discretise_batch: scipy.signal.cont2discrete(method='zoh') of env.py:46,50 for N systems, A [N][n][n], B [N][n][m];
+ *   a non-finite dt is F16_ERR_ARG.
  * dlqr_batch: utils.py:219-245, K [N][m][n] = (B'PB + R)^-1 B'PA with P [N][n][n] (may be NULL) from the discrete Riccati
- *   equation; Q [n][n], R [m][m] shared by all systems; info [N][2] = {0 ok / 1 not converged / <0 singular, doublings}.
+ *   equation; Q [n][n], R [m][m] shared by all systems; info [N][2] (may be NULL) = {status, doublings done}, status:
+ *      0  converged, P solves the equation (residual test), A - BK stable (its powers shrink below 1/2 in norm)
+ *      1  tolerance not met in 64 doublings     -4  R + B'PB singular
+ *     -1  R singular                            -5  converged to a P for which A - BK is not stable ((A, Q) not detectable)
+ *     -2  I + GH singular in a doubling         -6  converged to an H that fails the residual test (the doubling broke
+ *     -3  NaN or Inf in the data or an iterate      down numerically)
+ *   K of a system with a negative status is NaN; P is still written.
  * lqr_gain_batch: F16._calc_LQR_gain (env.py:344-358) for N operating points, device end to end: K [N][3][9] = -dlqr(...).
  * n <= 18, n + m <= 22. */
 int reduce_jacobian_batch(const double *A, long long N, double *A_na, double *B_na);

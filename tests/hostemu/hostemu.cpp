@@ -1,12 +1,13 @@
-// hostemu.cpp -- DEVELOPMENT AID, TESTS ONLY.  Compiles the device arithmetic header (csrc/f16_model.cuh) for the
-// host so that the kernels' logic (cell search, node-interleaved gathers, operation order) can be checked against
-// the oracle on a machine without a GPU.  It is never part of libf16_b200.so and nothing in the package loads it;
+// hostemu.cpp -- DEVELOPMENT AID, TESTS ONLY.  Compiles the device arithmetic headers (csrc/f16_model.cuh, f16_fast.cuh,
+// f16_linalg.cuh) for the host so that the kernels' logic (cell search, node-interleaved gathers, operation order, the
+// linalg bodies) can be checked against the oracle and high-precision references on a machine without a GPU.  It is never part of libf16_b200.so and nothing in the package loads it;
 // the product has no CPU path.
 #include <string>
 #include <vector>
 
 #include "../../f16_mpc_oop_py_b200/csrc/f16_model.cuh"
 #include "../../f16_mpc_oop_py_b200/csrc/f16_fast.cuh"
+#include "../../f16_mpc_oop_py_b200/csrc/f16_linalg.cuh"
 #include "../../f16_mpc_oop_py_b200/csrc/f16_tables_host.h"
 
 static std::vector<double> g_hifi, g_lofi, g_fast;
@@ -191,5 +192,26 @@ __attribute__((visibility("default"))) unsigned emu_trim(double h, double V, int
 __attribute__((visibility("default"))) void emu_div_by(const double* a, long long n, double y, double* out) {
   const double r = 1.0 / y;
   for (long long i = 0; i < n; i++) out[i] = f16::div_by(a[i], y, r);
+}
+// the linalg bodies of f16_linalg.cu, one system after the other (the kernels run one system per thread).  Without FMA
+// contraction, unlike linalg.o: the results agree with the device's to rounding, not bit for bit.
+__attribute__((visibility("default"))) void emu_zoh(const double* A, const double* B, int n, int m, long long N, double dt,
+                                                    double* Ad, double* Bd) {
+  const int sz = f16::linalg::MAXD * f16::linalg::MAXD;
+  std::vector<double> s(3 * sz);
+  for (long long p = 0; p < N; p++) f16::linalg::zoh_one(A, B, n, m, p, dt, Ad, Bd, &s[0], &s[sz], &s[2 * sz]);
+}
+// the library's settings are max_doublings = 64, tol = 1e-15 (f16_api.cu)
+__attribute__((visibility("default"))) void emu_dlqr(const double* A, const double* B, const double* Q, const double* R, int n, int m,
+                                                     long long N, int max_doublings, double tol, double* K, double* P, int* info) {
+  const int sz = f16::linalg::MAXD * f16::linalg::MAXD;
+  std::vector<double> s(7 * sz);
+  for (long long p = 0; p < N; p++)
+    f16::linalg::dlqr_one(A, B, Q, R, n, m, p, max_doublings, tol, K, P, info, &s[0], &s[sz], &s[2 * sz], &s[3 * sz], &s[4 * sz],
+                          &s[5 * sz], &s[6 * sz]);
+}
+__attribute__((visibility("default"))) void emu_reduce_jacobian(const double* A, long long N, double* A_na, double* B_na) {
+  for (long long p = 0; p < N; p++)
+    for (int k = 0; k < 108; k++) f16::linalg::reduce_one(A, p, k, A_na, B_na);
 }
 }
