@@ -22,9 +22,15 @@ static_assert(sizeof(f16_lqr_t) == sizeof(f16::LqrLaw), "f16_lqr_t and the devic
 
 namespace {
 
-struct DevBuf {  // grow-only device scratch for the host-pointer entry points
+struct DevBuf {  // grow-only device scratch; a reserve that grows it moves it
   void* p = nullptr;
   size_t cap = 0;
+  DevBuf() = default;
+  DevBuf(const DevBuf&) = delete;
+  DevBuf& operator=(const DevBuf&) = delete;
+  ~DevBuf() {
+    if (p) cudaFree(p);
+  }
   cudaError_t reserve(size_t bytes) {
     if (bytes <= cap) return cudaSuccess;
     if (p) cudaFree(p);
@@ -34,22 +40,21 @@ struct DevBuf {  // grow-only device scratch for the host-pointer entry points
     if (e == cudaSuccess) cap = bytes;
     return e;
   }
-  void release() {
-    if (p) cudaFree(p);
-    p = nullptr;
-    cap = 0;
-  }
 };
+
+constexpr int kMaxArrays = 16;    // per-aircraft arrays of one host-buffer call (lqr_gain_batch: 13)
+constexpr int kMaxContexts = 64;  // device contexts of f16_init_devices
 
 // Everything that belongs to ONE device: streams, events, the three table images, scratch.  The library keeps one context per
 // device handed to f16_init_devices (exactly one after f16_init); aircraft never interact, so contexts share nothing.
 struct Dev {
   int ordinal = -1;
   int sm_count = 0;
-  cudaStream_t stream = nullptr;                 // kernels (and the copies of the single-shot paths)
-  cudaStream_t s_in = nullptr, s_out = nullptr;  // H2D / D2H of the pipelined host-buffer entry points
+  cudaStream_t stream = nullptr;                 // kernels, and the copies of the *_dev-side helpers (f16_memcpy_*)
+  cudaStream_t s_in = nullptr, s_out = nullptr;  // H2D / D2H of the host-buffer entry points
   cudaEvent_t ev0 = nullptr, ev1 = nullptr;      // f16_timer_*
   cudaEvent_t e_in[3] = {}, e_work[3] = {}, e_out[3] = {};  // the three slots of the chunk pipeline
+  cudaEvent_t e_snap[2] = {}, e_snap_out[2] = {};         // step_batch_traj: snapshot slot filled (stream) / copied out (s_out)
   double* d_hifi = nullptr;
   double* d_lofi = nullptr;
   double* d_hifi_fast = nullptr;
@@ -57,24 +62,29 @@ struct Dev {
   // legacy single-aircraft path: mapped pinned host memory, the kernel reads and writes it directly
   double* pin = nullptr;      // [17 in | 18 out | 3 atmos in/out ...]
   double* pin_dev = nullptr;
-  DevBuf b_in, b_in2, b_out, b_fi, b_xcg, b_st, b_st2, b_a, b_b, b_flush, b_l1, b_l2, b_l3, b_l4, b_l5, b_sum, b_perm, b_pscr, b_px, b_pu, b_pxcg, b_pst, b_pk, b_redo, b_prog;
+  // Scratch.  A reserve may move a buffer, so two stages that are live at the same time never share one.
+  // slot[i]: array i of the running host-buffer call, all its chunk slots (run_pipeline).  What runs inside that call's work
+  // has its own buffers:
+  //   step_on_device -> step_partitioned: b_perm, b_pscr, b_px, b_pu, b_pxcg, b_pst, b_pk
+  //                  -> step_compacting:  b_perm, b_pscr, b_pk, b_c*  (the two are alternatives, neither runs inside the other)
+  //   the step kernels: b_prog;  run_xdot / run_linearise: b_redo;  the summary rows: b_sum;  step_batch_traj's two
+  //   snapshots: b_snap;  the Q / R of dlqr_batch and lqr_gain_batch: b_qr
+  // b_flush: f16_flush_l2, and the sink of f16_measure_fp64_peak; neither runs inside another call.
+  DevBuf slot[kMaxArrays];
+  DevBuf b_perm, b_pscr, b_px, b_pu, b_pxcg, b_pst, b_pk;
   DevBuf b_cx[2], b_cu[2], b_cxcg[2], b_cst[2], b_ck[2], b_co[2], b_cflag, b_ckl;  // survivor compaction (step_compacting)
-  std::vector<DevBuf*> bufs() {
-    return {&b_in, &b_in2, &b_out, &b_fi, &b_xcg, &b_st, &b_st2, &b_a, &b_b, &b_flush, &b_l1, &b_l2, &b_l3, &b_l4, &b_l5, &b_sum, &b_perm,
-            &b_pscr, &b_px, &b_pu, &b_pxcg, &b_pst, &b_pk, &b_redo, &b_prog, &b_cx[0], &b_cx[1], &b_cu[0], &b_cu[1], &b_cxcg[0],
-            &b_cxcg[1], &b_cst[0], &b_cst[1], &b_ck[0], &b_ck[1], &b_co[0], &b_co[1], &b_cflag, &b_ckl};
-  }
-  void destroy() {  // tolerant of a half-built context (a failed init releases what it had created)
+  DevBuf b_prog, b_redo, b_sum, b_snap, b_qr, b_flush;
+  ~Dev() {  // tolerant of a half-built context (a failed init releases what it had created); the buffers go after this body
     if (ordinal < 0 || cudaSetDevice(ordinal) != cudaSuccess) { cudaGetLastError(); return; }
     if (stream) cudaStreamSynchronize(stream);
     if (s_in) cudaStreamSynchronize(s_in);
     if (s_out) cudaStreamSynchronize(s_out);
-    for (DevBuf* b : bufs()) b->release();
     if (d_hifi) cudaFree(d_hifi);
     if (d_lofi) cudaFree(d_lofi);
     if (d_hifi_fast) cudaFree(d_hifi_fast);
     if (pin) cudaFreeHost(pin);
-    for (cudaEvent_t e : {ev0, ev1, e_in[0], e_in[1], e_in[2], e_work[0], e_work[1], e_work[2], e_out[0], e_out[1], e_out[2]})
+    for (cudaEvent_t e : {ev0, ev1, e_in[0], e_in[1], e_in[2], e_work[0], e_work[1], e_work[2], e_out[0], e_out[1], e_out[2],
+                          e_snap[0], e_snap[1], e_snap_out[0], e_snap_out[1]})
       if (e) cudaEventDestroy(e);
     for (cudaStream_t st : {stream, s_in, s_out})
       if (st) cudaStreamDestroy(st);
@@ -173,6 +183,10 @@ int create_context(Dev* d, int ordinal) {
     CK(cudaEventCreateWithFlags(&d->e_work[i], cudaEventDisableTiming));
     CK(cudaEventCreateWithFlags(&d->e_out[i], cudaEventDisableTiming));
   }
+  for (int i = 0; i < 2; i++) {
+    CK(cudaEventCreateWithFlags(&d->e_snap[i], cudaEventDisableTiming));
+    CK(cudaEventCreateWithFlags(&d->e_snap_out[i], cudaEventDisableTiming));
+  }
   CK(cudaHostAlloc((void**)&d->pin, 64 * sizeof(double), cudaHostAllocMapped));
   CK(cudaHostGetDevicePointer((void**)&d->pin_dev, d->pin, 0));
   return upload_tables();
@@ -203,7 +217,7 @@ int init_locked(const char* table_path, int device, const int* devices, int ndev
   }
   for (int o : want)
     if (o < 0 || o >= present) { set_err("device %d out of range (%d present)", o, present); return G.init_rc = F16_ERR_ARG; }
-  if (want.size() > 64) { set_err("more than 64 device contexts"); return G.init_rc = F16_ERR_ARG; }
+  if ((int)want.size() > kMaxContexts) { set_err("more than %d device contexts", kMaxContexts); return G.init_rc = F16_ERR_ARG; }
 
   std::string err;
   if (!f16::load_canonical(table_path, lib_dir(), G.payload, G.table_source, err)) {
@@ -227,7 +241,6 @@ int init_locked(const char* table_path, int device, const int* devices, int ndev
     const int rc = create_context(G.devs.back().get(), o);
     if (rc != F16_OK) {
       const std::string keep = t_err;
-      for (auto& d : G.devs) d->destroy();
       G.devs.clear();
       D = nullptr;
       t_err = keep;
@@ -271,36 +284,21 @@ f16::BatchSel sel_of(const unsigned char* fi, int fi_default, const double* xcg,
   return f16::BatchSel{fi, fi_default, xcg, xcg_default};
 }
 
-// host -> device staging of the optional per-aircraft selectors
-int stage_sel(const unsigned char* fi, const double* xcg, long long N, const unsigned char** d_fi, const double** d_xcg) {
-  *d_fi = nullptr;
-  *d_xcg = nullptr;
-  if (fi) {
-    CK(D->b_fi.reserve((size_t)N));
-    CK(cudaMemcpyAsync(D->b_fi.p, fi, (size_t)N, cudaMemcpyHostToDevice, D->stream));
-    *d_fi = (const unsigned char*)D->b_fi.p;
-  }
-  if (xcg) {
-    CK(D->b_xcg.reserve((size_t)N * 8));
-    CK(cudaMemcpyAsync(D->b_xcg.p, xcg, (size_t)N * 8, cudaMemcpyHostToDevice, D->stream));
-    *d_xcg = (const double*)D->b_xcg.p;
-  }
-  return F16_OK;
-}
-
 #define DISPATCH(fn, ...) (G.math_mode == F16_MATH_FAST ? f16::fast::fn(__VA_ARGS__) : f16::strict::fn(__VA_ARGS__))
 
 // the one-shot entry points: in F16_MATH_FAST a batch worth staging tables for runs the TMA-tiled kernels on the arithmetic of
 // f16_fast.cuh (f16_step_fast.cu); a handful of aircraft (the legacy Nlplant symbol among them) read the tables through L2
 bool oneshot_fast(long long N) { return G.math_mode == F16_MATH_FAST && G.smem_tables && N >= 4096; }
-cudaError_t run_nlplant(const f16::BatchSel& sel, const double* xu, long long ld_in, double* xdot, long long ld_out, long long N,
-                        int* status) {
+// Nlplant_batch (u == NULL: x is xu [17][ld_x]) and calc_xdot_batch
+cudaError_t run_xdot(const f16::BatchSel& sel, const double* x, long long ld_x, const double* u, long long ld_u, double* xdot,
+                     long long ld_out, long long N, int* status) {
   if (oneshot_fast(N)) {
     cudaError_t e = D->b_redo.reserve((size_t)((N + 31) / 32) * 4);
     if (e != cudaSuccess) return e;
-    return f16::fast::launch_xdot_fast(cfg(true), tabs(), sel, xu, ld_in, nullptr, 0, xdot, ld_out, N, status, (unsigned*)D->b_redo.p);
+    return f16::fast::launch_xdot_fast(cfg(true), tabs(), sel, x, ld_x, u, ld_u, xdot, ld_out, N, status, (unsigned*)D->b_redo.p);
   }
-  return DISPATCH(launch_nlplant, cfg(G.smem_tables && N >= 4096), tabs(), sel, xu, ld_in, xdot, ld_out, N, status);
+  if (!u) return DISPATCH(launch_nlplant, cfg(G.smem_tables && N >= 4096), tabs(), sel, x, ld_x, xdot, ld_out, N, status);
+  return DISPATCH(launch_calc_xdot, cfg(G.smem_tables && N >= 4096), tabs(), sel, x, ld_x, u, ld_u, xdot, ld_out, N, status);
 }
 // linearise_batch.  F16_MATH_STRICT: the staged reference-order kernels (variant 0 / 2: CTA per 32 aircraft, 1: warp per
 // aircraft).  F16_MATH_FAST, variant 0: the two-aircraft-per-warp kernel on the arithmetic of f16_fast.cuh
@@ -315,17 +313,13 @@ cudaError_t run_linearise(const f16::BatchSel& sel, const double* x, long long l
   }
   return f16::strict::launch_linearise(cfg(true), tabs(), sel, x, ld_x, u, ld_u, N, eps, scheme, A, B, status);
 }
-cudaError_t run_calc_xdot(const f16::BatchSel& sel, const double* x, long long ld_x, const double* u, long long ld_u, double* xdot,
-                          long long ld_out, long long N, int* status) {
-  if (oneshot_fast(N)) {
-    cudaError_t e = D->b_redo.reserve((size_t)((N + 31) / 32) * 4);
-    if (e != cudaSuccess) return e;
-    return f16::fast::launch_xdot_fast(cfg(true), tabs(), sel, x, ld_x, u, ld_u, xdot, ld_out, N, status, (unsigned*)D->b_redo.p);
-  }
-  return DISPATCH(launch_calc_xdot, cfg(G.smem_tables && N >= 4096), tabs(), sel, x, ld_x, u, ld_u, xdot, ld_out, N, status);
+
+int bad_arg(const char* entry) {
+  set_err("%s: bad argument", entry);
+  return F16_ERR_ARG;
 }
 
-
+// ---- the argument checks, one per operation: the host-buffer form of an operation is its *_dev form with every ld = N ----
 bool lqr_ok(const f16_lqr_t* lqr) {
   if (!lqr) return true;
   if (lqr->n_sel < 0 || lqr->n_sel > 18) return false;
@@ -333,21 +327,85 @@ bool lqr_ok(const f16_lqr_t* lqr) {
     if (lqr->sel[j] < 0 || lqr->sel[j] > 17) return false;
   return true;
 }
+bool nlplant_ok(const double* xu, long long ld_in, const double* xdot, long long ld_out, long long N) {
+  return N >= 0 && (N == 0 || (xu && xdot)) && ld_in >= N && ld_out >= N;
+}
+bool calc_xdot_ok(const double* x, long long ld_x, const double* u, long long ld_u, const double* xdot, long long ld_out, long long N) {
+  return nlplant_ok(x, ld_x, xdot, ld_out, N) && (N == 0 || u) && ld_u >= N;
+}
+bool step_ok(const double* x, long long ld_x, const double* u, long long ld_u, long long N, int K, const f16_lqr_t* lqr) {
+  return N >= 0 && K >= 0 && (N == 0 || (x && u)) && ld_x >= N && ld_u >= N && lqr_ok(lqr);
+}
+bool stats_ok(const double* x, long long ld_x, const double* u, long long ld_u, long long N, int K, int snap_every,
+              const f16_lqr_t* lqr, const double* rows) {
+  return step_ok(x, ld_x, u, ld_u, N, K, lqr) && snap_every >= 1 && (rows || K < snap_every);
+}
+bool linearise_ok(const double* x, long long ld_x, const double* u, long long ld_u, long long N, double eps, int scheme,
+                  const double* A, const double* B) {
+  return N >= 0 && (N == 0 || (x && u && A && B)) && ld_x >= N && ld_u >= N && (scheme == 0 || scheme == 1) &&
+         eps >= 1e-12 && eps <= 1e3;
+}
+bool trim_ok(const double* h, const double* V, long long N, double tol, int maxiter, const double* x_trim, long long ld_x,
+             const double* info, long long ld_info) {
+  return N >= 0 && (N == 0 || (h && V && x_trim)) && ld_x >= N && (!info || ld_info >= N) && tol >= 0 && maxiter >= 1;
+}
+bool summary_ok(const double* x, long long ld_x, long long N, const double* row) {
+  return N >= 0 && row && (N == 0 || x) && ld_x >= N;
+}
+bool dims_ok(int n, int m) { return n >= 1 && m >= 1 && n <= 18 && n + m <= 22; }
+bool reduce_ok(const double* A, long long N, const double* A_na, const double* B_na) {
+  return N >= 0 && (N == 0 || (A && A_na && B_na));
+}
+bool zoh_ok(const double* A, const double* B, int n, int m, long long N, double dt, const double* Ad, const double* Bd) {
+  return N >= 0 && dims_ok(n, m) && std::isfinite(dt) && (N == 0 || (A && B && Ad && Bd));
+}
+bool dlqr_ok(const double* Ad, const double* Bd, const double* Q, const double* R, int n, int m, long long N, const double* K) {
+  return N >= 0 && dims_ok(n, m) && (N == 0 || (Ad && Bd && Q && R && K));
+}
 
 // ---- host arrays <-> device slots of the host-buffer entry points -----------------------------------------------------
-// `planes` rows of m doubles: `ld_host` doubles apart in the caller's array, m apart on the device
-cudaError_t planes_h2d(void* dst, const double* src, long long ld_host, long long m, int planes, cudaStream_t st) {
-  if (ld_host == m || planes == 1) return cudaMemcpyAsync(dst, src, (size_t)planes * m * 8, cudaMemcpyHostToDevice, st);
-  return cudaMemcpy2DAsync(dst, (size_t)m * 8, src, (size_t)ld_host * 8, (size_t)m * 8, (size_t)planes, cudaMemcpyHostToDevice, st);
+// One per-aircraft array of a host-buffer call.  In the caller's array aircraft i has `planes` elements `ld` apart starting at
+// element i (SoA) or the `row` elements from i * row on (AoS); on the device a chunk of m aircraft is packed: planes m apart, or
+// m rows.  A NULL array gets no slot and the kernels see NULL, unless it is `scratch`: then the kernels get a slot and nothing
+// is copied (status words the caller does not want, the intermediates of lqr_gain_batch).
+enum Dir { IN = 1, OUT = 2, INOUT = 3 };
+struct Arr {
+  void* host;
+  int dir;
+  int esize;   // bytes per element
+  int planes;  // SoA: planes per aircraft (AoS: 1)
+  int row;     // AoS: elements per aircraft (SoA: 1)
+  bool scratch;
+};
+Arr soa(const void* host, int dir, int esize, int planes = 1, bool scratch = false) {
+  return Arr{const_cast<void*>(host), dir, esize, planes, 1, scratch};
 }
-cudaError_t planes_d2h(double* dst, long long ld_host, const void* src, long long m, int planes, cudaStream_t st) {
-  if (ld_host == m || planes == 1) return cudaMemcpyAsync(dst, src, (size_t)planes * m * 8, cudaMemcpyDeviceToHost, st);
-  return cudaMemcpy2DAsync(dst, (size_t)ld_host * 8, src, (size_t)m * 8, (size_t)m * 8, (size_t)planes, cudaMemcpyDeviceToHost, st);
+Arr aos(const void* host, int dir, int esize, int row, bool scratch = false) {
+  return Arr{const_cast<void*>(host), dir, esize, 1, row, scratch};
 }
+
+// aircraft [first, first + m) of `a` (plane stride ld) <-> its packed device slot
+cudaError_t copy_chunk(const Arr& a, void* slot, long long ld, long long first, long long m, cudaMemcpyKind kind, cudaStream_t st) {
+  char* host = (char*)a.host + (size_t)first * a.row * a.esize;
+  const size_t w = (size_t)m * a.row * a.esize;  // bytes of one plane of the chunk
+  const bool in = kind == cudaMemcpyHostToDevice;
+  void* dst = in ? slot : host;
+  const void* src = in ? (const void*)host : slot;
+  if (a.planes == 1 || ld == m) return cudaMemcpyAsync(dst, src, (size_t)a.planes * w, kind, st);
+  const size_t hp = (size_t)ld * a.esize;
+  return cudaMemcpy2DAsync(dst, in ? w : hp, src, in ? hp : w, w, (size_t)a.planes, kind, st);
+}
+
+struct Slots {  // the device slots of one chunk, by array position (NULL: the array was not passed)
+  void* p[kMaxArrays];
+  double* f64(int i) const { return (double*)p[i]; }
+  int* i32(int i) const { return (int*)p[i]; }
+  const unsigned char* u8(int i) const { return (const unsigned char*)p[i]; }
+};
 
 // A host-buffer call on one device is a pipeline of chunks: while the kernels of chunk c run on D->stream, chunk c + 1 arrives on
 // D->s_in and the result of chunk c - 1 leaves on D->s_out (PCIe is full duplex: a copy-bound call -- one derivative, one step --
-// takes max(in, out) instead of in + kernel + out).  Chunk c lives in slot c mod 3 of the device scratch; chunks are multiples
+// takes max(in, out) instead of in + kernel + out).  Chunk c lives in slot c mod 3 of each array's buffer; chunks are multiples
 // of 32 aircraft, so that slots stay 256-byte aligned and a warp-task never straddles two chunks.  Results do not depend on the
 // cut: every aircraft is computed by the same arithmetic wherever it lands.
 struct Chunks {
@@ -364,47 +422,64 @@ Chunks plan_chunks(long long n, long long min_chunk, int max_chunks) {
   c.slots = c.count < 3 ? c.count : 3;
   return c;
 }
+// a call whose kernels must see all n aircraft at once (n >= 1): a trim launch lasts as long as its slowest point, a summary
+// row reduces the whole slice
+Chunks one_chunk(long long n) { return plan_chunks(n, n, 1); }
 
-// in(slot, lo, m, stream): enqueue the H2D of aircraft [lo, lo + m) of this call into `slot`; work(slot, lo, m): enqueue the kernels
-// on D->stream; out(slot, lo, m, stream): enqueue the D2H.  All three return F16_* codes.  Returns after everything has landed.
-// Issue order on the host: normally in(c), work(c), out(c - 1) -- work() only enqueues, and a pageable in(c + 1), which blocks
-// the host while the driver stages it, then runs under the kernels of chunk c.  With work_blocks (work() waits on the device:
-// the survivor counts of step_compacting) the copies either side of a chunk are enqueued BEFORE its work: in(c + 1), out(c - 1),
-// work(c).
-template <class In, class Work, class Out>
-int run_pipeline(long long n, const Chunks& ch, bool work_blocks, In in, Work work, Out out) {
-  auto span = [&](int c, long long* lo, long long* m) {
-    *lo = (long long)c * ch.chunk;
-    *m = (n - *lo) < ch.chunk ? (n - *lo) : ch.chunk;
+// Aircraft [lo, lo + n) of the arrays `arr` (plane stride ld) in the chunks `ch`: the pipeline copies in the IN arrays of each
+// chunk, calls work(slots, m) to enqueue its kernels on D->stream, and copies out the OUT arrays.  Returns after everything has
+// landed.  Issue order on the host: normally in(c), work(c), out(c - 1) -- work() only enqueues, and a pageable in(c + 1), which
+// blocks the host while the driver stages it, then runs under the kernels of chunk c.  With work_blocks (work() waits on the
+// device: the survivor counts of step_compacting) the copies either side of a chunk are enqueued BEFORE its work: in(c + 1),
+// out(c - 1), work(c).
+template <size_t NA, class Work>
+int run_pipeline(const Arr (&arr)[NA], long long ld, long long lo, long long n, const Chunks& ch, bool work_blocks, Work work) {
+  static_assert(NA <= kMaxArrays, "one slot buffer per array");
+  size_t bytes[NA];  // per aircraft
+  for (size_t i = 0; i < NA; i++) {
+    bytes[i] = (size_t)arr[i].planes * arr[i].row * arr[i].esize;
+    if (arr[i].host || arr[i].scratch) CK(D->slot[i].reserve((size_t)ch.slots * ch.chunk * bytes[i]));
+  }
+  auto slot = [&](size_t i, int c) -> void* {
+    if (!arr[i].host && !arr[i].scratch) return nullptr;
+    return (char*)D->slot[i].p + (size_t)(c % 3) * ch.chunk * bytes[i];
+  };
+  auto span = [&](int c, long long* first, long long* m) {
+    *first = (long long)c * ch.chunk;
+    *m = (n - *first) < ch.chunk ? (n - *first) : ch.chunk;
+    *first += lo;
+  };
+  auto copies = [&](int c, int dir, cudaStream_t st) -> int {
+    long long first, m;
+    span(c, &first, &m);
+    for (size_t i = 0; i < NA; i++)
+      if (arr[i].host && (arr[i].dir & dir))
+        CK(copy_chunk(arr[i], slot(i, c), ld, first, m, dir == IN ? cudaMemcpyHostToDevice : cudaMemcpyDeviceToHost, st));
+    return F16_OK;
   };
   auto fetch = [&](int c) -> int {
-    const int s = c % 3;
-    long long lo, m;
-    span(c, &lo, &m);
-    if (c >= 3) CK(cudaStreamWaitEvent(D->s_in, D->e_out[s], 0));  // the slot is free once its previous result has left
-    const int rc = in(s, lo, m, D->s_in);
+    if (c >= 3) CK(cudaStreamWaitEvent(D->s_in, D->e_out[c % 3], 0));  // the slot is free once its previous result has left
+    const int rc = copies(c, IN, D->s_in);
     if (rc != F16_OK) return rc;
-    CK(cudaEventRecord(D->e_in[s], D->s_in));
+    CK(cudaEventRecord(D->e_in[c % 3], D->s_in));
     return F16_OK;
   };
   auto run = [&](int c) -> int {
-    const int s = c % 3;
-    long long lo, m;
-    span(c, &lo, &m);
-    CK(cudaStreamWaitEvent(D->stream, D->e_in[s], 0));
-    const int rc = work(s, lo, m);
+    long long first, m;
+    span(c, &first, &m);
+    Slots p;
+    for (size_t i = 0; i < NA; i++) p.p[i] = slot(i, c);
+    CK(cudaStreamWaitEvent(D->stream, D->e_in[c % 3], 0));
+    const int rc = work(p, m);
     if (rc != F16_OK) return rc;
-    CK(cudaEventRecord(D->e_work[s], D->stream));
+    CK(cudaEventRecord(D->e_work[c % 3], D->stream));
     return F16_OK;
   };
   auto flush = [&](int c) -> int {
-    const int s = c % 3;
-    long long lo, m;
-    span(c, &lo, &m);
-    CK(cudaStreamWaitEvent(D->s_out, D->e_work[s], 0));
-    const int rc = out(s, lo, m, D->s_out);
+    CK(cudaStreamWaitEvent(D->s_out, D->e_work[c % 3], 0));
+    const int rc = copies(c, OUT, D->s_out);
     if (rc != F16_OK) return rc;
-    CK(cudaEventRecord(D->e_out[s], D->s_out));
+    CK(cudaEventRecord(D->e_out[c % 3], D->s_out));
     return F16_OK;
   };
   int rc = F16_OK;
@@ -435,59 +510,65 @@ int run_pipeline(long long n, const Chunks& ch, bool work_blocks, In in, Work wo
 // ---- one call over several devices ------------------------------------------------------------------------------------
 // Aircraft are independent: the batch is cut into contiguous slices, one per device context (boundaries on multiples of 32
 // aircraft), and every slice runs the single-device path on its own context from its own host thread -- copies and kernels of
-// the slices overlap, nothing is exchanged between devices (SURVEY 8e: no collective on the data path).  f(lo, n) is called
-// with D set to the slice's context.  A batch too small to feed more than one device stays on the current context.
+// the slices overlap, nothing is exchanged between devices (SURVEY 8e: no collective on the data path).  A batch too small to
+// feed more than one device stays on the current context.
 struct Span {
   long long lo, n;
 };
-std::vector<Span> device_spans(long long N, long long min_per_device, long long contexts = -1) {
-  long long parts = contexts > 0 ? contexts : (long long)G.devs.size();
+struct Spans {
+  int count = 0;
+  Span at[kMaxContexts];
+};
+Spans device_spans(long long N, long long min_per_device, long long contexts) {
+  long long parts = contexts;
   if (min_per_device > 0 && N / min_per_device < parts) parts = N / min_per_device;
   if (parts < 1) parts = 1;
-  std::vector<Span> v;
+  Spans v;
   const long long groups = (N + 31) / 32;
   long long g0 = 0;
   for (long long i = 0; i < parts; i++) {
     const long long g1 = groups * (i + 1) / parts;
     const long long lo = g0 * 32, hi = g1 * 32 < N ? g1 * 32 : N;
-    if (hi > lo) v.push_back(Span{lo, hi - lo});
+    if (hi > lo) v.at[v.count++] = Span{lo, hi - lo};
     g0 = g1;
   }
   return v;
 }
+// the slices of a call over the library's contexts (N >= 1)
+Spans slices(long long N, long long min_per_device) { return device_spans(N, min_per_device, (long long)G.devs.size()); }
 
+// f(i, lo, n) for every slice i, with D set to context i (one slice: the current context, on the calling thread)
 template <class F>
-int on_devices(long long N, long long min_per_device, F f) {
+int on_devices(const Spans& spans, F f) {
+  if (spans.count <= 1) return f(0, spans.at[0].lo, spans.at[0].n);
   try {
-    const std::vector<Span> spans = G.devs.size() > 1 ? device_spans(N, min_per_device) : std::vector<Span>{Span{0, N}};
-    if (spans.size() <= 1) return f(0LL, N);  // current context, calling thread
-    std::vector<int> rcs(spans.size(), F16_OK);
-    std::vector<std::string> errs(spans.size());
+    std::vector<int> rcs(spans.count, F16_OK);
+    std::vector<std::string> errs(spans.count);
     std::vector<std::thread> workers;
-    auto body = [&](size_t i) {
+    auto body = [&](int i) {
       D = G.devs[i].get();
       if (cudaSetDevice(D->ordinal) != cudaSuccess) {
         set_err("cudaSetDevice(%d) failed", D->ordinal);
         rcs[i] = F16_ERR_CUDA;
       } else {
-        rcs[i] = f(spans[i].lo, spans[i].n);
+        rcs[i] = f(i, spans.at[i].lo, spans.at[i].n);
       }
       errs[i] = t_err;
     };
     Dev* mine = D;
-    size_t started = 1;
+    int started = 1;
     try {
-      for (; started < spans.size(); started++) workers.emplace_back(body, started);
+      for (; started < spans.count; started++) workers.emplace_back(body, started);
     } catch (...) {  // no more threads: the calling thread takes the remaining slices one after the other
     }
     body(0);
-    for (size_t i = started; i < spans.size(); i++) body(i);
+    for (int i = started; i < spans.count; i++) body(i);
     for (std::thread& w : workers) w.join();
     D = mine;
     cudaSetDevice(D->ordinal);
-    for (size_t i = 0; i < spans.size(); i++)
+    for (int i = 0; i < spans.count; i++)
       if (rcs[i] != F16_OK) {
-        set_err("device context %d (cuda:%d): %s", (int)i, G.devs[i]->ordinal, errs[i].c_str());
+        set_err("device context %d (cuda:%d): %s", i, G.devs[i]->ordinal, errs[i].c_str());
         return rcs[i];
       }
     return F16_OK;
@@ -510,6 +591,47 @@ void merge_summary_row(double* a, const double* b) {
       a[38 + i] = a[38 + i] + d * (nb / nt);
       a[56 + i] = a[56 + i] + b[56 + i] + d * d * (na * nb / nt);
     }
+  }
+}
+
+// K steps in launches of snap_every back to back on D->stream (step_batch is restartable bit for bit at any step boundary),
+// snap(j) after the j-th full launch
+template <class Snap>
+int snapshot_steps(double* d_x, long long ld_x, const double* d_u, long long ld_u, long long N, int K, int snap_every,
+                          double dt, const f16_lqr_t* lqr, const f16::BatchSel& sel, int* d_status, Snap snap) {
+  const bool smem = G.smem_tables && (N * (long long)snap_every >= 4096);
+  for (int done = 0, j = 0; done < K;) {
+    const int k = (K - done) < snap_every ? (K - done) : snap_every;
+    CK(DISPATCH(launch_step, cfg(smem), tabs(), sel, d_x, ld_x, d_u, ld_u, N, k, dt, reinterpret_cast<const f16::LqrLaw*>(lqr),
+                d_status, nullptr));
+    done += k;
+    if (k == snap_every) {
+      const int rc = snap(j++);
+      if (rc != F16_OK) return rc;
+    }
+  }
+  return F16_OK;
+}
+
+// Statistics of a batch sliced over the device contexts: f(lo, n, rows) writes the n_rows summary rows of aircraft [lo, lo + n)
+// on its context; the rows of the slices are combined on the host (Chan's update, slice order).  N >= 1.
+template <class F>
+int merged_rows(long long N, long long min_per_device, int n_rows, double* rows, F f) {
+  try {
+    const Spans spans = slices(N, min_per_device);
+    const size_t per = (size_t)n_rows * 74;
+    std::vector<double> part(spans.count * per);
+    const int rc = on_devices(spans, [&](int i, long long lo, long long n) { return f(lo, n, part.data() + i * per); });
+    if (rc != F16_OK) return rc;
+    for (int r = 0; r < n_rows; r++) {
+      double* dst = rows + (size_t)r * 74;
+      memcpy(dst, part.data() + (size_t)r * 74, 74 * 8);
+      for (int i = 1; i < spans.count; i++) merge_summary_row(dst, part.data() + i * per + (size_t)r * 74);
+    }
+    return F16_OK;
+  } catch (const std::exception& e) {
+    set_err("host resources: %s", e.what());
+    return F16_ERR_HOST;
   }
 }
 
@@ -542,7 +664,6 @@ int f16_init_devices(const char* table_path, const int* devices, int ndev) {
 
 void f16_shutdown(void) {
   std::lock_guard<std::mutex> lk(G_mu);
-  for (auto& d : G.devs) d->destroy();
   G.devs.clear();
   D = nullptr;
   G.ready = false;
@@ -555,17 +676,14 @@ void f16_shutdown(void) {
 // host logic only (no CUDA call): how a host-buffer batch call would cut N aircraft over `contexts` device contexts and, on one
 // context, into pipeline chunks.  lo_n [2 * contexts] = (first aircraft, count) per slice; returns the number of slices used.
 int f16_plan_slices(long long N, long long min_per_device, int contexts, long long* lo_n) {
-  if (N < 0 || contexts < 1 || contexts > 64 || !lo_n) return F16_ERR_ARG;
-  try {
-    const std::vector<Span> v = N > 0 ? device_spans(N, min_per_device, contexts) : std::vector<Span>();
-    for (size_t i = 0; i < v.size(); i++) {
-      lo_n[2 * i] = v[i].lo;
-      lo_n[2 * i + 1] = v[i].n;
-    }
-    return (int)v.size();
-  } catch (const std::exception&) {
-    return F16_ERR_HOST;
+  if (N < 0 || contexts < 1 || contexts > kMaxContexts || !lo_n) return F16_ERR_ARG;
+  if (N == 0) return 0;
+  const Spans v = device_spans(N, min_per_device, contexts);
+  for (int i = 0; i < v.count; i++) {
+    lo_n[2 * i] = v.at[i].lo;
+    lo_n[2 * i + 1] = v.at[i].n;
   }
+  return v.count;
 }
 int f16_plan_chunks(long long n, long long min_chunk, int max_chunks, long long* chunk, int* slots) {
   if (n < 1 || min_chunk < 1 || max_chunks < 1 || !chunk || !slots) return F16_ERR_ARG;
@@ -757,8 +875,8 @@ int Nlplant_batch_dev(const double* xu_soa, long long ld_in, double* xdot_soa, l
   std::lock_guard<std::mutex> lk(G_mu);
   int rc = ensure();
   if (rc != F16_OK) return rc;
-  if (N < 0 || (N > 0 && (!xu_soa || !xdot_soa)) || ld_in < N || ld_out < N) { set_err("Nlplant_batch_dev: bad argument"); return F16_ERR_ARG; }
-  CK(run_nlplant(sel_of(fi, fi_default, xcg, xcg_default), xu_soa, ld_in, xdot_soa, ld_out, N, status));
+  if (!nlplant_ok(xu_soa, ld_in, xdot_soa, ld_out, N)) return bad_arg("Nlplant_batch_dev");
+  CK(run_xdot(sel_of(fi, fi_default, xcg, xcg_default), xu_soa, ld_in, nullptr, 0, xdot_soa, ld_out, N, status));
   return F16_OK;
 }
 
@@ -768,8 +886,8 @@ int calc_xdot_batch_dev(const double* x_soa, long long ld_x, const double* u_soa
   std::lock_guard<std::mutex> lk(G_mu);
   int rc = ensure();
   if (rc != F16_OK) return rc;
-  if (N < 0 || (N > 0 && (!x_soa || !u_soa || !xdot_soa)) || ld_x < N || ld_u < N || ld_out < N) { set_err("calc_xdot_batch_dev: bad argument"); return F16_ERR_ARG; }
-  CK(run_calc_xdot(sel_of(fi, fi_default, xcg, xcg_default), x_soa, ld_x, u_soa, ld_u, xdot_soa, ld_out, N, status));
+  if (!calc_xdot_ok(x_soa, ld_x, u_soa, ld_u, xdot_soa, ld_out, N)) return bad_arg("calc_xdot_batch_dev");
+  CK(run_xdot(sel_of(fi, fi_default, xcg, xcg_default), x_soa, ld_x, u_soa, ld_u, xdot_soa, ld_out, N, status));
   return F16_OK;
 }
 
@@ -849,7 +967,7 @@ int step_batch_dev(double* x_soa, long long ld_x, const double* u_soa, long long
   std::lock_guard<std::mutex> lk(G_mu);
   int rc = ensure();
   if (rc != F16_OK) return rc;
-  if (N < 0 || K < 0 || (N > 0 && (!x_soa || !u_soa)) || ld_x < N || ld_u < N || !lqr_ok(lqr)) { set_err("step_batch_dev: bad argument"); return F16_ERR_ARG; }
+  if (!step_ok(x_soa, ld_x, u_soa, ld_u, N, K, lqr)) return bad_arg("step_batch_dev");
   reserve_step_progress(N);
   return step_on_device(x_soa, ld_x, u_soa, ld_u, N, K, dt, lqr, fi, fi_default, xcg, xcg_default, status, steps_done);
 }
@@ -860,77 +978,24 @@ int linearise_batch_dev(const double* x_soa, long long ld_x, const double* u_soa
   std::lock_guard<std::mutex> lk(G_mu);
   int rc = ensure();
   if (rc != F16_OK) return rc;
-  if (N < 0 || (N > 0 && (!x_soa || !u_soa || !A || !B)) || ld_x < N || ld_u < N || (scheme != 0 && scheme != 1) || !(eps >= 1e-12 && eps <= 1e3)) {
-    set_err("linearise_batch_dev: bad argument");
-    return F16_ERR_ARG;
-  }
+  if (!linearise_ok(x_soa, ld_x, u_soa, ld_u, N, eps, scheme, A, B)) return bad_arg("linearise_batch_dev");
   CK(run_linearise(sel_of(fi, fi_default, xcg, xcg_default), x_soa, ld_x, u_soa, ld_u, N, eps, scheme, A, B, status));
   return F16_OK;
 }
 
 // ---- host-pointer entry points: slices over the device contexts, a chunk pipeline on each -------------------------------
-#define H2D(dst, src, bytes) CK(cudaMemcpyAsync(dst, src, bytes, cudaMemcpyHostToDevice, D->stream))
-#define D2H(dst, src, bytes) CK(cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToHost, D->stream))
-
-// the per-aircraft selectors of a chunk: host arrays (offset already applied) -> slot s of b_fi / b_xcg
-static int sel_h2d(const unsigned char* fi, const double* xcg, long long chunk, int s, long long m, cudaStream_t st,
-                   const unsigned char** d_fi, const double** d_xcg) {
-  *d_fi = nullptr;
-  *d_xcg = nullptr;
-  if (fi) {
-    unsigned char* p = (unsigned char*)D->b_fi.p + (size_t)s * chunk;
-    CK(cudaMemcpyAsync(p, fi, (size_t)m, cudaMemcpyHostToDevice, st));
-    *d_fi = p;
-  }
-  if (xcg) {
-    double* p = (double*)D->b_xcg.p + (size_t)s * chunk;
-    CK(cudaMemcpyAsync(p, xcg, (size_t)m * 8, cudaMemcpyHostToDevice, st));
-    *d_xcg = p;
-  }
-  return F16_OK;
-}
-static int sel_reserve(const unsigned char* fi, const double* xcg, const Chunks& ch) {
-  if (fi) CK(D->b_fi.reserve((size_t)ch.slots * ch.chunk));
-  if (xcg) CK(D->b_xcg.reserve((size_t)ch.slots * ch.chunk * 8));
-  return F16_OK;
-}
+// The arrays of a call are listed in a fixed order; its work() finds the device slot of array i at p.*(i).
 
 // Nlplant_batch (u == NULL: x is xu [17][ld]) / calc_xdot_batch for aircraft [lo, lo + n) of the caller's arrays on the context D
 static int xdot_host(const double* x, const double* u, double* xdot, long long ld, long long lo, long long n, const unsigned char* fi,
                      int fi_default, const double* xcg, double xcg_default, int* status) {
-  const int NX = u ? 18 : 17;
-  const Chunks ch = plan_chunks(n, 1 << 16, 8);
-  const size_t cs = (size_t)ch.chunk;
-  CK(D->b_in.reserve((size_t)ch.slots * NX * cs * 8));
-  if (u) CK(D->b_in2.reserve((size_t)ch.slots * 4 * cs * 8));
-  CK(D->b_out.reserve((size_t)ch.slots * 18 * cs * 8));
-  CK(D->b_st.reserve((size_t)ch.slots * cs * 4));
-  int rc = sel_reserve(fi, xcg, ch);
-  if (rc != F16_OK) return rc;
-  const unsigned char* d_fi[3] = {};
-  const double* d_xcg[3] = {};
-  auto xs = [&](int s) { return (double*)D->b_in.p + (size_t)s * NX * cs; };
-  auto us = [&](int s) { return (double*)D->b_in2.p + (size_t)s * 4 * cs; };
-  auto os = [&](int s) { return (double*)D->b_out.p + (size_t)s * 18 * cs; };
-  auto ss = [&](int s) { return (int*)D->b_st.p + (size_t)s * cs; };
-  return run_pipeline(
-      n, ch, false,
-      [&](int s, long long c, long long m, cudaStream_t st) -> int {
-        CK(planes_h2d(xs(s), x + lo + c, ld, m, NX, st));
-        if (u) CK(planes_h2d(us(s), u + lo + c, ld, m, 4, st));
-        return sel_h2d(fi ? fi + lo + c : nullptr, xcg ? xcg + lo + c : nullptr, ch.chunk, s, m, st, &d_fi[s], &d_xcg[s]);
-      },
-      [&](int s, long long, long long m) -> int {
-        const f16::BatchSel sel = sel_of(d_fi[s], fi_default, d_xcg[s], xcg_default);
-        if (u) CK(run_calc_xdot(sel, xs(s), m, us(s), m, os(s), m, m, ss(s)));
-        else CK(run_nlplant(sel, xs(s), m, os(s), m, m, ss(s)));
-        return F16_OK;
-      },
-      [&](int s, long long c, long long m, cudaStream_t st) -> int {
-        CK(planes_d2h(xdot + lo + c, ld, os(s), m, 18, st));
-        if (status) CK(cudaMemcpyAsync(status + lo + c, ss(s), (size_t)m * 4, cudaMemcpyDeviceToHost, st));
-        return F16_OK;
-      });
+  return run_pipeline({soa(x, IN, 8, u ? 18 : 17), soa(u, IN, 8, 4), soa(fi, IN, 1), soa(xcg, IN, 8), soa(xdot, OUT, 8, 18),
+                       soa(status, OUT, 4, 1, true)},
+                      ld, lo, n, plan_chunks(n, 1 << 16, 8), false, [&](const Slots& p, long long m) -> int {
+                        CK(run_xdot(sel_of(p.u8(2), fi_default, p.f64(3), xcg_default), p.f64(0), m, p.f64(1), u ? m : 0, p.f64(4),
+                                    m, m, p.i32(5)));
+                        return F16_OK;
+                      });
 }
 
 int Nlplant_batch(const double* xu_soa, double* xdot_soa, const unsigned char* fi, int fi_default, const double* xcg,
@@ -938,9 +1003,9 @@ int Nlplant_batch(const double* xu_soa, double* xdot_soa, const unsigned char* f
   std::lock_guard<std::mutex> lk(G_mu);
   int rc = ensure();
   if (rc != F16_OK) return rc;
-  if (N < 0 || (N > 0 && (!xu_soa || !xdot_soa))) { set_err("Nlplant_batch: bad argument"); return F16_ERR_ARG; }
+  if (!nlplant_ok(xu_soa, N, xdot_soa, N, N)) return bad_arg("Nlplant_batch");
   if (N == 0) return F16_OK;
-  return on_devices(N, 16384, [&](long long lo, long long n) {
+  return on_devices(slices(N, 16384), [&](int, long long lo, long long n) {
     return xdot_host(xu_soa, nullptr, xdot_soa, N, lo, n, fi, fi_default, xcg, xcg_default, status);
   });
 }
@@ -950,9 +1015,9 @@ int calc_xdot_batch(const double* x_soa, const double* u_soa, double* xdot_soa, 
   std::lock_guard<std::mutex> lk(G_mu);
   int rc = ensure();
   if (rc != F16_OK) return rc;
-  if (N < 0 || (N > 0 && (!x_soa || !u_soa || !xdot_soa))) { set_err("calc_xdot_batch: bad argument"); return F16_ERR_ARG; }
+  if (!calc_xdot_ok(x_soa, N, u_soa, N, xdot_soa, N, N)) return bad_arg("calc_xdot_batch");
   if (N == 0) return F16_OK;
-  return on_devices(N, 16384, [&](long long lo, long long n) {
+  return on_devices(slices(N, 16384), [&](int, long long lo, long long n) {
     return xdot_host(x_soa, u_soa, xdot_soa, N, lo, n, fi, fi_default, xcg, xcg_default, status);
   });
 }
@@ -1077,40 +1142,18 @@ static int step_on_device(double* d_x, long long ld_x, const double* d_u, long l
 
 // step_batch for aircraft [lo, lo + n) of the caller's arrays on the context D.  A long run (K >= 512) is cut into at most four
 // chunks of >= 2^18 aircraft (the time-chunked schedule of the step kernel wants many rounds of warp-tasks per launch); a short
-// one, which is copy-bound, into up to eight of >= 2^16.
+// one, which is copy-bound, into up to eight of >= 2^16.  The kernels always get status and step-count slots: step_compacting
+// needs the status words.
 static int step_host(double* x, const double* u, long long ld, long long lo, long long n, int K, double dt, const f16_lqr_t* lqr,
                      const unsigned char* fi, int fi_default, const double* xcg, double xcg_default, int* status, int* steps_done) {
   const Chunks ch = K >= 512 ? plan_chunks(n, 1 << 18, 4) : plan_chunks(n, 1 << 16, 8);
-  const size_t cs = (size_t)ch.chunk;
-  CK(D->b_in.reserve((size_t)ch.slots * 18 * cs * 8));
-  CK(D->b_in2.reserve((size_t)ch.slots * 4 * cs * 8));
-  CK(D->b_st.reserve((size_t)ch.slots * cs * 4));
-  CK(D->b_st2.reserve((size_t)ch.slots * cs * 4));
-  int rc = sel_reserve(fi, xcg, ch);
-  if (rc != F16_OK) return rc;
   reserve_step_progress(ch.chunk);
-  const unsigned char* d_fi[3] = {};
-  const double* d_xcg[3] = {};
-  auto xs = [&](int s) { return (double*)D->b_in.p + (size_t)s * 18 * cs; };
-  auto us = [&](int s) { return (double*)D->b_in2.p + (size_t)s * 4 * cs; };
-  auto ss = [&](int s) { return (int*)D->b_st.p + (size_t)s * cs; };
-  auto ks = [&](int s) { return (int*)D->b_st2.p + (size_t)s * cs; };
-  return run_pipeline(
-      n, ch, G.compaction && K >= 4096,
-      [&](int s, long long c, long long m, cudaStream_t st) -> int {
-        CK(planes_h2d(xs(s), x + lo + c, ld, m, 18, st));
-        CK(planes_h2d(us(s), u + lo + c, ld, m, 4, st));
-        return sel_h2d(fi ? fi + lo + c : nullptr, xcg ? xcg + lo + c : nullptr, ch.chunk, s, m, st, &d_fi[s], &d_xcg[s]);
-      },
-      [&](int s, long long, long long m) -> int {
-        return step_on_device(xs(s), m, us(s), m, m, K, dt, lqr, d_fi[s], fi_default, d_xcg[s], xcg_default, ss(s), ks(s));
-      },
-      [&](int s, long long c, long long m, cudaStream_t st) -> int {
-        CK(planes_d2h(x + lo + c, ld, xs(s), m, 18, st));
-        if (status) CK(cudaMemcpyAsync(status + lo + c, ss(s), (size_t)m * 4, cudaMemcpyDeviceToHost, st));
-        if (steps_done) CK(cudaMemcpyAsync(steps_done + lo + c, ks(s), (size_t)m * 4, cudaMemcpyDeviceToHost, st));
-        return F16_OK;
-      });
+  return run_pipeline({soa(x, INOUT, 8, 18), soa(u, IN, 8, 4), soa(fi, IN, 1), soa(xcg, IN, 8), soa(status, OUT, 4, 1, true),
+                       soa(steps_done, OUT, 4, 1, true)},
+                      ld, lo, n, ch, G.compaction && K >= 4096, [&](const Slots& p, long long m) {
+                        return step_on_device(p.f64(0), m, p.f64(1), m, m, K, dt, lqr, p.u8(2), fi_default, p.f64(3), xcg_default,
+                                              p.i32(4), p.i32(5));
+                      });
 }
 
 int step_batch(double* x_soa, const double* u_soa, long long N, int K, double dt, const f16_lqr_t* lqr,
@@ -1119,56 +1162,36 @@ int step_batch(double* x_soa, const double* u_soa, long long N, int K, double dt
   std::lock_guard<std::mutex> lk(G_mu);
   int rc = ensure();
   if (rc != F16_OK) return rc;
-  if (N < 0 || K < 0 || (N > 0 && (!x_soa || !u_soa)) || !lqr_ok(lqr)) { set_err("step_batch: bad argument"); return F16_ERR_ARG; }
+  if (!step_ok(x_soa, N, u_soa, N, N, K, lqr)) return bad_arg("step_batch");
   if (N == 0) return F16_OK;
-  return on_devices(N, 16384, [&](long long lo, long long n) {
+  return on_devices(slices(N, 16384), [&](int, long long lo, long long n) {
     return step_host(x_soa, u_soa, N, lo, n, K, dt, lqr, fi, fi_default, xcg, xcg_default, status, steps_done);
   });
 }
 
-// K Euler steps with a snapshot of the whole state every `snap_every` steps: traj [K / snap_every][18][N].
-// Launches of snap_every steps back to back on one stream (step_batch is restartable bit for bit at any K boundary),
-// each snapshot copied out while the next chunk of steps runs.  Aircraft [lo, lo + n) of the caller's arrays on the context D.
-static int traj_host(double* x, const double* u, long long ld, long long lo, long long n_, int K, int snap_every, double dt,
+// K Euler steps with a snapshot of the whole state every `snap_every` steps: traj [K / snap_every][18][N], each snapshot copied
+// out of one of two device slots while the next launch runs.  Aircraft [lo, lo + n) of the caller's arrays on the context D.
+static int traj_host(double* x, const double* u, long long ld, long long lo, long long n, int K, int snap_every, double dt,
                      const f16_lqr_t* lqr, const unsigned char* fi, int fi_default, const double* xcg, double xcg_default,
                      double* traj, int* status) {
-  const size_t n = (size_t)n_;
-  CK(D->b_in.reserve(18 * n * 8));
-  CK(D->b_in2.reserve(4 * n * 8));
-  CK(D->b_out.reserve(2 * 18 * n * 8));  // two snapshot slots: copy-out of one overlaps the next chunk of steps
-  CK(D->b_st.reserve(n * 4));
-  const unsigned char* d_fi;
-  const double* d_xcg;
-  int rc = stage_sel(fi ? fi + lo : nullptr, xcg ? xcg + lo : nullptr, n_, &d_fi, &d_xcg);
-  if (rc != F16_OK) return rc;
-  CK(planes_h2d(D->b_in.p, x + lo, ld, n_, 18, D->stream));
-  CK(planes_h2d(D->b_in2.p, u + lo, ld, n_, 4, D->stream));
-  reserve_step_progress(n_);
-  const bool smem = G.smem_tables && (n_ * (long long)snap_every >= 4096);
-  const f16::BatchSel sel = sel_of(d_fi, fi_default, d_xcg, xcg_default);
-  int done = 0, snap = 0;
-  while (done < K) {
-    const int k = (K - done) < snap_every ? (K - done) : snap_every;
-    CK(DISPATCH(launch_step, cfg(smem), tabs(), sel, (double*)D->b_in.p, n_, (const double*)D->b_in2.p, n_, n_, k, dt,
-                reinterpret_cast<const f16::LqrLaw*>(lqr), (int*)D->b_st.p, nullptr));
-    done += k;
-    if (k == snap_every) {
-      double* slot = (double*)D->b_out.p + (size_t)(snap & 1) * 18 * n;
-      // the slot's previous copy-out (two snapshots ago, on s_out) has completed before this copy overwrites it
-      if (snap >= 2) CK(cudaStreamWaitEvent(D->stream, D->e_out[snap & 1], 0));
-      CK(cudaMemcpyAsync(slot, D->b_in.p, 18 * n * 8, cudaMemcpyDeviceToDevice, D->stream));
-      CK(cudaEventRecord(D->e_work[snap & 1], D->stream));
-      CK(cudaStreamWaitEvent(D->s_out, D->e_work[snap & 1], 0));
-      CK(planes_d2h(traj + (size_t)snap * 18 * (size_t)ld + lo, ld, slot, n_, 18, D->s_out));
-      CK(cudaEventRecord(D->e_out[snap & 1], D->s_out));
-      snap++;
-    }
-  }
-  CK(planes_d2h(x + lo, ld, D->b_in.p, n_, 18, D->stream));
-  if (status) D2H(status + lo, D->b_st.p, n * 4);
-  CK(cudaStreamSynchronize(D->stream));
-  CK(cudaStreamSynchronize(D->s_out));
-  return F16_OK;
+  CK(D->b_snap.reserve(2 * 18 * (size_t)n * 8));
+  reserve_step_progress(n);
+  return run_pipeline(
+      {soa(x, INOUT, 8, 18), soa(u, IN, 8, 4), soa(fi, IN, 1), soa(xcg, IN, 8), soa(status, OUT, 4, 1, true)}, ld, lo, n,
+      one_chunk(n), false, [&](const Slots& p, long long m) {
+        const f16::BatchSel sel = sel_of(p.u8(2), fi_default, p.f64(3), xcg_default);
+        return snapshot_steps(p.f64(0), m, p.f64(1), m, m, K, snap_every, dt, lqr, sel, p.i32(4), [&](int j) -> int {
+          double* snap = (double*)D->b_snap.p + (size_t)(j & 1) * 18 * m;
+          // the slot's previous copy-out (two snapshots ago, on s_out) has completed before this copy overwrites it
+          if (j >= 2) CK(cudaStreamWaitEvent(D->stream, D->e_snap_out[j & 1], 0));
+          CK(cudaMemcpyAsync(snap, p.f64(0), 18 * (size_t)m * 8, cudaMemcpyDeviceToDevice, D->stream));
+          CK(cudaEventRecord(D->e_snap[j & 1], D->stream));
+          CK(cudaStreamWaitEvent(D->s_out, D->e_snap[j & 1], 0));
+          CK(copy_chunk(soa(traj + (size_t)j * 18 * ld, OUT, 8, 18), snap, ld, lo, m, cudaMemcpyDeviceToHost, D->s_out));
+          CK(cudaEventRecord(D->e_snap_out[j & 1], D->s_out));
+          return F16_OK;
+        });
+      });
 }
 
 int step_batch_traj(double* x_soa, const double* u_soa, long long N, int K, int snap_every, double dt, const f16_lqr_t* lqr,
@@ -1176,12 +1199,9 @@ int step_batch_traj(double* x_soa, const double* u_soa, long long N, int K, int 
   std::lock_guard<std::mutex> lk(G_mu);
   int rc = ensure();
   if (rc != F16_OK) return rc;
-  if (N < 0 || K < 0 || snap_every < 1 || (N > 0 && (!x_soa || !u_soa || (!traj && K >= snap_every))) || !lqr_ok(lqr)) {
-    set_err("step_batch_traj: bad argument");
-    return F16_ERR_ARG;
-  }
+  if (!step_ok(x_soa, N, u_soa, N, N, K, lqr) || snap_every < 1 || (N > 0 && !traj && K >= snap_every)) return bad_arg("step_batch_traj");
   if (N == 0) return F16_OK;
-  return on_devices(N, 16384, [&](long long lo, long long n) {
+  return on_devices(slices(N, 16384), [&](int, long long lo, long long n) {
     return traj_host(x_soa, u_soa, N, lo, n, K, snap_every, dt, lqr, fi, fi_default, xcg, xcg_default, traj, status);
   });
 }
@@ -1190,39 +1210,13 @@ int step_batch_traj(double* x_soa, const double* u_soa, long long N, int K, int 
 // the pipeline keeps it running from the first chunk to the last
 static int linearise_host(const double* x, const double* u, long long ld, long long lo, long long n, double eps, int scheme, double* A,
                           double* B, const unsigned char* fi, int fi_default, const double* xcg, double xcg_default, int* status) {
-  const Chunks ch = plan_chunks(n, 1 << 14, 8);
-  const size_t cs = (size_t)ch.chunk;
-  CK(D->b_in.reserve((size_t)ch.slots * 18 * cs * 8));
-  CK(D->b_in2.reserve((size_t)ch.slots * 4 * cs * 8));
-  CK(D->b_a.reserve((size_t)ch.slots * 324 * cs * 8));
-  CK(D->b_b.reserve((size_t)ch.slots * 72 * cs * 8));
-  CK(D->b_st.reserve((size_t)ch.slots * cs * 4));
-  int rc = sel_reserve(fi, xcg, ch);
-  if (rc != F16_OK) return rc;
-  const unsigned char* d_fi[3] = {};
-  const double* d_xcg[3] = {};
-  auto xs = [&](int s) { return (double*)D->b_in.p + (size_t)s * 18 * cs; };
-  auto us = [&](int s) { return (double*)D->b_in2.p + (size_t)s * 4 * cs; };
-  auto as = [&](int s) { return (double*)D->b_a.p + (size_t)s * 324 * cs; };
-  auto bs = [&](int s) { return (double*)D->b_b.p + (size_t)s * 72 * cs; };
-  auto ss = [&](int s) { return (int*)D->b_st.p + (size_t)s * cs; };
-  return run_pipeline(
-      n, ch, false,
-      [&](int s, long long c, long long m, cudaStream_t st) -> int {
-        CK(planes_h2d(xs(s), x + lo + c, ld, m, 18, st));
-        CK(planes_h2d(us(s), u + lo + c, ld, m, 4, st));
-        return sel_h2d(fi ? fi + lo + c : nullptr, xcg ? xcg + lo + c : nullptr, ch.chunk, s, m, st, &d_fi[s], &d_xcg[s]);
-      },
-      [&](int s, long long, long long m) -> int {
-        CK(run_linearise(sel_of(d_fi[s], fi_default, d_xcg[s], xcg_default), xs(s), m, us(s), m, m, eps, scheme, as(s), bs(s), ss(s)));
-        return F16_OK;
-      },
-      [&](int s, long long c, long long m, cudaStream_t st) -> int {
-        CK(cudaMemcpyAsync(A + (size_t)(lo + c) * 324, as(s), (size_t)m * 324 * 8, cudaMemcpyDeviceToHost, st));
-        CK(cudaMemcpyAsync(B + (size_t)(lo + c) * 72, bs(s), (size_t)m * 72 * 8, cudaMemcpyDeviceToHost, st));
-        if (status) CK(cudaMemcpyAsync(status + lo + c, ss(s), (size_t)m * 4, cudaMemcpyDeviceToHost, st));
-        return F16_OK;
-      });
+  return run_pipeline({soa(x, IN, 8, 18), soa(u, IN, 8, 4), soa(fi, IN, 1), soa(xcg, IN, 8), aos(A, OUT, 8, 324), aos(B, OUT, 8, 72),
+                       soa(status, OUT, 4, 1, true)},
+                      ld, lo, n, plan_chunks(n, 1 << 14, 8), false, [&](const Slots& p, long long m) -> int {
+                        CK(run_linearise(sel_of(p.u8(2), fi_default, p.f64(3), xcg_default), p.f64(0), m, p.f64(1), m, m, eps, scheme,
+                                         p.f64(4), p.f64(5), p.i32(6)));
+                        return F16_OK;
+                      });
 }
 
 int linearise_batch(const double* x_soa, const double* u_soa, long long N, double eps, int scheme, double* A, double* B,
@@ -1230,12 +1224,9 @@ int linearise_batch(const double* x_soa, const double* u_soa, long long N, doubl
   std::lock_guard<std::mutex> lk(G_mu);
   int rc = ensure();
   if (rc != F16_OK) return rc;
-  if (N < 0 || (N > 0 && (!x_soa || !u_soa || !A || !B)) || (scheme != 0 && scheme != 1) || !(eps >= 1e-12 && eps <= 1e3)) {
-    set_err("linearise_batch: bad argument");
-    return F16_ERR_ARG;
-  }
+  if (!linearise_ok(x_soa, N, u_soa, N, N, eps, scheme, A, B)) return bad_arg("linearise_batch");
   if (N == 0) return F16_OK;
-  return on_devices(N, 4096, [&](long long lo, long long n) {
+  return on_devices(slices(N, 4096), [&](int, long long lo, long long n) {
     return linearise_host(x_soa, u_soa, N, lo, n, eps, scheme, A, B, fi, fi_default, xcg, xcg_default, status);
   });
 }
@@ -1249,39 +1240,25 @@ int trim_batch_dev(const double* h, const double* V, long long N, double tol, in
   std::lock_guard<std::mutex> lk(G_mu);
   int rc = ensure();
   if (rc != F16_OK) return rc;
-  if (N < 0 || (N > 0 && (!h || !V || !x_trim_soa)) || ld_x < N || (info_soa && ld_info < N) || !(tol >= 0) || maxiter < 1) {
-    set_err("trim_batch_dev: bad argument");
-    return F16_ERR_ARG;
-  }
+  if (!trim_ok(h, V, N, tol, maxiter, x_trim_soa, ld_x, info_soa, ld_info)) return bad_arg("trim_batch_dev");
   CK(DISPATCH(launch_trim, cfg(G.smem_tables && N >= 1024), tabs(), sel_of(fi, fi_default, xcg, xcg_default), h, V, N, tol, maxiter,
               ux0 ? ux0 : kTrimGuess, x_trim_soa, ld_x, info_soa, ld_info, status));
   return F16_OK;
 }
 
-// flight conditions [lo, lo + n_) of the caller's arrays on the context D (a search is ~2000 dependent evaluations per point:
+// flight conditions [lo, lo + n) of the caller's arrays on the context D (a search is ~2000 dependent evaluations per point:
 // nothing to pipeline, the copies are 16 + 180 B per point)
-static int trim_host(const double* h, const double* V, long long ld, long long lo, long long n_, double tol, int maxiter, const double* ux0,
+static int trim_host(const double* h, const double* V, long long ld, long long lo, long long n, double tol, int maxiter, const double* ux0,
                      double* x_trim, double* info, const unsigned char* fi, int fi_default, const double* xcg, double xcg_default,
                      int* status) {
-  const size_t n = (size_t)n_;
-  CK(D->b_in.reserve(2 * n * 8));
-  CK(D->b_out.reserve(18 * n * 8));
-  CK(D->b_a.reserve(4 * n * 8));
-  CK(D->b_st.reserve(n * 4));
-  const unsigned char* d_fi;
-  const double* d_xcg;
-  int rc = stage_sel(fi ? fi + lo : nullptr, xcg ? xcg + lo : nullptr, n_, &d_fi, &d_xcg);
-  if (rc != F16_OK) return rc;
-  double* d = (double*)D->b_in.p;
-  H2D(d, h + lo, n * 8);
-  H2D(d + n, V + lo, n * 8);
-  CK(DISPATCH(launch_trim, cfg(G.smem_tables && n_ >= 1024), tabs(), sel_of(d_fi, fi_default, d_xcg, xcg_default), d, d + n, n_, tol,
-              maxiter, ux0 ? ux0 : kTrimGuess, (double*)D->b_out.p, n_, (double*)D->b_a.p, n_, (int*)D->b_st.p));
-  CK(planes_d2h(x_trim + lo, ld, D->b_out.p, n_, 18, D->stream));
-  if (info) CK(planes_d2h(info + lo, ld, D->b_a.p, n_, 4, D->stream));
-  if (status) D2H(status + lo, D->b_st.p, n * 4);
-  CK(cudaStreamSynchronize(D->stream));
-  return F16_OK;
+  return run_pipeline({soa(h, IN, 8), soa(V, IN, 8), soa(fi, IN, 1), soa(xcg, IN, 8), soa(x_trim, OUT, 8, 18),
+                       soa(info, OUT, 8, 4, true), soa(status, OUT, 4, 1, true)},
+                      ld, lo, n, one_chunk(n), false, [&](const Slots& p, long long m) -> int {
+                        CK(DISPATCH(launch_trim, cfg(G.smem_tables && m >= 1024), tabs(),
+                                    sel_of(p.u8(2), fi_default, p.f64(3), xcg_default), p.f64(0), p.f64(1), m, tol, maxiter,
+                                    ux0 ? ux0 : kTrimGuess, p.f64(4), m, p.f64(5), m, p.i32(6)));
+                        return F16_OK;
+                      });
 }
 
 int trim_batch(const double* h, const double* V, long long N, double tol, int maxiter, const double* ux0, double* x_trim_soa,
@@ -1289,30 +1266,22 @@ int trim_batch(const double* h, const double* V, long long N, double tol, int ma
   std::lock_guard<std::mutex> lk(G_mu);
   int rc = ensure();
   if (rc != F16_OK) return rc;
-  if (N < 0 || (N > 0 && (!h || !V || !x_trim_soa)) || !(tol >= 0) || maxiter < 1) { set_err("trim_batch: bad argument"); return F16_ERR_ARG; }
+  if (!trim_ok(h, V, N, tol, maxiter, x_trim_soa, N, info_soa, N)) return bad_arg("trim_batch");
   if (N == 0) return F16_OK;
-  return on_devices(N, 2048, [&](long long lo, long long n) {
+  return on_devices(slices(N, 2048), [&](int, long long lo, long long n) {
     return trim_host(h, V, N, lo, n, tol, maxiter, ux0, x_trim_soa, info_soa, fi, fi_default, xcg, xcg_default, status);
   });
 }
 
 // ---- end-of-run statistics, reduced on the device (f16_stats.cu) ------------------------------------------------------
-// enqueue the two reduction kernels; row_dev (74 doubles) must not alias the scratch (PARTIAL_STRIDE doubles per CTA column)
-static int enqueue_summary(const double* d_x, long long ld, long long N, const int* d_status, double* row_dev, double* scratch,
-                           int grid) {
-  CK(f16::stats::launch_summary(cfg(false), d_x, ld, N, d_status, row_dev, scratch, grid));
-  return F16_OK;
-}
-
-static int summary_common(const double* d_x, long long ld, long long N, const int* d_status, double* row_host) {
+// enqueue the summary row of aircraft [0, N) and its copy to row_host (74 doubles) on D->stream
+static int summary_row(const double* d_x, long long ld, long long N, const int* d_status, double* row_host) {
   const int grid = f16::stats::summary_grid(cfg(false), N);
   CK(D->b_sum.reserve(((size_t)grid * f16::stats::PARTIAL_STRIDE + 80) * 8));
   double* scratch = (double*)D->b_sum.p;
-  double* row = scratch + (size_t)grid * f16::stats::PARTIAL_STRIDE;
-  int rc = enqueue_summary(d_x, ld, N, d_status, row, scratch, grid);
-  if (rc != F16_OK) return rc;
-  D2H(row_host, row, 74 * 8);
-  CK(cudaStreamSynchronize(D->stream));
+  double* row = scratch + (size_t)grid * f16::stats::PARTIAL_STRIDE;  // must not alias the scratch
+  CK(f16::stats::launch_summary(cfg(false), d_x, ld, N, d_status, row, scratch, grid));
+  CK(cudaMemcpyAsync(row_host, row, 74 * 8, cudaMemcpyDeviceToHost, D->stream));
   return F16_OK;
 }
 
@@ -1324,20 +1293,12 @@ static int step_stats_core(double* d_x, long long ld_x, const double* d_u, long 
   CK(D->b_sum.reserve(((size_t)grid * f16::stats::PARTIAL_STRIDE + (size_t)(n_rows > 0 ? n_rows : 1) * 74 + 8) * 8));
   double* scratch = (double*)D->b_sum.p;
   double* rows_dev = scratch + (size_t)grid * f16::stats::PARTIAL_STRIDE;
-  const bool smem = G.smem_tables && (N * (long long)snap_every >= 4096);
-  int done = 0, snap = 0;
-  while (done < K) {
-    const int k = (K - done) < snap_every ? (K - done) : snap_every;
-    CK(DISPATCH(launch_step, cfg(smem), tabs(), sel, d_x, ld_x, d_u, ld_u, N, k, dt, reinterpret_cast<const f16::LqrLaw*>(lqr),
-                d_status, nullptr));
-    done += k;
-    if (k == snap_every) {
-      int rc = enqueue_summary(d_x, ld_x, N, d_status, rows_dev + (size_t)snap * 74, scratch, grid);
-      if (rc != F16_OK) return rc;
-      snap++;
-    }
-  }
-  if (n_rows > 0) D2H(rows_host, rows_dev, (size_t)n_rows * 74 * 8);
+  const int rc = snapshot_steps(d_x, ld_x, d_u, ld_u, N, K, snap_every, dt, lqr, sel, d_status, [&](int j) -> int {
+    CK(f16::stats::launch_summary(cfg(false), d_x, ld_x, N, d_status, rows_dev + (size_t)j * 74, scratch, grid));
+    return F16_OK;
+  });
+  if (rc != F16_OK) return rc;
+  if (n_rows > 0) CK(cudaMemcpyAsync(rows_host, rows_dev, (size_t)n_rows * 74 * 8, cudaMemcpyDeviceToHost, D->stream));
   return F16_OK;
 }
 
@@ -1347,40 +1308,26 @@ int step_batch_stats_dev(double* x_soa, long long ld_x, const double* u_soa, lon
   std::lock_guard<std::mutex> lk(G_mu);
   int rc = ensure();
   if (rc != F16_OK) return rc;
-  if (N < 0 || K < 0 || snap_every < 1 || (N > 0 && (!x_soa || !u_soa || !status)) || ld_x < N || ld_u < N || !lqr_ok(lqr) ||
-      (!rows && K >= snap_every)) {
-    set_err("step_batch_stats_dev: bad argument");
-    return F16_ERR_ARG;
-  }
+  if (!stats_ok(x_soa, ld_x, u_soa, ld_u, N, K, snap_every, lqr, rows) || (N > 0 && !status)) return bad_arg("step_batch_stats_dev");
   rc = step_stats_core(x_soa, ld_x, u_soa, ld_u, N, K, snap_every, dt, lqr, sel_of(fi, fi_default, xcg, xcg_default), status, rows);
   if (rc != F16_OK) return rc;
   CK(cudaStreamSynchronize(D->stream));
   return F16_OK;
 }
 
-// aircraft [lo, lo + n_) of the caller's arrays on the context D; rows_out [K / snap_every][74] of this slice
-static int stats_host(double* x, const double* u, long long ld, long long lo, long long n_, int K, int snap_every, double dt,
+// aircraft [lo, lo + n) of the caller's arrays on the context D; rows_out [K / snap_every][74] of this slice.  The status slot
+// starts at 0: with K = 0 no step writes it.
+static int stats_host(double* x, const double* u, long long ld, long long lo, long long n, int K, int snap_every, double dt,
                       const f16_lqr_t* lqr, const unsigned char* fi, int fi_default, const double* xcg, double xcg_default,
                       double* rows_out, int* status) {
-  const size_t n = (size_t)n_;
-  CK(D->b_in.reserve(18 * n * 8));
-  CK(D->b_in2.reserve(4 * n * 8));
-  CK(D->b_st.reserve(n * 4));
-  const unsigned char* d_fi = nullptr;
-  const double* d_xcg = nullptr;
-  int rc = stage_sel(fi ? fi + lo : nullptr, xcg ? xcg + lo : nullptr, n_, &d_fi, &d_xcg);
-  if (rc != F16_OK) return rc;
-  CK(planes_h2d(D->b_in.p, x + lo, ld, n_, 18, D->stream));
-  CK(planes_h2d(D->b_in2.p, u + lo, ld, n_, 4, D->stream));
-  CK(cudaMemsetAsync(D->b_st.p, 0, n * 4, D->stream));
-  reserve_step_progress(n_);
-  rc = step_stats_core((double*)D->b_in.p, n_, (const double*)D->b_in2.p, n_, n_, K, snap_every, dt, lqr,
-                       sel_of(d_fi, fi_default, d_xcg, xcg_default), (int*)D->b_st.p, rows_out);
-  if (rc != F16_OK) return rc;
-  CK(planes_d2h(x + lo, ld, D->b_in.p, n_, 18, D->stream));
-  if (status) D2H(status + lo, D->b_st.p, n * 4);
-  CK(cudaStreamSynchronize(D->stream));
-  return F16_OK;
+  reserve_step_progress(n);
+  return run_pipeline(
+      {soa(x, INOUT, 8, 18), soa(u, IN, 8, 4), soa(fi, IN, 1), soa(xcg, IN, 8), soa(status, OUT, 4, 1, true)}, ld, lo, n,
+      one_chunk(n), false, [&](const Slots& p, long long m) {
+        CK(cudaMemsetAsync(p.i32(4), 0, (size_t)m * 4, D->stream));
+        return step_stats_core(p.f64(0), m, p.f64(1), m, m, K, snap_every, dt, lqr, sel_of(p.u8(2), fi_default, p.f64(3), xcg_default),
+                               p.i32(4), rows_out);
+      });
 }
 
 int step_batch_stats(double* x_soa, const double* u_soa, long long N, int K, int snap_every, double dt, const f16_lqr_t* lqr,
@@ -1388,97 +1335,53 @@ int step_batch_stats(double* x_soa, const double* u_soa, long long N, int K, int
   std::lock_guard<std::mutex> lk(G_mu);
   int rc = ensure();
   if (rc != F16_OK) return rc;
-  if (N < 0 || K < 0 || snap_every < 1 || (N > 0 && (!x_soa || !u_soa)) || !lqr_ok(lqr) || (!rows && K >= snap_every)) {
-    set_err("step_batch_stats: bad argument");
-    return F16_ERR_ARG;
-  }
-  const int n_rows = K / snap_every;
+  if (!stats_ok(x_soa, N, u_soa, N, N, K, snap_every, lqr, rows)) return bad_arg("step_batch_stats");
   if (N == 0) {  // an empty batch still has rows: count 0, min = +inf, max = -inf
-    CK(D->b_st.reserve(4));
-    rc = step_stats_core(nullptr, 0, nullptr, 0, 0, K, snap_every, dt, lqr, sel_of(nullptr, fi_default, nullptr, xcg_default),
-                         (int*)D->b_st.p, rows);
+    rc = step_stats_core(nullptr, 0, nullptr, 0, 0, K, snap_every, dt, lqr, sel_of(nullptr, fi_default, nullptr, xcg_default), nullptr,
+                         rows);
     if (rc != F16_OK) return rc;
     CK(cudaStreamSynchronize(D->stream));
     return F16_OK;
   }
-  try {
-    // every device context reduces its own slice; the per-slice rows are combined on the host (Chan's update, slice order)
-    const size_t parts = G.devs.size() > 1 ? device_spans(N, 16384).size() : 1;
-    if (parts <= 1) return stats_host(x_soa, u_soa, N, 0, N, K, snap_every, dt, lqr, fi, fi_default, xcg, xcg_default, rows, status);
-    std::vector<double> part((size_t)n_rows * 74 * parts);
-    const std::vector<Span> spans = device_spans(N, 16384);
-    rc = on_devices(N, 16384, [&](long long lo, long long n) {
-      size_t i = 0;
-      while (spans[i].lo != lo) i++;
-      return stats_host(x_soa, u_soa, N, lo, n, K, snap_every, dt, lqr, fi, fi_default, xcg, xcg_default,
-                        part.data() + i * (size_t)n_rows * 74, status);
-    });
-    if (rc != F16_OK) return rc;
-    for (int r = 0; r < n_rows; r++) {
-      double* dst = rows + (size_t)r * 74;
-      memcpy(dst, part.data() + (size_t)r * 74, 74 * 8);
-      for (size_t i = 1; i < parts; i++) merge_summary_row(dst, part.data() + (i * (size_t)n_rows + (size_t)r) * 74);
-    }
-    return F16_OK;
-  } catch (const std::exception& e) {
-    set_err("host resources: %s", e.what());
-    return F16_ERR_HOST;
-  }
+  return merged_rows(N, 16384, K / snap_every, rows, [&](long long lo, long long n, double* part) {
+    return stats_host(x_soa, u_soa, N, lo, n, K, snap_every, dt, lqr, fi, fi_default, xcg, xcg_default, part, status);
+  });
 }
 
 int state_summary_batch_dev(const double* x_soa, long long ld_x, long long N, const int* status, double* row) {
   std::lock_guard<std::mutex> lk(G_mu);
   int rc = ensure();
   if (rc != F16_OK) return rc;
-  if (N < 0 || !row || (N > 0 && !x_soa) || ld_x < N) { set_err("state_summary_batch_dev: bad argument"); return F16_ERR_ARG; }
-  return summary_common(x_soa, ld_x, N, status, row);
-}
-
-static int summary_host(const double* x, long long ld, long long lo, long long n_, const int* status, double* row) {
-  const size_t n = (size_t)n_;
-  CK(D->b_in.reserve((n ? 18 * n : 1) * 8));
-  if (n) CK(planes_h2d(D->b_in.p, x + lo, ld, n_, 18, D->stream));
-  const int* d_st = nullptr;
-  if (status && n) {
-    CK(D->b_st.reserve(n * 4));
-    H2D(D->b_st.p, status + lo, n * 4);
-    d_st = (const int*)D->b_st.p;
-  }
-  return summary_common((const double*)D->b_in.p, n_, n_, d_st, row);
+  if (!summary_ok(x_soa, ld_x, N, row)) return bad_arg("state_summary_batch_dev");
+  rc = summary_row(x_soa, ld_x, N, status, row);
+  if (rc != F16_OK) return rc;
+  CK(cudaStreamSynchronize(D->stream));
+  return F16_OK;
 }
 
 int state_summary_batch(const double* x_soa, long long N, const int* status, double* row) {
   std::lock_guard<std::mutex> lk(G_mu);
   int rc = ensure();
   if (rc != F16_OK) return rc;
-  if (N < 0 || !row || (N > 0 && !x_soa)) { set_err("state_summary_batch: bad argument"); return F16_ERR_ARG; }
-  try {
-    const std::vector<Span> spans = G.devs.size() > 1 ? device_spans(N, 65536) : std::vector<Span>();
-    if (spans.size() <= 1) return summary_host(x_soa, N, 0, N, status, row);
-    std::vector<double> part(74 * spans.size());
-    rc = on_devices(N, 65536, [&](long long lo, long long n) {
-      size_t i = 0;
-      while (spans[i].lo != lo) i++;
-      return summary_host(x_soa, N, lo, n, status, part.data() + 74 * i);
-    });
+  if (!summary_ok(x_soa, N, N, row)) return bad_arg("state_summary_batch");
+  if (N == 0) {  // the empty row
+    rc = summary_row(nullptr, 0, 0, nullptr, row);
     if (rc != F16_OK) return rc;
-    memcpy(row, part.data(), 74 * 8);
-    for (size_t i = 1; i < spans.size(); i++) merge_summary_row(row, part.data() + 74 * i);
+    CK(cudaStreamSynchronize(D->stream));
     return F16_OK;
-  } catch (const std::exception& e) {
-    set_err("host resources: %s", e.what());
-    return F16_ERR_HOST;
   }
+  return merged_rows(N, 65536, 1, row, [&](long long lo, long long n, double* part) {
+    return run_pipeline({soa(x_soa, IN, 8, 18), soa(status, IN, 4)}, N, lo, n, one_chunk(n), false,
+                        [&](const Slots& p, long long m) { return summary_row(p.f64(0), m, m, p.i32(1), part); });
+  });
 }
 
 // ---- between linearise and the LQR law: reduced model, zero-order hold, discrete LQR gain --------------------------------
-static bool dims_ok(int n, int m) { return n >= 1 && m >= 1 && n <= 18 && n + m <= 22; }
-
 int reduce_jacobian_batch_dev(const double* A, long long N, double* A_na, double* B_na) {
   std::lock_guard<std::mutex> lk(G_mu);
   int rc = ensure();
   if (rc != F16_OK) return rc;
-  if (N < 0 || (N > 0 && (!A || !A_na || !B_na))) { set_err("reduce_jacobian_batch_dev: bad argument"); return F16_ERR_ARG; }
+  if (!reduce_ok(A, N, A_na, B_na)) return bad_arg("reduce_jacobian_batch_dev");
   CK(f16::linalg::launch_reduce_jacobian(cfg(false), A, N, A_na, B_na));
   return F16_OK;
 }
@@ -1487,10 +1390,7 @@ int discretise_batch_dev(const double* A, const double* B, int n, int m, long lo
   std::lock_guard<std::mutex> lk(G_mu);
   int rc = ensure();
   if (rc != F16_OK) return rc;
-  if (N < 0 || !dims_ok(n, m) || !std::isfinite(dt) || (N > 0 && (!A || !B || !Ad || !Bd))) {
-    set_err("discretise_batch_dev: bad argument");
-    return F16_ERR_ARG;
-  }
+  if (!zoh_ok(A, B, n, m, N, dt, Ad, Bd)) return bad_arg("discretise_batch_dev");
   CK(f16::linalg::launch_zoh(cfg(false), A, B, n, m, N, dt, Ad, Bd));
   return F16_OK;
 }
@@ -1500,7 +1400,7 @@ int dlqr_batch_dev(const double* Ad, const double* Bd, const double* Q /* device
   std::lock_guard<std::mutex> lk(G_mu);
   int rc = ensure();
   if (rc != F16_OK) return rc;
-  if (N < 0 || !dims_ok(n, m) || (N > 0 && (!Ad || !Bd || !Q || !R || !K))) { set_err("dlqr_batch_dev: bad argument"); return F16_ERR_ARG; }
+  if (!dlqr_ok(Ad, Bd, Q, R, n, m, N, K)) return bad_arg("dlqr_batch_dev");
   CK(f16::linalg::launch_dlqr(cfg(false), Ad, Bd, Q, R, n, m, N, 64, 1e-15, K, P, info));
   return F16_OK;
 }
@@ -1509,41 +1409,33 @@ int reduce_jacobian_batch(const double* A, long long N, double* A_na, double* B_
   std::lock_guard<std::mutex> lk(G_mu);
   int rc = ensure();
   if (rc != F16_OK) return rc;
-  if (N < 0 || (N > 0 && (!A || !A_na || !B_na))) { set_err("reduce_jacobian_batch: bad argument"); return F16_ERR_ARG; }
+  if (!reduce_ok(A, N, A_na, B_na)) return bad_arg("reduce_jacobian_batch");
   if (N == 0) return F16_OK;
-  const size_t n = (size_t)N;
-  CK(D->b_l1.reserve(n * 324 * 8));
-  CK(D->b_l2.reserve(n * 81 * 8));
-  CK(D->b_l3.reserve(n * 27 * 8));
-  H2D(D->b_l1.p, A, n * 324 * 8);
-  CK(f16::linalg::launch_reduce_jacobian(cfg(false), (const double*)D->b_l1.p, N, (double*)D->b_l2.p, (double*)D->b_l3.p));
-  D2H(A_na, D->b_l2.p, n * 81 * 8);
-  D2H(B_na, D->b_l3.p, n * 27 * 8);
-  CK(cudaStreamSynchronize(D->stream));
-  return F16_OK;
+  return run_pipeline({aos(A, IN, 8, 324), aos(A_na, OUT, 8, 81), aos(B_na, OUT, 8, 27)}, N, 0, N, one_chunk(N), false,
+                      [&](const Slots& p, long long len) -> int {
+                        CK(f16::linalg::launch_reduce_jacobian(cfg(false), p.f64(0), len, p.f64(1), p.f64(2)));
+                        return F16_OK;
+                      });
 }
 
 int discretise_batch(const double* A, const double* B, int n, int m, long long N, double dt, double* Ad, double* Bd) {
   std::lock_guard<std::mutex> lk(G_mu);
   int rc = ensure();
   if (rc != F16_OK) return rc;
-  if (N < 0 || !dims_ok(n, m) || !std::isfinite(dt) || (N > 0 && (!A || !B || !Ad || !Bd))) {
-    set_err("discretise_batch: bad argument");
-    return F16_ERR_ARG;
-  }
+  if (!zoh_ok(A, B, n, m, N, dt, Ad, Bd)) return bad_arg("discretise_batch");
   if (N == 0) return F16_OK;
-  const size_t na = (size_t)N * n * n * 8, nb = (size_t)N * n * m * 8;
-  CK(D->b_l1.reserve(na));
-  CK(D->b_l2.reserve(nb));
-  CK(D->b_l3.reserve(na));
-  CK(D->b_l4.reserve(nb));
-  H2D(D->b_l1.p, A, na);
-  H2D(D->b_l2.p, B, nb);
-  CK(f16::linalg::launch_zoh(cfg(false), (const double*)D->b_l1.p, (const double*)D->b_l2.p, n, m, N, dt, (double*)D->b_l3.p,
-                             (double*)D->b_l4.p));
-  D2H(Ad, D->b_l3.p, na);
-  D2H(Bd, D->b_l4.p, nb);
-  CK(cudaStreamSynchronize(D->stream));
+  return run_pipeline({aos(A, IN, 8, n * n), aos(B, IN, 8, n * m), aos(Ad, OUT, 8, n * n), aos(Bd, OUT, 8, n * m)}, N, 0, N,
+                      one_chunk(N), false, [&](const Slots& p, long long len) -> int {
+                        CK(f16::linalg::launch_zoh(cfg(false), p.f64(0), p.f64(1), n, m, len, dt, p.f64(2), p.f64(3)));
+                        return F16_OK;
+                      });
+}
+
+// dlqr_batch and lqr_gain_batch: Q [n][n], R [m][m], shared by all systems, copied to b_qr on D->stream
+static int stage_qr(const double* Q, const double* R, int n, int m) {
+  CK(D->b_qr.reserve((size_t)(n * n + m * m) * 8));
+  CK(cudaMemcpyAsync(D->b_qr.p, Q, (size_t)n * n * 8, cudaMemcpyHostToDevice, D->stream));
+  CK(cudaMemcpyAsync((double*)D->b_qr.p + n * n, R, (size_t)m * m * 8, cudaMemcpyHostToDevice, D->stream));
   return F16_OK;
 }
 
@@ -1552,121 +1444,78 @@ int dlqr_batch(const double* Ad, const double* Bd, const double* Q, const double
   std::lock_guard<std::mutex> lk(G_mu);
   int rc = ensure();
   if (rc != F16_OK) return rc;
-  if (N < 0 || !dims_ok(n, m) || (N > 0 && (!Ad || !Bd || !Q || !R || !K))) { set_err("dlqr_batch: bad argument"); return F16_ERR_ARG; }
+  if (!dlqr_ok(Ad, Bd, Q, R, n, m, N, K)) return bad_arg("dlqr_batch");
   if (N == 0) return F16_OK;
-  const size_t na = (size_t)N * n * n * 8, nb = (size_t)N * n * m * 8, nk = (size_t)N * m * n * 8;
-  CK(D->b_l1.reserve(na));
-  CK(D->b_l2.reserve(nb));
-  CK(D->b_l3.reserve(nk));
-  CK(D->b_l4.reserve(na));
-  CK(D->b_l5.reserve((size_t)(n * n + m * m) * 8));
-  CK(D->b_st.reserve((size_t)N * 8));
-  H2D(D->b_l1.p, Ad, na);
-  H2D(D->b_l2.p, Bd, nb);
-  double* dQ = (double*)D->b_l5.p;
-  H2D(dQ, Q, (size_t)n * n * 8);
-  H2D(dQ + n * n, R, (size_t)m * m * 8);
-  CK(f16::linalg::launch_dlqr(cfg(false), (const double*)D->b_l1.p, (const double*)D->b_l2.p, dQ, dQ + n * n, n, m, N, 64, 1e-15,
-                              (double*)D->b_l3.p, P ? (double*)D->b_l4.p : nullptr, info ? (int*)D->b_st.p : nullptr));
-  D2H(K, D->b_l3.p, nk);
-  if (P) D2H(P, D->b_l4.p, na);
-  if (info) D2H(info, D->b_st.p, (size_t)N * 8);
-  CK(cudaStreamSynchronize(D->stream));
-  return F16_OK;
+  return run_pipeline({aos(Ad, IN, 8, n * n), aos(Bd, IN, 8, n * m), aos(K, OUT, 8, m * n), aos(P, OUT, 8, n * n), aos(info, OUT, 4, 2)},
+                      N, 0, N, one_chunk(N), false, [&](const Slots& p, long long len) -> int {
+                        const int st = stage_qr(Q, R, n, m);
+                        if (st != F16_OK) return st;
+                        const double* q = (const double*)D->b_qr.p;
+                        CK(f16::linalg::launch_dlqr(cfg(false), p.f64(0), p.f64(1), q, q + n * n, n, m, len, 64, 1e-15, p.f64(2),
+                                                    p.f64(3), p.i32(4)));
+                        return F16_OK;
+                      });
 }
 
 // F16._calc_LQR_gain (env.py:344-358) for N operating points, every stage on the device:
 // forward linearise -> reduced 9-state / 3-input model -> cont2discrete(dt) -> K = -dlqr(Ad, Bd, C'C = I, R = I)
-static int lqr_gain_impl(const double* x_soa, const double* u_soa, long long N, double dt, double* K /* [N][3][9] */, const unsigned char* fi,
-                         int fi_default, const double* xcg, double xcg_default, int* status) {
-  int rc = F16_OK;
-  if (N < 0 || (N > 0 && (!x_soa || !u_soa || !K)) || !(dt > 0)) { set_err("lqr_gain_batch: bad argument"); return F16_ERR_ARG; }
-  if (N == 0) return F16_OK;
-  const size_t n = (size_t)N;
-  CK(D->b_in.reserve(18 * n * 8));
-  CK(D->b_in2.reserve(4 * n * 8));
-  CK(D->b_a.reserve(324 * n * 8));
-  CK(D->b_b.reserve(72 * n * 8));
-  CK(D->b_st.reserve(n * 8));
-  CK(D->b_st2.reserve(n * 4));
-  CK(D->b_l1.reserve(n * 81 * 8));
-  CK(D->b_l2.reserve(n * 27 * 8));
-  CK(D->b_l3.reserve(n * 81 * 8));
-  CK(D->b_l4.reserve(n * 27 * 8));
-  CK(D->b_l5.reserve((81 + 9) * 8));
-  CK(D->b_out.reserve(n * 27 * 8));
-  const unsigned char* d_fi;
-  const double* d_xcg;
-  if ((rc = stage_sel(fi, xcg, N, &d_fi, &d_xcg)) != F16_OK) return rc;
-  // the reduced model evaluates at X with the actuator states replaced by the inputs (env.py:175-177)
-  std::vector<double> xs(x_soa, x_soa + 18 * n);
-  for (int k = 0; k < 3; k++) memcpy(&xs[(13 + k) * n], &u_soa[(1 + k) * n], n * 8);
-  double QR[90];
-  for (int i = 0; i < 81; i++) QR[i] = (i % 10 == 0) ? 1.0 : 0.0;
-  for (int i = 0; i < 9; i++) QR[81 + i] = (i % 4 == 0) ? 1.0 : 0.0;
-  CK(cudaMemcpyAsync(D->b_in.p, xs.data(), 18 * n * 8, cudaMemcpyHostToDevice, D->stream));
-  CK(cudaStreamSynchronize(D->stream));  // xs is a temporary
-  H2D(D->b_in2.p, u_soa, 4 * n * 8);
-  CK(cudaMemcpyAsync(D->b_l5.p, QR, sizeof QR, cudaMemcpyHostToDevice, D->stream));
-  CK(cudaStreamSynchronize(D->stream));  // QR is a temporary
-  CK(f16::strict::launch_linearise(cfg(true), tabs(), sel_of(d_fi, fi_default, d_xcg, xcg_default), (const double*)D->b_in.p, N,
-                                   (const double*)D->b_in2.p, N, N, 1e-5, F16_FD_FORWARD, (double*)D->b_a.p, (double*)D->b_b.p,
-                                   (int*)D->b_st2.p));
-  CK(f16::linalg::launch_reduce_jacobian(cfg(false), (const double*)D->b_a.p, N, (double*)D->b_l1.p, (double*)D->b_l2.p));
-  CK(f16::linalg::launch_zoh(cfg(false), (const double*)D->b_l1.p, (const double*)D->b_l2.p, 9, 3, N, dt, (double*)D->b_l3.p,
-                             (double*)D->b_l4.p));
-  double* dQ = (double*)D->b_l5.p;
-  CK(f16::linalg::launch_dlqr(cfg(false), (const double*)D->b_l3.p, (const double*)D->b_l4.p, dQ, dQ + 81, 9, 3, N, 64, 1e-15,
-                              (double*)D->b_out.p, nullptr, (int*)D->b_st.p));
-  std::vector<double> k(27 * n);
-  std::vector<int> info(2 * n), st(n);
-  CK(cudaMemcpyAsync(k.data(), D->b_out.p, 27 * n * 8, cudaMemcpyDeviceToHost, D->stream));
-  CK(cudaMemcpyAsync(info.data(), D->b_st.p, n * 8, cudaMemcpyDeviceToHost, D->stream));
-  CK(cudaMemcpyAsync(st.data(), D->b_st2.p, n * 4, cudaMemcpyDeviceToHost, D->stream));
-  CK(cudaStreamSynchronize(D->stream));
-  for (size_t i = 0; i < 27 * n; i++) K[i] = -k[i];  // env.py:356: K = - dlqr(A, B, Q, R)
-  if (status)
-    for (size_t i = 0; i < n; i++) status[i] = st[i] ? st[i] : (info[2 * i] < 0 ? (int)F16_ST_NAN : 0);
-  return F16_OK;
-}
-
 int lqr_gain_batch(const double* x_soa, const double* u_soa, long long N, double dt, double* K /* [N][3][9] */, const unsigned char* fi,
                    int fi_default, const double* xcg, double xcg_default, int* status) {
   std::lock_guard<std::mutex> lk(G_mu);
   int rc = ensure();
   if (rc != F16_OK) return rc;
-  try {  // the host-side staging vectors must not throw through the C ABI
-    return lqr_gain_impl(x_soa, u_soa, N, dt, K, fi, fi_default, xcg, xcg_default, status);
+  if (N < 0 || (N > 0 && (!x_soa || !u_soa || !K)) || !(dt > 0)) return bad_arg("lqr_gain_batch");
+  if (N == 0) return F16_OK;
+  static const double kI9[81] = {1, 0, 0, 0, 0, 0, 0, 0, 0, 0, 1, 0, 0, 0, 0, 0, 0, 0, 0, 0, 1, 0, 0, 0, 0, 0, 0,
+                                 0, 0, 0, 1, 0, 0, 0, 0, 0, 0, 0, 0, 0, 1, 0, 0, 0, 0, 0, 0, 0, 0, 0, 1, 0, 0, 0,
+                                 0, 0, 0, 0, 0, 0, 1, 0, 0, 0, 0, 0, 0, 0, 0, 0, 1, 0, 0, 0, 0, 0, 0, 0, 0, 0, 1};
+  static const double kI3[9] = {1, 0, 0, 0, 1, 0, 0, 0, 1};
+  const size_t n = (size_t)N;
+  try {  // the host copy of the dlqr info must not throw through the C ABI
+    std::vector<int> info(status ? 2 * n : 0);
+    rc = run_pipeline(
+        {soa(x_soa, IN, 8, 18), soa(u_soa, IN, 8, 4), soa(fi, IN, 1), soa(xcg, IN, 8), aos(K, OUT, 8, 27),
+         soa(status, OUT, 4, 1, true), aos(status ? info.data() : nullptr, OUT, 4, 2, true), aos(nullptr, OUT, 8, 324, true),
+         aos(nullptr, OUT, 8, 72, true), aos(nullptr, OUT, 8, 81, true), aos(nullptr, OUT, 8, 27, true),
+         aos(nullptr, OUT, 8, 81, true), aos(nullptr, OUT, 8, 27, true)},
+        N, 0, N, one_chunk(N), false, [&](const Slots& p, long long len) -> int {
+          // the reduced model evaluates at X with the actuator states replaced by the inputs (env.py:175-177)
+          CK(cudaMemcpyAsync(p.f64(0) + 13 * len, p.f64(1) + len, 3 * (size_t)len * 8, cudaMemcpyDeviceToDevice, D->stream));
+          const int st = stage_qr(kI9, kI3, 9, 3);
+          if (st != F16_OK) return st;
+          const double* q = (const double*)D->b_qr.p;
+          CK(f16::strict::launch_linearise(cfg(true), tabs(), sel_of(p.u8(2), fi_default, p.f64(3), xcg_default), p.f64(0), len,
+                                           p.f64(1), len, len, 1e-5, F16_FD_FORWARD, p.f64(7), p.f64(8), p.i32(5)));
+          CK(f16::linalg::launch_reduce_jacobian(cfg(false), p.f64(7), len, p.f64(9), p.f64(10)));
+          CK(f16::linalg::launch_zoh(cfg(false), p.f64(9), p.f64(10), 9, 3, len, dt, p.f64(11), p.f64(12)));
+          CK(f16::linalg::launch_dlqr(cfg(false), p.f64(11), p.f64(12), q, q + 81, 9, 3, len, 64, 1e-15, p.f64(4), nullptr, p.i32(6)));
+          return F16_OK;
+        });
+    if (rc != F16_OK) return rc;
+    for (size_t i = 0; i < 27 * n; i++) K[i] = -K[i];  // env.py:356: K = - dlqr(A, B, Q, R)
+    if (status)
+      for (size_t i = 0; i < n; i++) status[i] = status[i] ? status[i] : (info[2 * i] < 0 ? (int)F16_ST_NAN : 0);
+    return F16_OK;
   } catch (const std::exception& e) {
-    cudaStreamSynchronize(D->stream);
     set_err("lqr_gain_batch: host resources: %s", e.what());
     return F16_ERR_HOST;
   }
 }
 
-// ---- parity probes -----------------------------------------------------------------------------------------------
+// ---- parity probes: one chunk on the current context ----------------------------------------------------------------
 int f16_hifi_probe(const double* alpha_deg, const double* beta_deg, const double* el, long long N, double* coef, int* cells,
                    int* status) {
   std::lock_guard<std::mutex> lk(G_mu);
   int rc = ensure();
   if (rc != F16_OK) return rc;
-  if (N <= 0 || !alpha_deg || !beta_deg || !el || !coef || !cells) { set_err("f16_hifi_probe: bad argument"); return F16_ERR_ARG; }
-  const size_t n = (size_t)N;
-  CK(D->b_in.reserve(3 * n * 8));
-  CK(D->b_out.reserve(44 * n * 8));
-  CK(D->b_st.reserve(n * 4));
-  CK(D->b_st2.reserve(8 * n * 4));
-  double* d = (double*)D->b_in.p;
-  H2D(d, alpha_deg, n * 8);
-  H2D(d + n, beta_deg, n * 8);
-  H2D(d + 2 * n, el, n * 8);
-  CK(DISPATCH(launch_hifi_probe, cfg(false), tabs(), d, d + n, d + 2 * n, N, (double*)D->b_out.p, (int*)D->b_st2.p,
-              (int*)D->b_st.p));
-  D2H(coef, D->b_out.p, 44 * n * 8);
-  D2H(cells, D->b_st2.p, 8 * n * 4);
-  if (status) D2H(status, D->b_st.p, n * 4);
-  CK(cudaStreamSynchronize(D->stream));
-  return F16_OK;
+  if (N <= 0 || !alpha_deg || !beta_deg || !el || !coef || !cells) return bad_arg("f16_hifi_probe");
+  return run_pipeline({soa(alpha_deg, IN, 8), soa(beta_deg, IN, 8), soa(el, IN, 8), soa(coef, OUT, 8, 44), soa(cells, OUT, 4, 8),
+                       soa(status, OUT, 4, 1, true)},
+                      N, 0, N, one_chunk(N), false, [&](const Slots& p, long long m) -> int {
+                        CK(DISPATCH(launch_hifi_probe, cfg(false), tabs(), p.f64(0), p.f64(1), p.f64(2), m, p.f64(3), p.i32(4),
+                                    p.i32(5)));
+                        return F16_OK;
+                      });
 }
 
 int f16_fast_probe(const double* alpha_deg, const double* beta_deg, const double* el, long long N, double* coef, int* cells,
@@ -1674,24 +1523,14 @@ int f16_fast_probe(const double* alpha_deg, const double* beta_deg, const double
   std::lock_guard<std::mutex> lk(G_mu);
   int rc = ensure();
   if (rc != F16_OK) return rc;
-  if (N <= 0 || !alpha_deg || !beta_deg || !el || !coef || !cells || !lam) { set_err("f16_fast_probe: bad argument"); return F16_ERR_ARG; }
-  const size_t n = (size_t)N;
-  CK(D->b_in.reserve(3 * n * 8));
-  CK(D->b_out.reserve(48 * n * 8));
-  CK(D->b_st.reserve(n * 4));
-  CK(D->b_st2.reserve(4 * n * 4));
-  double* d = (double*)D->b_in.p;
-  H2D(d, alpha_deg, n * 8);
-  H2D(d + n, beta_deg, n * 8);
-  H2D(d + 2 * n, el, n * 8);
-  double* o = (double*)D->b_out.p;
-  CK(f16::fast::launch_fast_probe(cfg(false), tabs(), d, d + n, d + 2 * n, N, o, (int*)D->b_st2.p, o + 44 * n, (int*)D->b_st.p));
-  D2H(coef, o, 44 * n * 8);
-  D2H(lam, o + 44 * n, 4 * n * 8);
-  D2H(cells, D->b_st2.p, 4 * n * 4);
-  if (status) D2H(status, D->b_st.p, n * 4);
-  CK(cudaStreamSynchronize(D->stream));
-  return F16_OK;
+  if (N <= 0 || !alpha_deg || !beta_deg || !el || !coef || !cells || !lam) return bad_arg("f16_fast_probe");
+  return run_pipeline({soa(alpha_deg, IN, 8), soa(beta_deg, IN, 8), soa(el, IN, 8), soa(coef, OUT, 8, 44), soa(cells, OUT, 4, 4),
+                       soa(lam, OUT, 8, 4), soa(status, OUT, 4, 1, true)},
+                      N, 0, N, one_chunk(N), false, [&](const Slots& p, long long m) -> int {
+                        CK(f16::fast::launch_fast_probe(cfg(false), tabs(), p.f64(0), p.f64(1), p.f64(2), m, p.f64(3), p.i32(4),
+                                                        p.f64(5), p.i32(6)));
+                        return F16_OK;
+                      });
 }
 
 int f16_lofi_probe(const double* alpha_deg, const double* beta_deg, const double* el, const double* dail,
@@ -1699,54 +1538,38 @@ int f16_lofi_probe(const double* alpha_deg, const double* beta_deg, const double
   std::lock_guard<std::mutex> lk(G_mu);
   int rc = ensure();
   if (rc != F16_OK) return rc;
-  if (N <= 0 || !alpha_deg || !beta_deg || !el || !dail || !drud || !out) { set_err("f16_lofi_probe: bad argument"); return F16_ERR_ARG; }
-  const size_t n = (size_t)N;
-  CK(D->b_in.reserve(5 * n * 8));
-  CK(D->b_out.reserve(19 * n * 8));
-  double* d = (double*)D->b_in.p;
-  H2D(d, alpha_deg, n * 8);
-  H2D(d + n, beta_deg, n * 8);
-  H2D(d + 2 * n, el, n * 8);
-  H2D(d + 3 * n, dail, n * 8);
-  H2D(d + 4 * n, drud, n * 8);
-  CK(DISPATCH(launch_lofi_probe, cfg(false), tabs(), d, d + n, d + 2 * n, d + 3 * n, d + 4 * n, N, (double*)D->b_out.p));
-  D2H(out, D->b_out.p, 19 * n * 8);
-  CK(cudaStreamSynchronize(D->stream));
-  return F16_OK;
+  if (N <= 0 || !alpha_deg || !beta_deg || !el || !dail || !drud || !out) return bad_arg("f16_lofi_probe");
+  return run_pipeline({soa(alpha_deg, IN, 8), soa(beta_deg, IN, 8), soa(el, IN, 8), soa(dail, IN, 8), soa(drud, IN, 8),
+                       soa(out, OUT, 8, 19)},
+                      N, 0, N, one_chunk(N), false, [&](const Slots& p, long long m) -> int {
+                        CK(DISPATCH(launch_lofi_probe, cfg(false), tabs(), p.f64(0), p.f64(1), p.f64(2), p.f64(3), p.f64(4), m,
+                                    p.f64(5)));
+                        return F16_OK;
+                      });
 }
 
 int f16_div_probe(const double* a, const double* b, long long N, double* out) {
   std::lock_guard<std::mutex> lk(G_mu);
   int rc = ensure();
   if (rc != F16_OK) return rc;
-  if (N <= 0 || !a || !b || !out) { set_err("f16_div_probe: bad argument"); return F16_ERR_ARG; }
-  const size_t n = (size_t)N;
-  CK(D->b_in.reserve(2 * n * 8));
-  CK(D->b_out.reserve(3 * n * 8));
-  double* d = (double*)D->b_in.p;
-  H2D(d, a, n * 8);
-  H2D(d + n, b, n * 8);
-  CK(f16::strict::launch_div_probe(cfg(false), d, d + n, N, (double*)D->b_out.p));  // always the strict build's helpers
-  D2H(out, D->b_out.p, 3 * n * 8);
-  CK(cudaStreamSynchronize(D->stream));
-  return F16_OK;
+  if (N <= 0 || !a || !b || !out) return bad_arg("f16_div_probe");
+  return run_pipeline({soa(a, IN, 8), soa(b, IN, 8), soa(out, OUT, 8, 3)}, N, 0, N, one_chunk(N), false,
+                      [&](const Slots& p, long long m) -> int {
+                        CK(f16::strict::launch_div_probe(cfg(false), p.f64(0), p.f64(1), m, p.f64(2)));  // always the strict build's
+                        return F16_OK;
+                      });
 }
 
 int atmos_batch(const double* alt, const double* vt, long long N, double* coeff_soa) {
   std::lock_guard<std::mutex> lk(G_mu);
   int rc = ensure();
   if (rc != F16_OK) return rc;
-  if (N <= 0 || !alt || !vt || !coeff_soa) { set_err("atmos_batch: bad argument"); return F16_ERR_ARG; }
-  const size_t n = (size_t)N;
-  CK(D->b_in.reserve(2 * n * 8));
-  CK(D->b_out.reserve(3 * n * 8));
-  double* d = (double*)D->b_in.p;
-  H2D(d, alt, n * 8);
-  H2D(d + n, vt, n * 8);
-  CK(DISPATCH(launch_atmos, cfg(false), d, d + n, N, (double*)D->b_out.p));
-  D2H(coeff_soa, D->b_out.p, 3 * n * 8);
-  CK(cudaStreamSynchronize(D->stream));
-  return F16_OK;
+  if (N <= 0 || !alt || !vt || !coeff_soa) return bad_arg("atmos_batch");
+  return run_pipeline({soa(alt, IN, 8), soa(vt, IN, 8), soa(coeff_soa, OUT, 8, 3)}, N, 0, N, one_chunk(N), false,
+                      [&](const Slots& p, long long m) -> int {
+                        CK(DISPATCH(launch_atmos, cfg(false), p.f64(0), p.f64(1), m, p.f64(2)));
+                        return F16_OK;
+                      });
 }
 
 // ---- memory / timing helpers ------------------------------------------------------------------------------------------
@@ -1830,14 +1653,14 @@ int f16_measure_fp64_peak(double ms, double* tflops) {
   std::lock_guard<std::mutex> lk(G_mu);
   int rc = ensure();
   if (rc != F16_OK) return rc;
-  CK(D->b_st.reserve(64));
+  CK(D->b_flush.reserve(64));
   double flops = 0;
   float t = 0;
   long long iters = 2000;
   // calibrate, then run for about `ms`
   for (int pass = 0; pass < 2; pass++) {
     CK(cudaEventRecord(D->ev0, D->stream));
-    CK(f16::launch_dfma_peak(D->stream, D->sm_count, iters, (double*)D->b_st.p, &flops));
+    CK(f16::launch_dfma_peak(D->stream, D->sm_count, iters, (double*)D->b_flush.p, &flops));
     ++D->launches;
     CK(cudaEventRecord(D->ev1, D->stream));
     CK(cudaEventSynchronize(D->ev1));

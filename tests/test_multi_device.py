@@ -303,3 +303,128 @@ def test_entry_points_from_concurrent_host_threads(f16):
         assert not bad, bad
     finally:
         f16.lib.f16_set_math_mode(prev)
+
+
+# ---- argument checks --------------------------------------------------------------------------------------------------
+# Every host-buffer and *_dev entry point (the linalg calls: tests/test_linalg.py) as (arguments, pointers that must not be
+# NULL when N > 0, further rejected values, what N = 0 does).  Array arguments are ("f8" | "i4" | "u1", count) and are filled with
+# canaries; a _dev entry point gets device copies of them, except for the ("host", ...) ones, which the ABI takes on the host.
+def _sel(n):
+    return [("fi", ("u1", n)), ("fi_default", 1), ("xcg", ("f8", n)), ("xcg_default", 0.25)]
+
+
+_BAD_LAWS = [{"lqr": ("law", 19, 0)}, {"lqr": ("law", -1, 0)}, {"lqr": ("law", 1, 18)}, {"lqr": ("law", 1, -1)}]
+_STEP_BAD = [{"K": -1}] + _BAD_LAWS
+_SNAP_BAD = _STEP_BAD + [{"snap_every": 0}]
+_LIN_BAD = [{"scheme": 2}, {"scheme": -1}, {"eps": 1e-13}, {"eps": 2e3}, {"eps": float("nan")}]
+_TRIM_BAD = [{"tol": -1.0}, {"tol": float("nan")}, {"maxiter": 0}]
+_ENTRY = {
+    "Nlplant_batch": (lambda n: [("xu", ("f8", 17 * n)), ("xdot", ("f8", 18 * n))] + _sel(n) + [("N", n), ("status", ("i4", n))],
+                      ["xu", "xdot"], [], "ok"),
+    "calc_xdot_batch": (lambda n: [("x", ("f8", 18 * n)), ("u", ("f8", 4 * n)), ("xdot", ("f8", 18 * n))] + _sel(n) +
+                        [("N", n), ("status", ("i4", n))], ["x", "u", "xdot"], [], "ok"),
+    "step_batch": (lambda n: [("x", ("f8", 18 * n)), ("u", ("f8", 4 * n)), ("N", n), ("K", 2), ("dt", 1e-3), ("lqr", None)] + _sel(n) +
+                   [("status", ("i4", n)), ("steps", ("i4", n))], ["x", "u"], _STEP_BAD, "ok"),
+    "step_batch_traj": (lambda n: [("x", ("f8", 18 * n)), ("u", ("f8", 4 * n)), ("N", n), ("K", 4), ("snap_every", 2), ("dt", 1e-3),
+                                   ("lqr", None)] + _sel(n) + [("traj", ("f8", 2 * 18 * n)), ("status", ("i4", n))],
+                        ["x", "u", "traj"], _SNAP_BAD, "ok"),
+    "linearise_batch": (lambda n: [("x", ("f8", 18 * n)), ("u", ("f8", 4 * n)), ("N", n), ("eps", 1e-5), ("scheme", 0),
+                                   ("A", ("f8", 324 * n)), ("B", ("f8", 72 * n))] + _sel(n) + [("status", ("i4", n))],
+                        ["x", "u", "A", "B"], _LIN_BAD, "ok"),
+    "trim_batch": (lambda n: [("h", ("f8", n)), ("V", ("f8", n)), ("N", n), ("tol", 1e-10), ("maxiter", 100), ("ux0", None),
+                              ("x_trim", ("f8", 18 * n)), ("info", ("f8", 4 * n))] + _sel(n) + [("status", ("i4", n))],
+                   ["h", "V", "x_trim"], _TRIM_BAD, "ok"),
+    "step_batch_stats": (lambda n: [("x", ("f8", 18 * n)), ("u", ("f8", 4 * n)), ("N", n), ("K", 4), ("snap_every", 2), ("dt", 1e-3),
+                                    ("lqr", None)] + _sel(n) + [("rows", ("f8", 2 * 74)), ("status", ("i4", n))],
+                         ["x", "u", "rows"], _SNAP_BAD, "rows"),
+    "state_summary_batch": (lambda n: [("x", ("f8", 18 * n)), ("N", n), ("status", ("i4", n)), ("row", ("f8", 74))],
+                            ["x", "row"], [], "rows"),
+    "lqr_gain_batch": (lambda n: [("x", ("f8", 18 * n)), ("u", ("f8", 4 * n)), ("N", n), ("dt", 0.02), ("K", ("f8", 27 * n))] +
+                       _sel(n) + [("status", ("i4", n))], ["x", "u", "K"], [{"dt": 0.0}, {"dt": float("nan")}], "ok"),
+    "f16_hifi_probe": (lambda n: [("a", ("f8", n)), ("b", ("f8", n)), ("el", ("f8", n)), ("N", n), ("coef", ("f8", 44 * n)),
+                                  ("cells", ("i4", 8 * n)), ("status", ("i4", n))], ["a", "b", "el", "coef", "cells"], [], "arg"),
+    "f16_fast_probe": (lambda n: [("a", ("f8", n)), ("b", ("f8", n)), ("el", ("f8", n)), ("N", n), ("coef", ("f8", 44 * n)),
+                                  ("cells", ("i4", 4 * n)), ("lam", ("f8", 4 * n)), ("status", ("i4", n))],
+                       ["a", "b", "el", "coef", "cells", "lam"], [], "arg"),
+    "f16_lofi_probe": (lambda n: [("a", ("f8", n)), ("b", ("f8", n)), ("el", ("f8", n)), ("dail", ("f8", n)), ("drud", ("f8", n)),
+                                  ("N", n), ("out", ("f8", 19 * n))], ["a", "b", "el", "dail", "drud", "out"], [], "arg"),
+    "f16_div_probe": (lambda n: [("a", ("f8", n)), ("b", ("f8", n)), ("N", n), ("out", ("f8", 3 * n))], ["a", "b", "out"], [], "arg"),
+    "atmos_batch": (lambda n: [("alt", ("f8", n)), ("vt", ("f8", n)), ("N", n), ("coeff", ("f8", 3 * n))], ["alt", "vt", "coeff"],
+                    [], "arg"),
+    "Nlplant_batch_dev": (lambda n: [("xu", ("f8", 17 * n)), ("ld_in", n), ("xdot", ("f8", 18 * n)), ("ld_out", n)] + _sel(n) +
+                          [("N", n), ("status", ("i4", n))], ["xu", "xdot"], [{"ld_in": 63}, {"ld_out": 63}], "ok"),
+    "calc_xdot_batch_dev": (lambda n: [("x", ("f8", 18 * n)), ("ld_x", n), ("u", ("f8", 4 * n)), ("ld_u", n), ("xdot", ("f8", 18 * n)),
+                                       ("ld_out", n)] + _sel(n) + [("N", n), ("status", ("i4", n))],
+                            ["x", "u", "xdot"], [{"ld_x": 63}, {"ld_u": 63}, {"ld_out": 63}], "ok"),
+    "step_batch_dev": (lambda n: [("x", ("f8", 18 * n)), ("ld_x", n), ("u", ("f8", 4 * n)), ("ld_u", n), ("N", n), ("K", 2),
+                                  ("dt", 1e-3), ("lqr", None)] + _sel(n) + [("status", ("i4", n)), ("steps", ("i4", n))],
+                       ["x", "u"], _STEP_BAD + [{"ld_x": 63}, {"ld_u": 63}], "ok"),
+    "linearise_batch_dev": (lambda n: [("x", ("f8", 18 * n)), ("ld_x", n), ("u", ("f8", 4 * n)), ("ld_u", n), ("N", n), ("eps", 1e-5),
+                                       ("scheme", 0), ("A", ("f8", 324 * n)), ("B", ("f8", 72 * n))] + _sel(n) +
+                            [("status", ("i4", n))], ["x", "u", "A", "B"], _LIN_BAD + [{"ld_x": 63}, {"ld_u": 63}], "ok"),
+    "trim_batch_dev": (lambda n: [("h", ("f8", n)), ("V", ("f8", n)), ("N", n), ("tol", 1e-10), ("maxiter", 100), ("ux0", None),
+                                  ("x_trim", ("f8", 18 * n)), ("ld_x", n), ("info", ("f8", 4 * n)), ("ld_info", n)] + _sel(n) +
+                       [("status", ("i4", n))], ["h", "V", "x_trim"], _TRIM_BAD + [{"ld_x": 63}, {"ld_info": 63}], "ok"),
+    "state_summary_batch_dev": (lambda n: [("x", ("f8", 18 * n)), ("ld_x", n), ("N", n), ("status", ("i4", n)),
+                                           ("row", ("host", "f8", 74))], ["x", "row"], [{"ld_x": 63}], "rows"),
+    "step_batch_stats_dev": (lambda n: [("x", ("f8", 18 * n)), ("ld_x", n), ("u", ("f8", 4 * n)), ("ld_u", n), ("N", n), ("K", 4),
+                                        ("snap_every", 2), ("dt", 1e-3), ("lqr", None)] + _sel(n) +
+                             [("rows", ("host", "f8", 2 * 74)), ("status", ("i4", n))],
+                             ["x", "u", "rows", "status"], _SNAP_BAD + [{"ld_x": 63}, {"ld_u": 63}], "rows"),
+}
+
+
+@pytest.mark.parametrize("name", sorted(_ENTRY))
+def test_argument_checks(f16, name):
+    """Each rejected argument gives F16_ERR_ARG, names the entry point in f16_last_error() and leaves every array as it was.
+    N = 0 is F16_OK and touches nothing, except that the statistics calls write their empty rows and the probes reject it."""
+    L = f16.lib
+    args_of, nulls, bad, empty = _ENTRY[name]
+    fn, on_dev, n = getattr(L, name), name.endswith("_dev"), 64
+    fill = {"f8": -1.2345678901234567e+300, "i4": 0x5A5A5A5A, "u1": 0xA5}
+
+    def call(**over):
+        arrays, vals, laws = {}, [], []
+        for k, v in args_of(n):
+            v = over.get(k, v)
+            if isinstance(v, tuple) and v[0] == "law":
+                laws.append(f16.LqrLaw())
+                laws[-1].n_sel, laws[-1].sel[0] = v[1], v[2]
+                v = ctypes.byref(laws[-1])
+            elif isinstance(v, tuple):
+                host = v[0] == "host"
+                kind, count = v[-2:]
+                a = np.full(count, fill[kind], dtype={"f8": np.float64, "i4": np.int32, "u1": np.uint8}[kind])
+                p = a.ctypes.data
+                if on_dev and not host:
+                    p = L.f16_dev_alloc(a.nbytes)
+                    assert p and L.f16_memcpy_h2d(p, a.ctypes.data, a.nbytes) == 0
+                arrays[k] = (a, p if on_dev and not host else None)
+                v = ctypes.cast(ctypes.c_void_p(p), ctypes.POINTER(np.ctypeslib.as_ctypes_type(a.dtype)))
+            vals.append(v)
+        rc = fn(*vals)
+        assert L.f16_sync() == 0
+        now = {}
+        for k, (a, p) in arrays.items():
+            b = a.copy()
+            if p is not None:
+                assert L.f16_memcpy_d2h(b.ctypes.data, p, b.nbytes) == 0
+                L.f16_dev_free(p)
+            now[k] = (a, b)
+        return rc, now
+
+    rejections = [{k: None} for k in nulls] + [{"N": -1}] + bad
+    for over in rejections:
+        rc, arrays = call(**over)
+        assert rc == -3, (name, over, rc)
+        assert name.encode() in L.f16_last_error(), (name, over, L.f16_last_error())
+        for k, (a, b) in arrays.items():
+            assert np.array_equal(a, b), (name, over, k)
+    rc, arrays = call(N=0)
+    assert rc == (-3 if empty == "arg" else 0), (name, rc)
+    for k, (a, b) in arrays.items():
+        if empty == "rows" and k in ("row", "rows"):
+            rows = b.reshape(-1, 74)
+            assert np.all(rows[:, :2] == 0) and np.all(rows[:, 2:20] == np.inf) and np.all(rows[:, 20:38] == -np.inf), name
+        else:
+            assert np.array_equal(a, b), (name, k)
