@@ -284,34 +284,50 @@ f16::BatchSel sel_of(const unsigned char* fi, int fi_default, const double* xcg,
   return f16::BatchSel{fi, fi_default, xcg, xcg_default};
 }
 
-#define DISPATCH(fn, ...) (G.math_mode == F16_MATH_FAST ? f16::fast::fn(__VA_ARGS__) : f16::strict::fn(__VA_ARGS__))
+// F16_MATH_FAST runs the kernels of f16_step_fast.cu and f16_linearise_fast.cu (the arithmetic of f16_fast.cuh) where the entry
+// point below takes them, and the parity build (f16::strict) everywhere else
+bool fast_mode() { return G.math_mode == F16_MATH_FAST; }
 
-// the one-shot entry points: in F16_MATH_FAST a batch worth staging tables for runs the TMA-tiled kernels on the arithmetic of
-// f16_fast.cuh (f16_step_fast.cu); a handful of aircraft (the legacy Nlplant symbol among them) read the tables through L2
-bool oneshot_fast(long long N) { return G.math_mode == F16_MATH_FAST && G.smem_tables && N >= 4096; }
-// Nlplant_batch (u == NULL: x is xu [17][ld_x]) and calc_xdot_batch
+// Nlplant_batch (u == NULL: x is xu [17][ld_x]) and calc_xdot_batch.  A batch worth staging tables for runs the TMA-tiled kernels
+// of f16_step_fast.cu in F16_MATH_FAST; a handful of aircraft (the legacy Nlplant symbol among them) read the tables through L2
 cudaError_t run_xdot(const f16::BatchSel& sel, const double* x, long long ld_x, const double* u, long long ld_u, double* xdot,
                      long long ld_out, long long N, int* status) {
-  if (oneshot_fast(N)) {
+  const bool staged = G.smem_tables && N >= 4096;
+  if (fast_mode() && staged) {
     cudaError_t e = D->b_redo.reserve((size_t)((N + 31) / 32) * 4);
     if (e != cudaSuccess) return e;
     return f16::fast::launch_xdot_fast(cfg(true), tabs(), sel, x, ld_x, u, ld_u, xdot, ld_out, N, status, (unsigned*)D->b_redo.p);
   }
-  if (!u) return DISPATCH(launch_nlplant, cfg(G.smem_tables && N >= 4096), tabs(), sel, x, ld_x, xdot, ld_out, N, status);
-  return DISPATCH(launch_calc_xdot, cfg(G.smem_tables && N >= 4096), tabs(), sel, x, ld_x, u, ld_u, xdot, ld_out, N, status);
+  if (!u) return f16::strict::launch_nlplant(cfg(staged), tabs(), sel, x, ld_x, xdot, ld_out, N, status);
+  return f16::strict::launch_calc_xdot(cfg(staged), tabs(), sel, x, ld_x, u, ld_u, xdot, ld_out, N, status);
 }
 // linearise_batch.  F16_MATH_STRICT: the staged reference-order kernels (variant 0 / 2: CTA per 32 aircraft, 1: warp per
 // aircraft).  F16_MATH_FAST, variant 0: the two-aircraft-per-warp kernel on the arithmetic of f16_fast.cuh
 // (f16_linearise_fast.cu); variants 1 and 2 keep the strict kernels in fast mode as well.
 cudaError_t run_linearise(const f16::BatchSel& sel, const double* x, long long ld_x, const double* u, long long ld_u, long long N,
                           double eps, int scheme, double* A, double* B, int* status) {
-  if (G.math_mode == F16_MATH_FAST && G.lin_variant == 0 && N < (1LL << 31)) {
+  if (fast_mode() && G.lin_variant == 0 && N < (1LL << 31)) {
     cudaError_t e = D->b_redo.reserve((size_t)((N + 1) / 2) * 4);
     if (e != cudaSuccess) return e;
     return f16::fast::launch_linearise_fast(cfg(true), tabs(), sel, x, ld_x, u, ld_u, N, eps, scheme, A, B, status,
                                             (unsigned*)D->b_redo.p);
   }
   return f16::strict::launch_linearise(cfg(true), tabs(), sel, x, ld_x, u, ld_u, N, eps, scheme, A, B, status);
+}
+// every launch of the fused step: in F16_MATH_FAST both fidelities run the step kernels of f16_step_fast.cu
+cudaError_t run_step(const f16::LaunchCfg& c, const f16::BatchSel& sel, double* x, long long ld_x, const double* u, long long ld_u,
+                     long long N, int K, double dt, const f16::LqrLaw* law, int* status, int* steps_done) {
+  return (fast_mode() ? f16::fast::launch_step : f16::strict::launch_step)(c, tabs(), sel, x, ld_x, u, ld_u, N, K, dt, law, status,
+                                                                           steps_done);
+}
+// trim_batch: in F16_MATH_FAST with table staging on, the objective of f16_step_fast.cu at every batch size -- measured on a B200
+// (1000 W), 1 / 512 points take 2.5 / 11.9 ms there and 5.1 / 25.4 ms on the parity build; that stages its tables from 1024 points
+cudaError_t run_trim(const f16::BatchSel& sel, const double* h, const double* V, long long N, double tol, int maxiter, const double* ux0,
+                     double* x_trim, long long ld_x, double* info, long long ld_info, int* status) {
+  if (fast_mode() && G.smem_tables)
+    return f16::fast::launch_trim(cfg(true), tabs(), sel, h, V, N, tol, maxiter, ux0, x_trim, ld_x, info, ld_info, status);
+  return f16::strict::launch_trim(cfg(G.smem_tables && N >= 1024), tabs(), sel, h, V, N, tol, maxiter, ux0, x_trim, ld_x, info,
+                                  ld_info, status);
 }
 
 int bad_arg(const char* entry) {
@@ -602,8 +618,7 @@ int snapshot_steps(double* d_x, long long ld_x, const double* d_u, long long ld_
   const bool smem = G.smem_tables && (N * (long long)snap_every >= 4096);
   for (int done = 0, j = 0; done < K;) {
     const int k = (K - done) < snap_every ? (K - done) : snap_every;
-    CK(DISPATCH(launch_step, cfg(smem), tabs(), sel, d_x, ld_x, d_u, ld_u, N, k, dt, reinterpret_cast<const f16::LqrLaw*>(lqr),
-                d_status, nullptr));
+    CK(run_step(cfg(smem), sel, d_x, ld_x, d_u, ld_u, N, k, dt, reinterpret_cast<const f16::LqrLaw*>(lqr), d_status, nullptr));
     done += k;
     if (k == snap_every) {
       const int rc = snap(j++);
@@ -829,8 +844,8 @@ void f16_nlplant_xcg(const double* xu, double* xdot, int fidelity, double xcg) {
   int* st_host = reinterpret_cast<int*>(D->pin + 40);
   int* st_dev = reinterpret_cast<int*>(D->pin_dev + 40);
   // one aircraft: tables read through L2 (no 105 KB staging), inputs and outputs in mapped pinned memory
-  cudaError_t e = DISPATCH(launch_nlplant, cfg(false), tabs(), sel_of(nullptr, fidelity, nullptr, xcg), D->pin_dev, 1,
-                           D->pin_dev + 17, 1, 1, st_dev);
+  cudaError_t e = f16::strict::launch_nlplant(cfg(false), tabs(), sel_of(nullptr, fidelity, nullptr, xcg), D->pin_dev, 1,
+                                              D->pin_dev + 17, 1, 1, st_dev);
   if (e == cudaSuccess) e = cudaStreamSynchronize(D->stream);
   if (e != cudaSuccess) {
     cuda_fail(e, "Nlplant");
@@ -857,7 +872,7 @@ void f16_atmos(double alt, double vt, double* coeff) {
   }
   D->pin[48] = alt;
   D->pin[49] = vt;
-  cudaError_t e = DISPATCH(launch_atmos, cfg(false), D->pin_dev + 48, D->pin_dev + 49, 1, D->pin_dev + 50);
+  cudaError_t e = f16::strict::launch_atmos(cfg(false), D->pin_dev + 48, D->pin_dev + 49, 1, D->pin_dev + 50);
   if (e == cudaSuccess) e = cudaStreamSynchronize(D->stream);
   if (e != cudaSuccess) {
     cuda_fail(e, "atmos");
@@ -942,10 +957,10 @@ static int step_partitioned(double* d_x, long long ld_x, const double* d_u, long
   if (d_xcg) CK(f16::partition::launch_gather_f64(c, d_xcg, N, pxcg, N, 1, perm, N));
   const f16::LqrLaw* law = reinterpret_cast<const f16::LqrLaw*>(lqr);
   if (n1 > 0)
-    CK(DISPATCH(launch_step, c, tabs(), sel_of(nullptr, 1, pxcg, xcg_default), px, N, pu, N, n1, K, dt, law, pst, pk));
+    CK(run_step(c, sel_of(nullptr, 1, pxcg, xcg_default), px, N, pu, N, n1, K, dt, law, pst, pk));
   if (n0 > 0)
-    CK(DISPATCH(launch_step, c, tabs(), sel_of(nullptr, 0, pxcg ? pxcg + n1 : nullptr, xcg_default), px + n1, N, pu + n1, N, n0, K,
-                dt, law, pst + n1, pk + n1));
+    CK(run_step(c, sel_of(nullptr, 0, pxcg ? pxcg + n1 : nullptr, xcg_default), px + n1, N, pu + n1, N, n0, K, dt, law, pst + n1,
+                pk + n1));
   if (nbad > 0) {  // neither model: the state stays as it is, status = F16_ST_FIDELITY, no step taken
     CK(f16::partition::launch_fill_i32(c, pst + n1 + n0, (int)F16_ST_FIDELITY, nbad));
     CK(cudaMemsetAsync(pk + n1 + n0, 0, (size_t)nbad * 4, D->stream));
@@ -1066,7 +1081,7 @@ static int step_compacting(double* d_x, long long ld_x, const double* d_u, long 
   long long idle_before = 0;  // stopped aircraft still inside the active set
   while (base < K) {
     const int kc = (K - base) < chunk ? (K - base) : chunk;
-    CK(DISPATCH(launch_step, c, tabs(), sel_of(nullptr, fi, xcg, xcg_default), x, ldx, u, ldu, n_act, kc, dt, law, st, kl));
+    CK(run_step(c, sel_of(nullptr, fi, xcg, xcg_default), x, ldx, u, ldu, n_act, kc, dt, law, st, kl));
     CK(f16::partition::launch_mark_survivors(c, st, kl, ktot, base, n_act, flag));
     base += kc;
     if (base >= K) break;
@@ -1135,7 +1150,7 @@ static int step_on_device(double* d_x, long long ld_x, const double* d_u, long l
   const bool smem = G.smem_tables && (n * (long long)(K > 0 ? K : 1) >= 4096);
   if (G.compaction && !d_fi && d_st && K >= 4096 && n >= 65536 && n < (1LL << 31) && (fi_default == 0 || fi_default == 1))
     return step_compacting(d_x, ld_x, d_u, ld_u, n, K, dt, lqr, fi_default, d_xcg, xcg_default, d_st, d_k, smem);
-  CK(DISPATCH(launch_step, cfg(smem), tabs(), sel_of(d_fi, fi_default, d_xcg, xcg_default), d_x, ld_x, d_u, ld_u, n, K, dt,
+  CK(run_step(cfg(smem), sel_of(d_fi, fi_default, d_xcg, xcg_default), d_x, ld_x, d_u, ld_u, n, K, dt,
               reinterpret_cast<const f16::LqrLaw*>(lqr), d_st, d_k));
   return F16_OK;
 }
@@ -1241,8 +1256,8 @@ int trim_batch_dev(const double* h, const double* V, long long N, double tol, in
   int rc = ensure();
   if (rc != F16_OK) return rc;
   if (!trim_ok(h, V, N, tol, maxiter, x_trim_soa, ld_x, info_soa, ld_info)) return bad_arg("trim_batch_dev");
-  CK(DISPATCH(launch_trim, cfg(G.smem_tables && N >= 1024), tabs(), sel_of(fi, fi_default, xcg, xcg_default), h, V, N, tol, maxiter,
-              ux0 ? ux0 : kTrimGuess, x_trim_soa, ld_x, info_soa, ld_info, status));
+  CK(run_trim(sel_of(fi, fi_default, xcg, xcg_default), h, V, N, tol, maxiter, ux0 ? ux0 : kTrimGuess, x_trim_soa, ld_x, info_soa,
+              ld_info, status));
   return F16_OK;
 }
 
@@ -1254,8 +1269,7 @@ static int trim_host(const double* h, const double* V, long long ld, long long l
   return run_pipeline({soa(h, IN, 8), soa(V, IN, 8), soa(fi, IN, 1), soa(xcg, IN, 8), soa(x_trim, OUT, 8, 18),
                        soa(info, OUT, 8, 4, true), soa(status, OUT, 4, 1, true)},
                       ld, lo, n, one_chunk(n), false, [&](const Slots& p, long long m) -> int {
-                        CK(DISPATCH(launch_trim, cfg(G.smem_tables && m >= 1024), tabs(),
-                                    sel_of(p.u8(2), fi_default, p.f64(3), xcg_default), p.f64(0), p.f64(1), m, tol, maxiter,
+                        CK(run_trim(sel_of(p.u8(2), fi_default, p.f64(3), xcg_default), p.f64(0), p.f64(1), m, tol, maxiter,
                                     ux0 ? ux0 : kTrimGuess, p.f64(4), m, p.f64(5), m, p.i32(6)));
                         return F16_OK;
                       });
@@ -1512,8 +1526,8 @@ int f16_hifi_probe(const double* alpha_deg, const double* beta_deg, const double
   return run_pipeline({soa(alpha_deg, IN, 8), soa(beta_deg, IN, 8), soa(el, IN, 8), soa(coef, OUT, 8, 44), soa(cells, OUT, 4, 8),
                        soa(status, OUT, 4, 1, true)},
                       N, 0, N, one_chunk(N), false, [&](const Slots& p, long long m) -> int {
-                        CK(DISPATCH(launch_hifi_probe, cfg(false), tabs(), p.f64(0), p.f64(1), p.f64(2), m, p.f64(3), p.i32(4),
-                                    p.i32(5)));
+                        CK(f16::strict::launch_hifi_probe(cfg(false), tabs(), p.f64(0), p.f64(1), p.f64(2), m, p.f64(3), p.i32(4),
+                                                          p.i32(5)));
                         return F16_OK;
                       });
 }
@@ -1542,8 +1556,8 @@ int f16_lofi_probe(const double* alpha_deg, const double* beta_deg, const double
   return run_pipeline({soa(alpha_deg, IN, 8), soa(beta_deg, IN, 8), soa(el, IN, 8), soa(dail, IN, 8), soa(drud, IN, 8),
                        soa(out, OUT, 8, 19)},
                       N, 0, N, one_chunk(N), false, [&](const Slots& p, long long m) -> int {
-                        CK(DISPATCH(launch_lofi_probe, cfg(false), tabs(), p.f64(0), p.f64(1), p.f64(2), p.f64(3), p.f64(4), m,
-                                    p.f64(5)));
+                        CK(f16::strict::launch_lofi_probe(cfg(false), tabs(), p.f64(0), p.f64(1), p.f64(2), p.f64(3), p.f64(4), m,
+                                                          p.f64(5)));
                         return F16_OK;
                       });
 }
@@ -1555,7 +1569,7 @@ int f16_div_probe(const double* a, const double* b, long long N, double* out) {
   if (N <= 0 || !a || !b || !out) return bad_arg("f16_div_probe");
   return run_pipeline({soa(a, IN, 8), soa(b, IN, 8), soa(out, OUT, 8, 3)}, N, 0, N, one_chunk(N), false,
                       [&](const Slots& p, long long m) -> int {
-                        CK(f16::strict::launch_div_probe(cfg(false), p.f64(0), p.f64(1), m, p.f64(2)));  // always the strict build's
+                        CK(f16::strict::launch_div_probe(cfg(false), p.f64(0), p.f64(1), m, p.f64(2)));
                         return F16_OK;
                       });
 }
@@ -1567,7 +1581,7 @@ int atmos_batch(const double* alt, const double* vt, long long N, double* coeff_
   if (N <= 0 || !alt || !vt || !coeff_soa) return bad_arg("atmos_batch");
   return run_pipeline({soa(alt, IN, 8), soa(vt, IN, 8), soa(coeff_soa, OUT, 8, 3)}, N, 0, N, one_chunk(N), false,
                       [&](const Slots& p, long long m) -> int {
-                        CK(DISPATCH(launch_atmos, cfg(false), p.f64(0), p.f64(1), m, p.f64(2)));
+                        CK(f16::strict::launch_atmos(cfg(false), p.f64(0), p.f64(1), m, p.f64(2)));
                         return F16_OK;
                       });
 }

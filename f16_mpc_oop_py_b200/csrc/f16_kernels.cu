@@ -1,6 +1,6 @@
-// f16_kernels.cu -- sm_100a kernels of the batched F-16 plant.  Compiled twice (see Makefile):
-//   -DF16_NS=strict -fmad=false   reference operation order, no FMA contraction (parity build)
-//   -DF16_NS=fast   -fmad=true    same expressions, FMA contraction allowed
+// f16_kernels.cu -- sm_100a kernels of the batched F-16 plant in the reference operation order, compiled with -fmad=false
+// (no FMA contraction): the parity build, namespace f16::strict.  F16_MATH_FAST runs the kernels of f16_step_fast.cu and
+// f16_linearise_fast.cu where they apply and these everywhere else.
 //
 // Execution model: one thread per aircraft (or per aircraft x perturbation column in linearise), the 18-element
 // state lives in registers across the K fused Euler steps of step_kernel.  The aero tables (105 KB hifi image,
@@ -12,9 +12,6 @@
 #include "f16_kernels.cuh"
 #include "f16_kernels_common.cuh"
 
-#ifndef F16_NS
-#error "compile with -DF16_NS=strict or -DF16_NS=fast"
-#endif
 #define F16_THREADS 384  // derivative-only kernels: one CTA per SM, 12 warps, <= 168 registers per thread
 // step_kernel is instantiated for 256 / 384 / 512 threads per CTA (254 / 168 / 128 registers per thread, one CTA
 // per SM because of the 105 KB table image); LaunchCfg::step_threads picks one at run time.
@@ -22,7 +19,7 @@
 #define F16_LIN_TILE_LD 397  // doubles per aircraft in the output tile (396 + 1: conflict-free for both phases)
 
 namespace f16 {
-namespace F16_NS {
+namespace strict {
 
 template <int FI>
 struct Img {
@@ -319,9 +316,9 @@ linearise_kernel(DevTables tabs, BatchSel sel, const double* __restrict__ x_g, l
       sincos_pair(ang, sn, cs);
       stage[(2 * k) * 32 + lane] = sn;  // the field order of XB_TRIG
       stage[(2 * k + 1) * 32 + lane] = cs;
-#if defined(__CUDA_ARCH__) && !F16_FASTPATH
+#if defined(__CUDA_ARCH__)
       if (k == 2) stage[60 * 32 + lane] = nb ? F16_DIV(sn, cs) : tan(xu0[4]);
-#elif !F16_FASTPATH
+#else
       if (k == 2) stage[60 * 32 + lane] = tan(xu0[4]);
 #endif
     } else if (own == 1) {
@@ -704,16 +701,6 @@ cudaError_t launch_step(const LaunchCfg& cfg, const DevTables& tabs, const Batch
   for (int FI = 1; FI >= 0 && e == cudaSuccess; FI--) {
     if (!wants(sel, FI)) continue;
     int threads = cfg.step_threads;
-#if defined(F16_FAST)
-    if (FI == 1) {  // the hifi step of F16_MATH_FAST lives in f16_step_fast.cu (explicit FMAs, -fmad=false)
-      e = launch_step_hifi_fast(cfg, tabs, sel, x, ld_x, u, ld_u, N, K, dt, lqr_host, status, steps_done);
-      continue;
-    }
-    if (FI == 0) {  // ... and so does the lofi step
-      e = launch_step_lofi_fast(cfg, tabs, sel, x, ld_x, u, ld_u, N, K, dt, lqr_host, status, steps_done);
-      continue;
-    }
-#endif
     StepKern k = FI ? (lqr_host ? pick_step<1, true>(cfg.smem_tables, threads) : pick_step<1, false>(cfg.smem_tables, threads))
                     : (lqr_host ? pick_step<0, true>(cfg.smem_tables, threads) : pick_step<0, false>(cfg.smem_tables, threads));
     const int smem = FI ? table_smem<1>(cfg.smem_tables) : table_smem<0>(cfg.smem_tables);
@@ -757,14 +744,6 @@ cudaError_t launch_trim(const LaunchCfg& cfg, const DevTables& tabs, const Batch
   g.fixed_point_exit = cfg.trim_fixed_point_exit ? 1 : 0;
   cudaError_t e = cudaSuccess;
   const bool s = cfg.smem_tables;
-#if defined(F16_FAST)
-  if (s) {  // the objective on the step kernel's arithmetic (f16_step_fast.cu)
-    if (wants(sel, 1)) e = launch_trim_fast(cfg, tabs, sel, 1, h, v, N, tol, maxiter, ux0, x_trim, ld_x, info, ld_info, status);
-    if (e == cudaSuccess && wants(sel, 0))
-      e = launch_trim_fast(cfg, tabs, sel, 0, h, v, N, tol, maxiter, ux0, x_trim, ld_x, info, ld_info, status);
-    return e;
-  }
-#endif
   if (wants(sel, 1))
     e = launch_persistent(cfg, s ? trim_kernel<1, true> : trim_kernel<1, false>, F16_TRIM_THREADS, table_smem<1>(s), N,
                           F16_TRIM_THREADS, tabs, sel, h, v, N, tol, maxiter, g, x_trim, ld_x, info, ld_info, status);
@@ -817,5 +796,5 @@ cudaError_t launch_atmos(const LaunchCfg& cfg, const double* alt, const double* 
   return cudaGetLastError();
 }
 
-}  // namespace F16_NS
+}  // namespace strict
 }  // namespace f16

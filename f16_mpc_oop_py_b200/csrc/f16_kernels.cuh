@@ -1,5 +1,6 @@
-// f16_kernels.cuh -- launch interface between the C ABI (f16_api.cu) and the kernel translation unit, which is
-// compiled twice: f16_kernels.cu with -fmad=false as namespace f16::strict and with -fmad=true as f16::fast.
+// f16_kernels.cuh -- launch interface between the C ABI (f16_api.cu) and the kernel translation units.  f16::strict is
+// f16_kernels.cu, the parity build (reference operation order, -fmad=false); f16::fast is f16_step_fast.cu and
+// f16_linearise_fast.cu, the arithmetic of f16_fast.cuh that F16_MATH_FAST runs.
 #pragma once
 #include <cuda_runtime.h>
 
@@ -35,43 +36,32 @@ struct LaunchCfg {
   bool trim_fixed_point_exit = true;  // Nelder-Mead: leave a search that has reached a bitwise fixed point (f16_model.cuh)
 };
 
-#define F16_DECLARE_LAUNCHERS                                                                                        \
-  cudaError_t launch_nlplant(const LaunchCfg&, const DevTables&, const BatchSel&, const double* xu, long long ld_in,  \
-                             double* xdot, long long ld_out, long long N, int* status);                              \
-  cudaError_t launch_calc_xdot(const LaunchCfg&, const DevTables&, const BatchSel&, const double* x, long long ld_x,  \
-                               const double* u, long long ld_u, double* xdot, long long ld_out, long long N,         \
-                               int* status);                                                                         \
-  cudaError_t launch_step(const LaunchCfg&, const DevTables&, const BatchSel&, double* x, long long ld_x,            \
-                          const double* u, long long ld_u, long long N, int K, double dt, const LqrLaw* lqr_host,    \
-                          int* status, int* steps_done);                                                             \
-  cudaError_t launch_linearise(const LaunchCfg&, const DevTables&, const BatchSel&, const double* x, long long ld_x,  \
-                               const double* u, long long ld_u, long long N, double eps, int scheme, double* A,      \
-                               double* B, int* status);                                                              \
-  cudaError_t launch_hifi_probe(const LaunchCfg&, const DevTables&, const double* alpha, const double* beta,         \
-                                const double* el, long long N, double* coef, int* cells, int* status);              \
-  cudaError_t launch_lofi_probe(const LaunchCfg&, const DevTables&, const double* alpha, const double* beta,         \
-                                const double* el, const double* dail, const double* drud, long long N, double* out); \
-  cudaError_t launch_atmos(const LaunchCfg&, const double* alt, const double* vt, long long N, double* coeff);       \
-  cudaError_t launch_div_probe(const LaunchCfg&, const double* a, const double* b, long long N, double* out);        \
-  cudaError_t launch_trim(const LaunchCfg&, const DevTables&, const BatchSel&, const double* h, const double* v,     \
-                          long long N, double tol, int maxiter, const double* ux0, double* x_trim, long long ld_x,    \
-                          double* info, long long ld_info, int* status);
-
 namespace strict {
-F16_DECLARE_LAUNCHERS
-}
+cudaError_t launch_nlplant(const LaunchCfg&, const DevTables&, const BatchSel&, const double* xu, long long ld_in, double* xdot,
+                           long long ld_out, long long N, int* status);
+cudaError_t launch_calc_xdot(const LaunchCfg&, const DevTables&, const BatchSel&, const double* x, long long ld_x, const double* u,
+                             long long ld_u, double* xdot, long long ld_out, long long N, int* status);
+cudaError_t launch_step(const LaunchCfg&, const DevTables&, const BatchSel&, double* x, long long ld_x, const double* u, long long ld_u,
+                        long long N, int K, double dt, const LqrLaw* lqr_host, int* status, int* steps_done);
+cudaError_t launch_linearise(const LaunchCfg&, const DevTables&, const BatchSel&, const double* x, long long ld_x, const double* u,
+                             long long ld_u, long long N, double eps, int scheme, double* A, double* B, int* status);
+cudaError_t launch_hifi_probe(const LaunchCfg&, const DevTables&, const double* alpha, const double* beta, const double* el,
+                              long long N, double* coef, int* cells, int* status);
+cudaError_t launch_lofi_probe(const LaunchCfg&, const DevTables&, const double* alpha, const double* beta, const double* el,
+                              const double* dail, const double* drud, long long N, double* out);
+cudaError_t launch_atmos(const LaunchCfg&, const double* alt, const double* vt, long long N, double* coeff);
+cudaError_t launch_div_probe(const LaunchCfg&, const double* a, const double* b, long long N, double* out);
+cudaError_t launch_trim(const LaunchCfg&, const DevTables&, const BatchSel&, const double* h, const double* v, long long N, double tol,
+                        int maxiter, const double* ux0, double* x_trim, long long ld_x, double* info, long long ld_info, int* status);
+}  // namespace strict
+
 namespace fast {
-F16_DECLARE_LAUNCHERS
-// f16_step_fast.cu: the hifi step on the arithmetic of f16_fast.cuh
-cudaError_t launch_step_hifi_fast(const LaunchCfg&, const DevTables&, const BatchSel&, double* x, long long ld_x,
-                                  const double* u, long long ld_u, long long N, int K, double dt, const LqrLaw* lqr_host,
-                                  int* status, int* steps_done);
-cudaError_t launch_trim_fast(const LaunchCfg&, const DevTables&, const BatchSel&, int FI, const double* h, const double* v,
-                             long long N, double tol, int maxiter, const double* ux0, double* x_trim, long long ld_x,
-                             double* info, long long ld_info, int* status);
-cudaError_t launch_step_lofi_fast(const LaunchCfg&, const DevTables&, const BatchSel&, double* x, long long ld_x,
-                                  const double* u, long long ld_u, long long N, int K, double dt, const LqrLaw* lqr_host,
-                                  int* status, int* steps_done);
+// f16_step_fast.cu: step_batch, both fidelities
+cudaError_t launch_step(const LaunchCfg&, const DevTables&, const BatchSel&, double* x, long long ld_x, const double* u, long long ld_u,
+                        long long N, int K, double dt, const LqrLaw* lqr_host, int* status, int* steps_done);
+// trim_batch with the objective on the step kernel's arithmetic; always stages the tables in shared memory
+cudaError_t launch_trim(const LaunchCfg&, const DevTables&, const BatchSel&, const double* h, const double* v, long long N, double tol,
+                        int maxiter, const double* ux0, double* x_trim, long long ld_x, double* info, long long ld_info, int* status);
 // Nlplant_batch (u == nullptr, x = xu [17][N]) / calc_xdot_batch on the arithmetic of f16_fast.cuh, TMA-staged input tiles
 cudaError_t launch_xdot_fast(const LaunchCfg&, const DevTables&, const BatchSel&, const double* x, long long ld_x, const double* u,
                              long long ld_u, double* xdot, long long ld_out, long long N, int* status, unsigned* redo);
@@ -80,7 +70,7 @@ cudaError_t launch_linearise_fast(const LaunchCfg&, const DevTables&, const Batc
                                   long long ld_u, long long N, double eps, int scheme, double* A, double* B, int* status, unsigned* redo);
 cudaError_t launch_fast_probe(const LaunchCfg&, const DevTables&, const double* alpha, const double* beta, const double* el,
                               long long N, double* coef, int* cells, double* lam, int* status);
-}
+}  // namespace fast
 
 // f16_linalg.cu: reduced-model gather, zero-order-hold discretisation, discrete LQR gain (one thread per aircraft)
 namespace linalg {

@@ -22,6 +22,8 @@ namespace fast {
 // ------------------------------------------------------------------------------------------------------
 constexpr int FAST_SMEM_BYTES = F16_FI_BYTES + 16;
 
+static bool sel_wants(const BatchSel& s, int FI) { return s.fi != nullptr || s.fi_default == FI || (FI == 1 && s.fi_default != 0); }
+
 template <bool SMEM, bool LQR, int THREADS, int COLMASK = 0>
 __global__ void __launch_bounds__(THREADS, 1)
 step_hifi_fast_kernel(DevTables tabs, BatchSel sel, double* __restrict__ x_g, long long ld_x,
@@ -298,18 +300,21 @@ trim_fast_kernel(DevTables tabs, BatchSel sel, const double* __restrict__ h_g, c
   }
 }
 
-cudaError_t launch_trim_fast(const LaunchCfg& cfg, const DevTables& tabs, const BatchSel& sel, int FI, const double* h,
-                             const double* v, long long N, double tol, int maxiter, const double* ux0, double* x_trim,
-                             long long ld_x, double* info, long long ld_info, int* status) {
+cudaError_t launch_trim(const LaunchCfg& cfg, const DevTables& tabs, const BatchSel& sel, const double* h, const double* v, long long N,
+                        double tol, int maxiter, const double* ux0, double* x_trim, long long ld_x, double* info, long long ld_info,
+                        int* status) {
   if (N <= 0) return cudaSuccess;
   TrimGuessFast g;
   for (int k = 0; k < 5; k++) g.ux[k] = ux0[k];
   g.fixed_point_exit = cfg.trim_fixed_point_exit ? 1 : 0;
-  if (FI)
-    return launch_persistent(cfg, trim_fast_kernel<1>, 256, FAST_SMEM_BYTES, N, 256, tabs, sel, h, v, N, tol, maxiter, g, x_trim,
-                             ld_x, info, ld_info, status);
-  return launch_persistent(cfg, trim_fast_kernel<0>, 256, F16_LOFI_STEP_IMG_DOUBLES * 8, N, 256, tabs, sel, h, v, N, tol, maxiter,
-                           g, x_trim, ld_x, info, ld_info, status);
+  cudaError_t e = cudaSuccess;
+  if (sel_wants(sel, 1))
+    e = launch_persistent(cfg, trim_fast_kernel<1>, 256, FAST_SMEM_BYTES, N, 256, tabs, sel, h, v, N, tol, maxiter, g, x_trim, ld_x,
+                          info, ld_info, status);
+  if (e == cudaSuccess && sel_wants(sel, 0))
+    e = launch_persistent(cfg, trim_fast_kernel<0>, 256, F16_LOFI_STEP_IMG_DOUBLES * 8, N, 256, tabs, sel, h, v, N, tol, maxiter, g,
+                          x_trim, ld_x, info, ld_info, status);
+  return e;
 }
 
 // ------------------------------------------------------------------------------------------------------
@@ -676,8 +681,6 @@ static cudaError_t launch_xdot_fast_one(const LaunchCfg& cfg, const DevTables& t
                            ld_u, xd, ld_out, N, status, tma ? 1 : 0, redo);
 }
 
-static bool sel_wants(const BatchSel& s, int FI) { return s.fi != nullptr || s.fi_default == FI || (FI == 1 && s.fi_default != 0); }
-
 // u == nullptr: Nlplant_batch (x is xu [17][N]); else calc_xdot_batch
 // redo: device scratch of one unsigned per 32 aircraft (which lanes of a task take the reference-order path)
 cudaError_t launch_xdot_fast(const LaunchCfg& cfg, const DevTables& tabs, const BatchSel& sel, const double* x, long long ld_x,
@@ -762,9 +765,9 @@ static StepKern pick_step_hifi_fast(bool smem_tables, int& threads) {
   return step_hifi_fast_kernel<true, LQR, 768>;
 }
 
-cudaError_t launch_step_hifi_fast(const LaunchCfg& cfg, const DevTables& tabs, const BatchSel& sel, double* x, long long ld_x,
-                                  const double* u, long long ld_u, long long N, int K, double dt, const LqrLaw* lqr_host,
-                                  int* status, int* steps_done) {
+static cudaError_t launch_step_hifi_fast(const LaunchCfg& cfg, const DevTables& tabs, const BatchSel& sel, double* x, long long ld_x,
+                                         const double* u, long long ld_u, long long N, int K, double dt, const LqrLaw* lqr_host,
+                                         int* status, int* steps_done) {
   if (N <= 0) return cudaSuccess;
   fastmath::LqrDense dense = fastmath::LqrDense();
   if (lqr_host) fastmath::make_dense_law(*lqr_host, dense);
@@ -806,9 +809,9 @@ cudaError_t launch_step_hifi_fast(const LaunchCfg& cfg, const DevTables& tabs, c
   return launch_persistent(cfg, k, threads, smem, N, threads, tabs, sel, x, ld_x, u, ld_u, N, K, dt, status, steps_done, dense);
 }
 
-cudaError_t launch_step_lofi_fast(const LaunchCfg& cfg, const DevTables& tabs, const BatchSel& sel, double* x, long long ld_x,
-                                  const double* u, long long ld_u, long long N, int K, double dt, const LqrLaw* lqr_host,
-                                  int* status, int* steps_done) {
+static cudaError_t launch_step_lofi_fast(const LaunchCfg& cfg, const DevTables& tabs, const BatchSel& sel, double* x, long long ld_x,
+                                         const double* u, long long ld_u, long long N, int K, double dt, const LqrLaw* lqr_host,
+                                         int* status, int* steps_done) {
   if (N <= 0) return cudaSuccess;
   fastmath::LqrDense dense = fastmath::LqrDense();
   if (lqr_host) fastmath::make_dense_law(*lqr_host, dense);
@@ -819,6 +822,15 @@ cudaError_t launch_step_lofi_fast(const LaunchCfg& cfg, const DevTables& tabs, c
                : (dense.colmask == F16_LQR_MPC_COLMASK && dense.row_mask == 0xE) ? step_lofi_fast_kernel<true, 384, F16_LQR_MPC_SHAPE>
                                                       : step_lofi_fast_kernel<true, 384>;
   return launch_persistent(cfg, k, 384, smem, N, 384, tabs, sel, x, ld_x, u, ld_u, N, K, dt, status, steps_done, dense);
+}
+
+cudaError_t launch_step(const LaunchCfg& cfg, const DevTables& tabs, const BatchSel& sel, double* x, long long ld_x, const double* u,
+                        long long ld_u, long long N, int K, double dt, const LqrLaw* lqr_host, int* status, int* steps_done) {
+  cudaError_t e = cudaSuccess;
+  if (sel_wants(sel, 1)) e = launch_step_hifi_fast(cfg, tabs, sel, x, ld_x, u, ld_u, N, K, dt, lqr_host, status, steps_done);
+  if (e == cudaSuccess && sel_wants(sel, 0))
+    e = launch_step_lofi_fast(cfg, tabs, sel, x, ld_x, u, ld_u, N, K, dt, lqr_host, status, steps_done);
+  return e;
 }
 
 }  // namespace fast

@@ -47,16 +47,21 @@ extern "C" {
 
 /* ---- arithmetic mode ---------------------------------------------------------------------------- */
 #define F16_MATH_STRICT 0 /* reference operation order, no FMA contraction: the parity build */
-#define F16_MATH_FAST 1   /* throughput build.  step_batch / trim_batch run the RE-ASSOCIATED arithmetic of csrc/f16_fast.cuh
-                           * ((f, d) table image with node deltas, polynomial sin/cos and tfac^4.14, one shared reciprocal,
-                           * wind-axis equations with vt cancelled); Nlplant_batch / calc_xdot_batch run the strict
-                           * expressions with FMA contraction and reciprocal multiplies.  Both stay within the parity bars
-                           * (<= 1e-12 scaled per derivative, <= 1e-9 after 10 s; tests/test_gpu_parity.py);
-                           * linearise_batch runs f16_fast.cuh too (two aircraft per warp, csrc/f16_linearise_fast.cu): the quotient
-                           * multiplies last-bit differences of f by 1/eps, so its entries agree with the reference's to
-                           * 1e-8 + 4 ulp(f_i) / h (up to 3.4e-8 on the 900 ft/s navigation rows; the reference's own source built
-                           * with -O3 -march=native moves as much, profiles/r02_jacobian_noise_floor.md).
-                           * f16_set_linearise_variant(2) keeps the strict kernel in fast mode. */
+#define F16_MATH_FAST 1   /* throughput build: the RE-ASSOCIATED arithmetic of csrc/f16_fast.cuh ((f, d) table image with node
+                           * deltas, polynomial sin/cos and tfac^4.14, one shared reciprocal, wind-axis equations with vt
+                           * cancelled) where its kernels apply, and the bits of F16_MATH_STRICT everywhere else:
+                           *  - step_batch, step_batch_traj, step_batch_stats (and their _dev forms), every batch: f16_fast.cuh;
+                           *  - trim_batch, with table staging on (f16_set_table_staging): f16_fast.cuh.  Staging off: strict;
+                           *  - Nlplant_batch / calc_xdot_batch from 4096 aircraft, with table staging on: f16_fast.cuh.
+                           *    Smaller batches, or staging off: strict;
+                           *  - linearise_batch: f16_fast.cuh (two aircraft per warp, csrc/f16_linearise_fast.cu), except under
+                           *    f16_set_linearise_variant(1) or (2), which keep the strict kernels;
+                           *  - the legacy Nlplant and atmos symbols, atmos_batch, f16_hifi_probe, f16_lofi_probe: strict.
+                           * f16_fast.cuh stays within the parity bars (<= 1e-12 scaled per derivative, <= 1e-9 after 10 s;
+                           * tests/test_gpu_parity.py).  A Jacobian's quotient multiplies last-bit differences of f by 1/eps, so
+                           * the fast entries agree with the reference's to 1e-8 + 4 ulp(f_i) / h (up to 3.4e-8 on the 900 ft/s
+                           * navigation rows; the reference's own source built with -O3 -march=native moves as much,
+                           * profiles/r02_jacobian_noise_floor.md). */
 
 /* ---- CLr table quirk ---------------------------------------------------------------------------
  * The reference never loads CL1320_ALPHA1_606.dat (hifi_F16_AeroData.c:965-972: the fscanf loop is the
@@ -169,7 +174,7 @@ int step_batch(double *x_soa, const double *u_soa, long long N, int K, double dt
 int step_batch_traj(double *x_soa, const double *u_soa, long long N, int K, int snap_every, double dt, const f16_lqr_t *lqr,
                     const unsigned char *fi, int fi_default, const double *xcg, double xcg_default, double *traj, int *status);
 /* Finite-difference Jacobians of _calc_xdot (env.py:294-342): A [N][18][18], B [N][18][4], row-major.
- * Always computed by the strict (no FMA contraction) build: the quotient amplifies rounding noise by 1/eps.
+ * F16_MATH_FAST computes them on csrc/f16_linearise_fast.cu (see F16_MATH_FAST): the quotient amplifies rounding noise by 1/eps.
  * eps must lie in [1e-12, 1e3] (the reference uses 1e-5). */
 int linearise_batch(const double *x_soa, const double *u_soa, long long N, double eps, int scheme, double *A, double *B,
                     const unsigned char *fi, int fi_default, const double *xcg, double xcg_default, int *status);

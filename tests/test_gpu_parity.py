@@ -75,8 +75,7 @@ def test_atmosphere_over_the_whole_altitude_range(f16, oracle, mode):
     vt[::7] = 0.005
     out = f16.atmos(alt, vt)
     ref = np.array([oracle.atmos(float(a), float(v)) for a, v in zip(alt, vt)]).T
-    # strict: reference operation order, 4 ulp for the power; F16_MATH_FAST contracts the products around it: 1e-13
-    bar = 4 * np.spacing(np.abs(ref)) if mode == "strict" else 1e-13 * np.abs(ref)
+    bar = 4 * np.spacing(np.abs(ref))   # both modes run the parity build here
     assert np.all(np.abs(out - ref) <= bar), float(np.max(np.abs(out - ref) / np.abs(ref)))
 
 
@@ -320,12 +319,91 @@ def test_oneshot_fast_kernels_load_paths_agree(f16, fi):
             assert np.array_equal(fbm.last_status, full_st[:m]), m
             o2, s2 = f16.nlplant(np.ascontiguousarray(x[:17, :m]), fi, 0.3)
             assert np.array_equal(o2, nl[:, :m], equal_nan=True) and np.array_equal(s2, nl_st[:m]), m
-        # the small-batch path (tables through L2, f16_model.cuh arithmetic) agrees to the derivative tolerance
-        small = f16.F16Batch(x[:, :1000], u[:, :1000], fi_flag=fi, xcg=0.3)._calc_xdot(np.ascontiguousarray(x[:, :1000]),
-                                                                                     np.ascontiguousarray(u[:, :1000]))
-        ok = full_st[:1000] == 0
-        fin = np.isfinite(full[:, :1000]).all(axis=0) & ok
+        # the small-batch path (tables through L2) is the parity build: the bits and status words of F16_MATH_STRICT
+        xs, us = np.ascontiguousarray(x[:, :1000]), np.ascontiguousarray(u[:, :1000])
+        fbs = f16.F16Batch(xs, us, fi_flag=fi, xcg=0.3)
+        small = fbs._calc_xdot(xs, us)
+        small_st = fbs.last_status.copy()
+        fin = np.isfinite(full[:, :1000]).all(axis=0) & (full_st[:1000] == 0)
         assert scaled_err(small[:, fin], full[:, :1000][:, fin]) < TOL_DERIV
+        f16.lib.f16_set_math_mode(f16.MATH_STRICT)
+        assert np.array_equal(small, fbs._calc_xdot(xs, us), equal_nan=True) and np.array_equal(small_st, fbs.last_status)
+    finally:
+        f16.lib.f16_set_math_mode(prev)
+
+
+def test_fast_mode_off_its_kernels_is_the_parity_build(f16):
+    """F16_MATH_FAST runs f16_fast.cuh only where its kernels are taken (include/f16_b200.h): one-shot batches below 4096
+    aircraft, anything with table staging off, the legacy symbols, atmos_batch and the table probes give the bits and status
+    words of F16_MATH_STRICT -- a result does not depend on the batch size through a third arithmetic.  A fast-mode trim runs
+    f16_fast.cuh at every batch size: a few points get the bits they get inside a batch of 1024."""
+    r = np.random.default_rng(31)
+    batches = []
+    for n in (1, 31, 1000, 4095):
+        xu = random_envelope_xu(n, seed=n, hifi=True)
+        x = np.vstack([xu, r.uniform(-30, 30, (1, n))])
+        u = np.stack([r.uniform(500, 20000, n), r.uniform(-30, 30, n), r.uniform(-25, 25, n), r.uniform(-35, 35, n)])
+        if n > 1:
+            x[7, n - 1] = np.deg2rad(60.0)   # outside the hifi tables: a status word
+        fi, xcg = r.integers(0, 2, n).astype(np.uint8), r.uniform(0.25, 0.35, n)
+        batches.append((x, u, [(1, 0.3), (0, 0.3), (fi, xcg)]))
+    nl = load_golden("xcg25")["nl_xu"].copy()
+    alt = np.linspace(-10_000, 120_000, 3001)
+    vt = np.linspace(0.005, 1000.0, alt.size)
+    a, b, e = _probe_points()
+    m = a.size
+    da, dr = r.uniform(-1, 1, m), r.uniform(-1, 1, m)
+    h, v = np.array([5000.0, 20000.0, 35000.0]), np.array([400.0, 700.0, 900.0])
+    xb = np.vstack([random_envelope_xu(5000, seed=5, hifi=True), r.uniform(-30, 30, (1, 5000))])
+    ub = np.stack([r.uniform(500, 20000, 5000), r.uniform(-30, 30, 5000), r.uniform(-25, 25, 5000), r.uniform(-35, 35, 5000)])
+
+    def run():
+        out = []
+        for x, u, sels in batches:
+            for fi, xcg in sels:
+                out += list(f16.nlplant(x[:17], fi, xcg))
+                fb = f16.F16Batch(x, u, fi_flag=fi, xcg=xcg)
+                out += [fb._calc_xdot(x, u), fb.last_status.copy()]
+        for fi in (1, 0):
+            xd = np.zeros(18)
+            f16.lib.Nlplant(ctypes.c_void_p(nl.ctypes.data), ctypes.c_void_p(xd.ctypes.data), ctypes.c_int(fi))
+            out += [xd, f16.lib.f16_last_status()]
+        coeff = np.zeros(3)
+        f16.lib.atmos(ctypes.c_double(nl[2]), ctypes.c_double(nl[6]), ctypes.c_void_p(coeff.ctypes.data))
+        out += [coeff, f16.atmos(alt, vt)]
+        coef, cells, st = np.empty((44, m)), np.empty((8, m), dtype=np.int32), np.zeros(m, dtype=np.int32)
+        assert f16.lib.f16_hifi_probe(a.ctypes.data, b.ctypes.data, e.ctypes.data, m, coef.ctypes.data, cells.ctypes.data,
+                                      st.ctypes.data) == 0
+        lofi = np.empty((19, m))
+        assert f16.lib.f16_lofi_probe(a.ctypes.data, b.ctypes.data, e.ctypes.data, da.ctypes.data, dr.ctypes.data, m,
+                                      lofi.ctypes.data) == 0
+        out += [coef, cells, st, lofi]
+        prev = f16.lib.f16_set_table_staging(0)
+        try:
+            fb = f16.F16Batch(xb, ub, fi_flag=1, xcg=0.3)
+            out += [fb._calc_xdot(xb, ub), fb.last_status.copy()]
+            xt, opt = f16.trim(h[:1], v[:1], fi=1, xcg=0.3)
+            out += [xt, opt["fun"], opt["nit"], opt["status"]]
+        finally:
+            f16.lib.f16_set_table_staging(prev)
+        return out
+
+    res = {}
+    for mode in (f16.MATH_STRICT, f16.MATH_FAST):
+        prev = f16.lib.f16_set_math_mode(mode)
+        try:
+            res[mode] = run()
+        finally:
+            f16.lib.f16_set_math_mode(prev)
+    differ = [i for i, (s, q) in enumerate(zip(res[f16.MATH_STRICT], res[f16.MATH_FAST])) if not np.array_equal(s, q, equal_nan=True)]
+    assert not differ, differ
+    prev = f16.lib.f16_set_math_mode(f16.MATH_FAST)
+    try:
+        hb, vb = np.resize(h, 1024), np.resize(v, 1024)
+        for fi in (1, 0):
+            few, big = f16.trim(h, v, fi=fi, xcg=0.3), f16.trim(hb, vb, fi=fi, xcg=0.3)
+            assert np.array_equal(few[0], big[0][:, :3], equal_nan=True), fi
+            assert all(np.array_equal(few[1][k], big[1][k][:3], equal_nan=True) for k in few[1]), fi
     finally:
         f16.lib.f16_set_math_mode(prev)
 
