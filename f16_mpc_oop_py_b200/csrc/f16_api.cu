@@ -1291,9 +1291,10 @@ int trim_batch(const double* h, const double* V, long long N, double tol, int ma
 // enqueue the summary row of aircraft [0, N) and its copy to row_host (74 doubles) on D->stream
 static int summary_row(const double* d_x, long long ld, long long N, const int* d_status, double* row_host) {
   const int grid = f16::stats::summary_grid(cfg(false), N);
-  CK(D->b_sum.reserve(((size_t)grid * f16::stats::PARTIAL_STRIDE + 80) * 8));
+  const size_t scratch_n = f16::stats::summary_scratch(grid);
+  CK(D->b_sum.reserve((scratch_n + 74) * 8));
   double* scratch = (double*)D->b_sum.p;
-  double* row = scratch + (size_t)grid * f16::stats::PARTIAL_STRIDE;  // must not alias the scratch
+  double* row = scratch + scratch_n;  // must not alias the scratch
   CK(f16::stats::launch_summary(cfg(false), d_x, ld, N, d_status, row, scratch, grid));
   CK(cudaMemcpyAsync(row_host, row, 74 * 8, cudaMemcpyDeviceToHost, D->stream));
   return F16_OK;
@@ -1304,9 +1305,10 @@ static int step_stats_core(double* d_x, long long ld_x, const double* d_u, long 
                            double dt, const f16_lqr_t* lqr, const f16::BatchSel& sel, int* d_status, double* rows_host) {
   const int n_rows = K / snap_every;
   const int grid = f16::stats::summary_grid(cfg(false), N);
-  CK(D->b_sum.reserve(((size_t)grid * f16::stats::PARTIAL_STRIDE + (size_t)(n_rows > 0 ? n_rows : 1) * 74 + 8) * 8));
+  const size_t scratch_n = f16::stats::summary_scratch(grid);
+  CK(D->b_sum.reserve((scratch_n + (size_t)(n_rows > 0 ? n_rows : 1) * 74) * 8));
   double* scratch = (double*)D->b_sum.p;
-  double* rows_dev = scratch + (size_t)grid * f16::stats::PARTIAL_STRIDE;
+  double* rows_dev = scratch + scratch_n;
   const int rc = snapshot_steps(d_x, ld_x, d_u, ld_u, N, K, snap_every, dt, lqr, sel, d_status, [&](int j) -> int {
     CK(f16::stats::launch_summary(cfg(false), d_x, ld_x, N, d_status, rows_dev + (size_t)j * 74, scratch, grid));
     return F16_OK;

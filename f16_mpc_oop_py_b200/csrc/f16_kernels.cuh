@@ -83,7 +83,7 @@ cudaError_t launch_dlqr(const LaunchCfg&, const double* Ad, const double* Bd, co
 
 // f16_stats.cu: per-state summary of a batch (count, alive, min, max, mean, M2), reduced on the device
 namespace stats {
-constexpr int PARTIAL_STRIDE = 80;  // doubles of device scratch per CTA column of the reduction (73 used)
+size_t summary_scratch(int grid);  // doubles of device scratch launch_summary needs at this grid
 cudaError_t launch_summary(const LaunchCfg&, const double* x, long long ld, long long N, const int* status, double* row,
                            double* scratch, int grid);
 int summary_grid(const LaunchCfg&, long long N);

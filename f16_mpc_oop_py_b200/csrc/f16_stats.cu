@@ -5,17 +5,21 @@
 // is what a rank contributes to the only collective of a run (an all-gather of these rows, shard.py::merge_summaries).
 //
 // HBM-bound, ONE pass: every plane of the SoA state is read once and the status words three times (once per group of six
-// states), 152 B per aircraft, fully coalesced (thread n reads x[i][n]).  Mean and M2 come out of the same pass without
-// cancellation by the textbook shifted-data form: with a shift c_i taken from INSIDE the data -- state i of the first
-// surviving aircraft among the first 32 of the batch (aircraft 0 if none survives there) -- the kernel accumulates
-// S1 = sum (v - c) and S2 = sum (v - c)^2, which add up exactly like plain sums over threads, warps and CTAs, and the finishing
-// CTA forms mean = c + S1 / n, M2 = S2 - S1^2 / n.  The subtraction v - c is exact for values within a factor of two of c and
-// the final difference loses (|mean - c| / sigma)^2 ulps: nothing for a shift inside the cloud, 1e-10 relative only when that
-// one aircraft sits a thousand standard deviations out.  (Combining per-thread MEANS by Chan's update is first-order in the
-// rounding of those means and misses 1e-10 on a plane like h = 10000 +- 0.001 ft; two passes -- sums, then squared deviations
-// about the mean, the round-1 kernel -- cost twice the bytes: 0.119 ms at 2^20 aircraft.)  Reductions are a fixed tree
-// (per thread -> warp shuffles -> shared memory -> one partial per CTA -> one finishing CTA, lane-strided), so the result is
-// bit-reproducible for a given device and batch size; no atomics.
+// states), 152 B per aircraft, fully coalesced (thread n reads x[i][n]).  Mean and M2 come out of the same pass by the
+// textbook shifted-data form: with a shift c_i taken from INSIDE the data -- state i of the first surviving aircraft of the
+// batch (aircraft 0 when there is no status array) -- the kernel accumulates S1 = sum (v - c) and S2 = sum (v - c)^2, which
+// add up exactly like plain sums over threads, warps and CTAs, and the finishing CTA forms mean = c + S1 / n,
+// M2 = S2 - S1^2 / n.  The subtraction v - c is exact for values within a factor of two of c, and the final difference loses
+// (|mean - c| / sigma)^2 ulps: nothing for a shift inside the cloud, 1e-10 relative only when the first survivor sits a
+// thousand standard deviations out.  The shift must be a survivor: a dead aircraft's state is frozen wherever it left the
+// envelope (a crash below h = 0, a NaN), arbitrarily far from the survivors, and a shift of 0 against h = 1e4 +- 1e-3 ft
+// costs 6e-3 of M2.  So when a status array is given, first_alive_kernel finds that aircraft first (a 64-bit atomicMin;
+// warps stop scanning above a survivor already found, so a batch whose first survivor is aircraft j reads about
+// j + 128 x (warps in the grid) status words).  (Combining per-thread MEANS by Chan's update is first-order in the rounding
+// of those means and misses 1e-10 on a plane like h = 10000 +- 0.001 ft; two passes -- sums, then squared deviations about
+// the mean, the round-1 kernel -- cost twice the bytes: 0.119 ms at 2^20 aircraft.)  Reductions are a fixed tree (per
+// thread -> warp shuffles -> shared memory -> one partial per CTA -> one finishing CTA, lane-strided), so the result is
+// bit-reproducible for a given device and batch size; the one atomic picks a minimum, which does not depend on the order.
 #include <math.h>
 #include <stdint.h>
 
@@ -26,6 +30,7 @@ namespace stats {
 
 constexpr int THREADS = 256;
 constexpr int NS = 18;
+constexpr int PARTIAL_STRIDE = 80;  // doubles of scratch per CTA column of the reduction (73 used)
 
 __device__ __forceinline__ double warp_sum(double v) {
 #pragma unroll
@@ -47,27 +52,58 @@ __device__ __forceinline__ double warp_max(double v) {
 // blockIdx.y picks NS / NG of the eighteen states (six: 24 accumulators + 6 shifts per thread); the loads in flight, not the
 // arithmetic, set the pace.
 
-// the common shift: state s of the first aircraft with status 0 among the first min(N, 32), else of aircraft 0
-__device__ __forceinline__ long long shift_aircraft(const int* __restrict__ status, long long N) {
+// the shift aircraft: the first survivor (*first, from first_alive_kernel), aircraft 0 without a status array, -1 when no
+// aircraft survives
+__device__ __forceinline__ long long shift_aircraft(const int* status, long long N, const unsigned long long* first) {
+  if (N <= 0) return -1;  // launch_summary neither clears nor searches for an empty batch: *first is not read
+  if (!status) return 0;
+  const unsigned long long f = *first;
+  return f < (unsigned long long)N ? (long long)f : -1;
+}
+
+// *first = the lowest n with status[n] == 0 (left at its initial ULLONG_MAX when there is none).  Warp w scans status words
+// [128 w, 128 w + 128), then the same span one grid of warps further on, and stops at a span that starts above a survivor
+// some warp has already found.
+constexpr int SPAN = 128;
+__global__ void __launch_bounds__(THREADS)
+first_alive_kernel(const int* __restrict__ status, long long N, unsigned long long* first) {
   const int lane = threadIdx.x & 31;
-  const bool ok = lane < N && (!status || status[lane] == 0);
-  const unsigned m = __ballot_sync(0xffffffffu, ok);
-  return m ? (long long)(__ffs(m) - 1) : 0;
+  const long long warps = (long long)gridDim.x * (THREADS / 32);
+  for (long long base = ((long long)blockIdx.x * (THREADS / 32) + (threadIdx.x >> 5)) * SPAN; base < N; base += warps * SPAN) {
+    unsigned long long known = lane == 0 ? *(volatile const unsigned long long*)first : 0;
+    known = __shfl_sync(0xffffffffu, known, 0);
+    if ((unsigned long long)base >= known) return;
+    int st[SPAN / 32];
+#pragma unroll
+    for (int k = 0; k < SPAN / 32; k++) {
+      const long long n = base + k * 32 + lane;
+      st[k] = n < N ? status[n] : 1;
+    }
+#pragma unroll
+    for (int k = 0; k < SPAN / 32; k++) {
+      const unsigned m = __ballot_sync(0xffffffffu, st[k] == 0);
+      if (m) {
+        if (lane == 0) atomicMin(first, (unsigned long long)(base + k * 32 + __ffs(m) - 1));
+        return;
+      }
+    }
+  }
 }
 
 template <int NG, int MINB>
 __global__ void __launch_bounds__(THREADS, MINB)
-partial_kernel(const double* __restrict__ x, long long ld, long long N, const int* __restrict__ status, double* __restrict__ partial) {
+partial_kernel(const double* __restrict__ x, long long ld, long long N, const int* __restrict__ status,
+               const unsigned long long* __restrict__ first, double* __restrict__ partial) {
   constexpr int NH = NS / NG;
   __shared__ double red[THREADS / 32][4 * NH + 1];
   const int s0 = blockIdx.y * NH;  // first state of this group
   x += (long long)s0 * ld;
-  const long long j0 = N > 0 ? shift_aircraft(status, N) : 0;
+  const long long j0 = shift_aircraft(status, N, first);
   double c[NH], s1[NH], s2[NH], mn[NH], mx[NH];
   double cnt = 0.0;
 #pragma unroll
   for (int i = 0; i < NH; i++) {
-    const double v0 = N > 0 ? x[i * ld + j0] : 0.0;
+    const double v0 = j0 >= 0 ? x[i * ld + j0] : 0.0;
     c[i] = fabs(v0) < INFINITY ? v0 : 0.0;  // a NaN or an infinity is no shift
     s1[i] = 0.0;
     s2[i] = 0.0;
@@ -117,14 +153,9 @@ partial_kernel(const double* __restrict__ x, long long ld, long long N, const in
 // same shuffle tree); then 18 threads form the 74-double row from the totals and the shift
 __global__ void __launch_bounds__(1024)
 finish_kernel(const double* __restrict__ partial, int n_part, const double* __restrict__ x, long long ld, long long N,
-              const int* __restrict__ status, double* __restrict__ row) {
+              const int* __restrict__ status, const unsigned long long* __restrict__ first, double* __restrict__ row) {
   __shared__ double tot[4 * NS + 1];
-  __shared__ long long j0_sh;
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  if (warp == 0) {
-    const long long j0 = N > 0 ? shift_aircraft(status, N) : 0;
-    if (lane == 0) j0_sh = j0;
-  }
   for (int f = warp; f < 4 * NS + 1; f += 32) {
     const bool is_min = f >= 2 * NS && f < 3 * NS, is_max = f >= 3 * NS && f < 4 * NS;
     double a = is_min ? INFINITY : is_max ? -INFINITY : 0.0;
@@ -143,7 +174,8 @@ finish_kernel(const double* __restrict__ partial, int n_part, const double* __re
   }
   if (f < NS) {
     const double n = tot[4 * NS];
-    const double v0 = N > 0 ? x[f * ld + j0_sh] : 0.0;
+    const long long j0 = shift_aircraft(status, N, first);
+    const double v0 = j0 >= 0 ? x[f * ld + j0] : 0.0;
     const double c = fabs(v0) < INFINITY ? v0 : 0.0;
     const double s1 = tot[f], s2 = tot[NS + f];
     const double inv = n > 0.0 ? 1.0 / n : 0.0;
@@ -156,13 +188,26 @@ finish_kernel(const double* __restrict__ partial, int n_part, const double* __re
   }
 }
 
-// row: 74 doubles on the device; scratch: at least PARTIAL_STRIDE * grid doubles on the device
+size_t summary_scratch(int grid) { return (size_t)grid * PARTIAL_STRIDE + 1; }
+
+// row: 74 doubles on the device; scratch: summary_scratch(grid) doubles on the device, the per-CTA partials and then the
+// first survivor's index
 cudaError_t launch_summary(const LaunchCfg& cfg, const double* x, long long ld, long long N, const int* status, double* row,
                            double* scratch, int grid) {
+  unsigned long long* first = reinterpret_cast<unsigned long long*>(scratch + (size_t)grid * PARTIAL_STRIDE);
+  if (status && N > 0) {
+    const cudaError_t e = cudaMemsetAsync(first, 0xff, sizeof *first, cfg.stream);
+    if (e != cudaSuccess) return e;
+    first_alive_kernel<<<grid, THREADS, 0, cfg.stream>>>(status, N, first);
+    if (cfg.launch_counter) ++*cfg.launch_counter;
+  }
   // six states per CTA, two CTAs (512 threads, 116 registers, no spills) per SM: measured best of {2, 3, 6} groups x {2, 3, 4}
-  // CTAs per SM -- 0.265 ms = 4.8 TB/s at 2^23 aircraft; the three-CTA build spills its accumulators (0.298 ms)
-  partial_kernel<3, 2><<<dim3(grid, 3), THREADS, 0, cfg.stream>>>(x, ld, N, status, scratch);
-  finish_kernel<<<1, 1024, 0, cfg.stream>>>(scratch, grid, x, ld, N, status, row);
+  // CTAs per SM; the three-CTA build spills its accumulators.  tools/bench_entry_points.py --only summary on a B200 (1000 W),
+  // L2 flushed, best of 20, 2^20 / 2^23 aircraft: no status array 0.096 / 0.263 ms (4.8 TB/s at 2^23); status words, all
+  // alive 0.121 / 0.489 ms (0.117 / 0.484 ms with the search limited to the first 32 aircraft); only the last aircraft alive,
+  // the search reading every status word, 0.078 / 0.166 ms (0.074 / 0.172 ms).
+  partial_kernel<3, 2><<<dim3(grid, 3), THREADS, 0, cfg.stream>>>(x, ld, N, status, first, scratch);
+  finish_kernel<<<1, 1024, 0, cfg.stream>>>(scratch, grid, x, ld, N, status, first, row);
   if (cfg.launch_counter) *cfg.launch_counter += 2;
   return cudaGetLastError();
 }

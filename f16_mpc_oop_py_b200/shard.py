@@ -33,7 +33,9 @@ def summarise(x, status):
     out = np.zeros(2 + 4 * 18)
     out[0], out[1] = x.shape[1], alive.sum()
     if alive.any():
-        xa = x[:, alive]
+        # C order, so the sums along each state run over contiguous memory and numpy sums them pairwise: the F-ordered copy
+        # that x[:, alive] gives is summed one value after another, an error that grows with n (2300 ulp at 16 000 values)
+        xa = np.ascontiguousarray(x[:, alive])
         mean = xa.mean(axis=1)
         out[2:20], out[20:38], out[38:56] = xa.min(axis=1), xa.max(axis=1), mean
         out[56:74] = ((xa - mean[:, None]) ** 2).sum(axis=1)

@@ -213,8 +213,16 @@ int lqr_gain_batch(const double *x_soa, const double *u_soa, long long N, double
 /* ---- end-of-run statistics, reduced on the device (f16_stats.cu; SURVEY 8e: the row a rank contributes to the one
  * collective of a run; the reference's drivers keep the whole x_storage on the host instead, test_env.py:452-462) ----
  * Over the aircraft with status[n] == 0 (all of them if status == NULL):
- *   row [74] = { N, alive, min[18], max[18], mean[18], M2[18] },  M2 = sum (x - mean)^2  (two passes, no cancellation).
- * An empty selection gives min = +inf, max = -inf, mean = M2 = 0.  Bit-reproducible for a given device and N. */
+ *   row [74] = { N, alive, min[18], max[18], mean[18], M2[18] },  M2 = sum (x - mean)^2.
+ * One pass over the state: sums of x - c and (x - c)^2, with the shift c = the state of the first aircraft with status 0
+ * (aircraft 0 when status == NULL).  Counts, min and max are exact.  The mean is within 4 ulp + O(depth eps) mean |x - c| and
+ * M2 within O(depth eps) (M2 + alive (mean - c)^2) of the exact values, depth = the additions of the reduction tree (about
+ * 70 at 2^22 aircraft on 148 SMs): the closer the first survivor sits to the others, the closer M2 (tests/test_stats.py).
+ * Dead aircraft never reach the row, whatever their states hold (NaN, infinities, 1e300).  A survivor's NaN or infinity
+ * (status == NULL, or a caller's own mask) is counted as it is: min and max skip a NaN; that state's M2 is NaN, and its mean
+ * NaN when the state holds a NaN or both infinities, else that infinity.
+ * An empty selection gives min = +inf, max = -inf, mean = M2 = 0.  Bit-reproducible for a given device and N.  The host-buffer
+ * call over several contexts merges the rows of the slices by Chan's update (each slice takes its own shift). */
 int state_summary_batch(const double *x_soa /* [18][N] */, long long N, const int *status, double *row);
 /* A Monte-Carlo rollout that keeps statistics instead of trajectories (BASELINE cfg 5: 64 Mi aircraft -- x_storage of
  * test_env.py:452-462 would be 9 GB per snapshot): K steps as step_batch, and after every snap_every steps the summary row of

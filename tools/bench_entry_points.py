@@ -108,6 +108,15 @@ def main():
             row = np.empty(74)
             b, a = timed(lambda: ck(L.state_summary_batch_dev(d_x, n, n, None, row.ctypes.data), "summary"))
             report("state_summary_batch_dev (one pass + 592 B D2H)", b, a, nbytes=n * 152, units=n, unit_name="aircraft_per_s")
+            # with status words: every aircraft alive (the first-survivor search stops at once), and only the last one alive
+            # (the search reads every status word)
+            for name, last_only in (("all alive", False), ("one survivor, the last", True)):
+                st = np.zeros(n, dtype=np.int32)
+                if last_only:
+                    st[:-1] = 4
+                ck(L.f16_memcpy_h2d(d_st, st.ctypes.data, st.nbytes), "h2d")
+                b, a = timed(lambda: ck(L.state_summary_batch_dev(d_x, n, n, d_st, row.ctypes.data), "summary"))
+                report(f"state_summary_batch_dev, status: {name}", b, a, nbytes=n * 152, units=n, unit_name="aircraft_per_s")
         if (not only or "linearise" in only) and n <= (1 << 18):
             d_A, d_B = L.f16_dev_alloc(n * 324 * 8), L.f16_dev_alloc(n * 72 * 8)
             for scheme, nm, fl in ((0, "forward", 17200.0), (1, "central", 32300.0)):
