@@ -102,8 +102,7 @@ struct State {
   int math_mode = F16_MATH_STRICT;
   int clr_mode = F16_CLR_AS_BUILT;
   bool smem_tables = true;
-  int step_threads = 384;
-  int lin_variant = 0;
+  int lin_variant = 0;         // f16_set_linearise_variant: 0 = the default kernel of the math mode, 1 / 2 = reference order
   bool step_chunking = true;
   bool host_pipeline = true;   // chunked H2D / kernel / D2H overlap in the host-buffer entry points
   bool trim_fp_exit = true;    // trim_batch: fixed-point exit of the Nelder-Mead search (same results, see f16_model.cuh)
@@ -229,7 +228,6 @@ int init_locked(const char* table_path, int device, const int* devices, int ndev
   if (const char* v = getenv("F16_XCG")) G.default_xcg = atof(v);
   if (const char* v = getenv("F16_MATH")) G.math_mode = (!strcmp(v, "fast") || !strcmp(v, "1")) ? F16_MATH_FAST : F16_MATH_STRICT;
   if (const char* v = getenv("F16_CLR")) G.clr_mode = (!strcmp(v, "file") || !strcmp(v, "1")) ? F16_CLR_FROM_FILE : F16_CLR_AS_BUILT;
-  if (const char* v = getenv("F16_STEP_THREADS")) G.step_threads = atoi(v);
   if (const char* v = getenv("F16_TABLE_STAGING")) G.smem_tables = atoi(v) != 0;
   if (const char* v = getenv("F16_STEP_CHUNKING")) G.step_chunking = atoi(v) != 0;
   if (const char* v = getenv("F16_HOST_PIPELINE")) G.host_pipeline = atoi(v) != 0;
@@ -269,9 +267,7 @@ f16::LaunchCfg cfg(bool smem_tables) {
   f16::LaunchCfg c;
   c.stream = D->stream;
   c.sm_count = D->sm_count;
-  c.step_threads = G.step_threads;
   c.smem_tables = smem_tables;
-  c.lin_variant = G.lin_variant;
   c.launch_counter = &D->launches;
   c.step_chunking = G.step_chunking;
   c.step_progress = (int*)D->b_prog.p;
@@ -301,9 +297,9 @@ cudaError_t run_xdot(const f16::BatchSel& sel, const double* x, long long ld_x, 
   if (!u) return f16::strict::launch_nlplant(cfg(staged), tabs(), sel, x, ld_x, xdot, ld_out, N, status);
   return f16::strict::launch_calc_xdot(cfg(staged), tabs(), sel, x, ld_x, u, ld_u, xdot, ld_out, N, status);
 }
-// linearise_batch.  F16_MATH_STRICT: the staged reference-order kernels (variant 0 / 2: CTA per 32 aircraft, 1: warp per
-// aircraft).  F16_MATH_FAST, variant 0: the two-aircraft-per-warp kernel on the arithmetic of f16_fast.cuh
-// (f16_linearise_fast.cu); variants 1 and 2 keep the strict kernels in fast mode as well.
+// linearise_batch.  F16_MATH_STRICT: the staged reference-order kernel (CTA per 32 aircraft).  F16_MATH_FAST, variant 0: the
+// two-aircraft-per-warp kernel on the arithmetic of f16_fast.cuh (f16_linearise_fast.cu); variants 1 and 2 keep the
+// reference-order kernel in fast mode as well.
 cudaError_t run_linearise(const f16::BatchSel& sel, const double* x, long long ld_x, const double* u, long long ld_u, long long N,
                           double eps, int scheme, double* A, double* B, int* status) {
   if (fast_mode() && G.lin_variant == 0 && N < (1LL << 31)) {
@@ -777,13 +773,6 @@ int f16_set_table_staging(int mode) {
   std::lock_guard<std::mutex> lk(G_mu);
   int prev = G.smem_tables ? 1 : 0;
   G.smem_tables = mode != 0;
-  return prev;
-}
-
-int f16_set_step_threads(int threads) {
-  std::lock_guard<std::mutex> lk(G_mu);
-  int prev = G.step_threads;
-  G.step_threads = threads;
   return prev;
 }
 

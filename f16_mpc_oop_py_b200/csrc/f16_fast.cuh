@@ -223,10 +223,9 @@ F16_FD void locate_hifi(const double* img, double alpha, double beta, double el,
 }
 
 // value of table `slot` of an (f, d) node at alpha weight la
-// Two 8-byte loads, not one 16-byte load: on B200 a warp-wide LDS.128 occupies the shared-memory pipe for 2 cycles
-// (uniform address) to 4 cycles (>= 4 distinct addresses per quarter-warp), an LDS.64 for 0.57 to 1.0
-// (tools/microbench/mb_lds.cu), i.e. half the pipe time per byte.  ptxas re-fuses adjacent 8-byte loads whenever it
-// can prove 16-byte alignment, so the kernel derives `img` from a run-time offset (DevTables::zero) it cannot see through.
+// On B200 a warp-wide LDS.128 occupies the shared-memory pipe for 2 cycles (uniform address) to 4 cycles (>= 4 distinct
+// addresses per quarter-warp), an LDS.64 for 0.57 to 1.0 (tools/microbench/mb_lds.cu).  ptxas fuses the two 8-byte loads of
+// a node into one 16-byte load wherever it can prove 16-byte alignment; forcing two 8-byte loads measured slower (DESIGN.md).
 F16_FD double fd(const double* node, int slot, double la) { return fma(la, node[2 * slot + 1], node[2 * slot]); }
 F16_FD double mix(double lam, double lo, double hi) { return fma(lam, hi - lo, lo); }
 

@@ -13,8 +13,8 @@
 #include "f16_kernels_common.cuh"
 
 #define F16_THREADS 384  // derivative-only kernels: one CTA per SM, 12 warps, <= 168 registers per thread
-// step_kernel is instantiated for 256 / 384 / 512 threads per CTA (254 / 168 / 128 registers per thread, one CTA
-// per SM because of the 105 KB table image); LaunchCfg::step_threads picks one at run time.
+// step_kernel: 384 threads per CTA with the tables staged (168 registers per thread, one CTA per SM because of the 105 KB
+// table image), 256 with the tables read through L2.
 #define F16_LIN_WARPS 8    // linearise: 8 warps x 32 aircraft per CTA, <= 255 registers per thread (the staged evaluation holds 60 doubles of reusable stages)
 #define F16_LIN_TILE_LD 397  // doubles per aircraft in the output tile (396 + 1: conflict-free for both phases)
 
@@ -308,7 +308,7 @@ linearise_kernel(DevTables tabs, BatchSel sel, const double* __restrict__ x_g, l
       const double ang = k == 0 ? xu0[7] : k == 1 ? xu0[8] : k == 2 ? xu0[4] : k == 3 ? xu0[3] : xu0[5];
       double sn, cs;
 #if defined(__CUDA_ARCH__)
-      // the five angles decide together, exactly as trig_eval does, so that every variant of the kernel sees the same bits
+      // the five angles decide together, exactly as trig_eval does, so that the staged sines carry a full evaluation's bits
       const bool nb = trig_small(xu0[7]) & trig_small(xu0[8]) & trig_small(xu0[4]) & trig_small(xu0[3]) & trig_small(xu0[5]);
       if (nb) sincos_nb(ang, sn, cs);
       else
@@ -464,74 +464,10 @@ linearise_kernel(DevTables tabs, BatchSel sel, const double* __restrict__ x_g, l
 }
 
 // ------------------------------------------------------------------------------------------------------
-// linearise_batch, warp-per-aircraft variant: lane = perturbation column (0..17 states, 18..21 inputs, 22 = the
-// unperturbed point of the forward scheme), so one warp-wide evaluation of _calc_xdot yields every column of one
-// aircraft.  All lanes sit in the same table cell (shared-memory gathers broadcast), there is no shared output tile and
-// no CTA barrier; for a fixed row r the lanes write 18 (A) + 4 (B) consecutive doubles.  Forward differences take f(x)
-// from lane 22 by shuffle; central differences run the evaluation twice.
-// ------------------------------------------------------------------------------------------------------
-template <int FI>
-__global__ void __launch_bounds__(F16_THREADS, 1)
-linearise_warp_kernel(DevTables tabs, BatchSel sel, const double* __restrict__ x_g, long long ld_x,
-                      const double* __restrict__ u_g, long long ld_u, long long N, double eps, int scheme,
-                      double* __restrict__ A_g, double* __restrict__ B_g, int* __restrict__ status) {
-  const double* img = acquire_tables<FI, true>(tabs);
-  const int lane = threadIdx.x & 31;
-  const long long warps = ((long long)gridDim.x * blockDim.x) >> 5;
-  const int ncol = scheme == 0 ? 23 : 22;
-  const FdQuot fd(eps, scheme);
-  for (long long n = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5; n < N; n += warps) {
-    const int own = owns<FI>(sel, n);
-    if (own == 0) continue;
-    double v[18];
-    unsigned st = own < 0 ? ST_FIDELITY : 0u;
-    if (own == 1 && lane < ncol) {
-      const double xcg = sel.xcg ? sel.xcg[n] : sel.xcg_default;
-      const int passes = scheme == 0 ? 1 : 2;
-#pragma unroll 1
-      for (int pass = 0; pass < passes; pass++) {
-        const double d = pass ? -eps : eps;
-        double x[18], u[4], f[18];
-#pragma unroll
-        for (int i = 0; i < 18; i++) x[i] = x_g[i * ld_x + n] + (i == lane ? d : 0.0);
-#pragma unroll
-        for (int i = 0; i < 4; i++) u[i] = u_g[i * ld_u + n] + (i + 18 == lane ? d : 0.0);
-        st |= calc_xdot<FI>(img, x, u, xcg, f);
-#pragma unroll
-        for (int r = 0; r < 18; r++) v[r] = pass ? fd(v[r] - f[r]) : f[r];
-      }
-    }
-    if (scheme == 0) {  // env.py:330,339: (f(x + eps e_c) - f(x)) / eps; a failed f(x) voids every column
-      const unsigned st0 = __shfl_sync(0xffffffffu, st, 22);
-#pragma unroll
-      for (int r = 0; r < 18; r++) v[r] = fd(v[r] - __shfl_sync(0xffffffffu, v[r], 22));
-      st |= st0;
-    }
-    if (st) {
-#pragma unroll
-      for (int r = 0; r < 18; r++) v[r] = qnan();
-    }
-    if (lane < 18) {
-#pragma unroll
-      for (int r = 0; r < 18; r++) A_g[n * 324 + r * 18 + lane] = v[r];
-    } else if (lane < 22) {
-#pragma unroll
-      for (int r = 0; r < 18; r++) B_g[n * 72 + r * 4 + (lane - 18)] = v[r];
-    }
-    const unsigned all = __reduce_or_sync(0xffffffffu, lane < ncol ? st : 0u);
-    if (status && lane == 0) status[n] = (int)all;
-  }
-}
-
-// ------------------------------------------------------------------------------------------------------
 // trim_batch: env.py::trim (Nelder-Mead, ~2000 objective evaluations) for N flight conditions, one thread each.
 // The simplex lives in registers (f16_model.cuh::nelder_mead_trim); lanes differ only in how many iterations they need.
 // ------------------------------------------------------------------------------------------------------
 #define F16_TRIM_THREADS 256
-struct TrimGuess {
-  double ux[5];
-  int fixed_point_exit;
-};
 
 template <int FI, bool SMEM>
 __global__ void __launch_bounds__(F16_TRIM_THREADS, 1)
@@ -640,8 +576,6 @@ atmos_kernel(const double* __restrict__ alt, const double* __restrict__ vt, long
 // ------------------------------------------------------------------------------------------------------
 // launchers
 // ------------------------------------------------------------------------------------------------------
-static bool wants(const BatchSel& s, int FI) { return s.fi != nullptr || s.fi_default == FI || (FI == 1 && s.fi_default != 0); }
-
 template <int FI>
 static int table_smem(bool smem_tables) { return smem_tables ? Img<FI>::SMEM_BYTES : 0; }
 
@@ -681,16 +615,10 @@ cudaError_t launch_calc_xdot(const LaunchCfg& cfg, const DevTables& tabs, const 
 using StepKern = void (*)(DevTables, BatchSel, double*, long long, const double*, long long, long long, int, double, int*,
                           int*, const LqrLaw);
 
+// 384 threads with the tables staged, 256 with the tables read through L2 (the other CTA sizes measured slower: DESIGN.md)
 template <int FI, bool LQR>
-static StepKern pick_step(bool smem_tables, int& threads) {
-  if (!smem_tables) { threads = 256; return step_kernel<FI, false, LQR, 256>; }
-  if (threads <= 256) { threads = 256; return step_kernel<FI, true, LQR, 256>; }
-  if (threads <= 384) { threads = 384; return step_kernel<FI, true, LQR, 384>; }
-  if (threads <= 512) { threads = 512; return step_kernel<FI, true, LQR, 512>; }
-  if (threads <= 640) { threads = 640; return step_kernel<FI, true, LQR, 640>; }
-  if (threads <= 768) { threads = 768; return step_kernel<FI, true, LQR, 768>; }
-  threads = 1024;
-  return step_kernel<FI, true, LQR, 1024>;
+static StepKern step_kern(bool smem_tables) {
+  return smem_tables ? step_kernel<FI, true, LQR, 384> : step_kernel<FI, false, LQR, 256>;
 }
 
 cudaError_t launch_step(const LaunchCfg& cfg, const DevTables& tabs, const BatchSel& sel, double* x, long long ld_x,
@@ -698,11 +626,11 @@ cudaError_t launch_step(const LaunchCfg& cfg, const DevTables& tabs, const Batch
                         int* status, int* steps_done) {
   if (N <= 0) return cudaSuccess;
   cudaError_t e = cudaSuccess;
+  const int threads = cfg.smem_tables ? 384 : 256;
   for (int FI = 1; FI >= 0 && e == cudaSuccess; FI--) {
     if (!wants(sel, FI)) continue;
-    int threads = cfg.step_threads;
-    StepKern k = FI ? (lqr_host ? pick_step<1, true>(cfg.smem_tables, threads) : pick_step<1, false>(cfg.smem_tables, threads))
-                    : (lqr_host ? pick_step<0, true>(cfg.smem_tables, threads) : pick_step<0, false>(cfg.smem_tables, threads));
+    StepKern k = FI ? (lqr_host ? step_kern<1, true>(cfg.smem_tables) : step_kern<1, false>(cfg.smem_tables))
+                    : (lqr_host ? step_kern<0, true>(cfg.smem_tables) : step_kern<0, false>(cfg.smem_tables));
     const int smem = FI ? table_smem<1>(cfg.smem_tables) : table_smem<0>(cfg.smem_tables);
     e = launch_persistent(cfg, k, threads, smem, N, threads, tabs, sel, x, ld_x, u, ld_u, N, K, dt, status, steps_done,
                           lqr_host ? *lqr_host : LqrLaw());
@@ -715,15 +643,6 @@ cudaError_t launch_linearise(const LaunchCfg& cfg, const DevTables& tabs, const 
                              double* A, double* B, int* status) {
   if (N <= 0) return cudaSuccess;
   cudaError_t e = cudaSuccess;
-  if (cfg.lin_variant == 1) {  // warp per aircraft
-    if (wants(sel, 1))
-      e = launch_persistent(cfg, linearise_warp_kernel<1>, F16_THREADS, table_smem<1>(true), N, F16_THREADS / 32, tabs, sel, x,
-                            ld_x, u, ld_u, N, eps, scheme, A, B, status);
-    if (e == cudaSuccess && wants(sel, 0))
-      e = launch_persistent(cfg, linearise_warp_kernel<0>, F16_THREADS, table_smem<0>(true), N, F16_THREADS / 32, tabs, sel, x,
-                            ld_x, u, ld_u, N, eps, scheme, A, B, status);
-    return e;
-  }
   const long long groups = (N + 31) / 32;
   const int threads = F16_LIN_WARPS * 32;
   if (wants(sel, 1))

@@ -12,7 +12,10 @@ struct DevTables {
   const double* hifi;  // F16_IMG_HIFI_DOUBLES, 16-byte aligned
   const double* lofi;  // F16_IMG_LOFI_DOUBLES
   const double* hifi_fast;  // F16_FI_DOUBLES: the (f, d) image of f16_fast.cuh, used by the F16_MATH_FAST step kernel
-  int zero;                 // always 0: a run-time offset that hides the image's 16-byte alignment from ptxas
+  // Read by no kernel, but part of the parameter block of every kernel that takes DevTables: without it the later parameters
+  // move up by 8 bytes and ptxas allocates registers differently in the step kernels (166 <-> 168 / 252 <-> 254 registers),
+  // which has not been measured on the GPU.
+  int zero;
 };
 
 struct BatchSel {           // which aircraft run which model
@@ -25,9 +28,7 @@ struct BatchSel {           // which aircraft run which model
 struct LaunchCfg {
   cudaStream_t stream;
   int sm_count;
-  int step_threads;  // CTA size of step_kernel: 256, 384 or 512
   bool smem_tables;  // stage tables in shared memory with TMA bulk copies (default) or read them through L1/L2
-  int lin_variant;   // linearise kernel: 0 = CTA per 32 aircraft with staged columns, 1 = warp per aircraft
   unsigned long long* launch_counter;
   // time-chunked scheduling of the fast hifi step (f16_step_fast.cu): on/off, and the device scratch of one int per 32 aircraft
   bool step_chunking = false;

@@ -1,5 +1,5 @@
 // f16_kernels_common.cuh -- pieces shared by the kernel translation units (f16_kernels.cu, f16_step_fast.cu):
-// TMA table staging, per-aircraft model selection and the persistent-launch helper.
+// TMA table staging, per-aircraft model selection, the trim start point and the persistent-launch helper.
 #pragma once
 #include <stdint.h>
 
@@ -56,6 +56,15 @@ __device__ __forceinline__ int owns(const BatchSel& s, long long n) {
   if (FI == 1 && f != 0) return -1;
   return 0;
 }
+
+// does a batch hold aircraft of fidelity FI?  (per-aircraft flags: the launch for each fidelity picks its own)
+static bool wants(const BatchSel& s, int FI) { return s.fi != nullptr || s.fi_default == FI || (FI == 1 && s.fi_default != 0); }
+
+// start point of the trim search, and whether it may leave at a bitwise fixed point (trim kernels of both builds)
+struct TrimGuess {
+  double ux[5];
+  int fixed_point_exit;
+};
 
 __device__ __forceinline__ double qnan() { return __longlong_as_double(0x7ff8000000000000LL); }
 

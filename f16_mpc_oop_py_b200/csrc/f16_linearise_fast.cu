@@ -40,13 +40,7 @@ namespace fast {
 //   forward kernel at 384 threads / 168 registers (12 warps per SM; its 24 bytes of spills stay in L1): 1.11e9  <- forward
 //   forward kernel at 320 threads: 1.00e9 (uneven warps per scheduler)
 //   central kernel: 256 threads / 255 registers, no spills (the 55 KB stash of a 384-thread CTA leaves no L1)  <- central
-#ifndef F16_LF_THREADS_CENTRAL
-#define F16_LF_THREADS_CENTRAL 256
-#endif
-#ifndef F16_LF_THREADS_FORWARD
-#define F16_LF_THREADS_FORWARD 384
-#endif
-constexpr int LF_THREADS_CENTRAL = F16_LF_THREADS_CENTRAL, LF_THREADS_FORWARD = F16_LF_THREADS_FORWARD;
+constexpr int LF_THREADS_CENTRAL = 256, LF_THREADS_FORWARD = 384;
 constexpr int LF_IN_LD = 24;  // 18 states + 4 inputs (+ 2 pad) per staged aircraft
 
 template <int FI, int THREADS, bool CENTRAL>

@@ -3,7 +3,6 @@
 // result does not depend on which mul/add pairs ptxas would have chosen to contract in a given instantiation
 // (CTA size, table staging) -- all variants of the kernel, and the host emulation of the tests, agree bit for bit.
 #include <cuda.h>
-#include <stdlib.h>
 #include <string.h>
 
 #include "f16_kernels_common.cuh"
@@ -22,8 +21,6 @@ namespace fast {
 // ------------------------------------------------------------------------------------------------------
 constexpr int FAST_SMEM_BYTES = F16_FI_BYTES + 16;
 
-static bool sel_wants(const BatchSel& s, int FI) { return s.fi != nullptr || s.fi_default == FI || (FI == 1 && s.fi_default != 0); }
-
 template <bool SMEM, bool LQR, int THREADS, int COLMASK = 0>
 __global__ void __launch_bounds__(THREADS, 1)
 step_hifi_fast_kernel(DevTables tabs, BatchSel sel, double* __restrict__ x_g, long long ld_x,
@@ -34,9 +31,6 @@ step_hifi_fast_kernel(DevTables tabs, BatchSel sel, double* __restrict__ x_g, lo
     stage_tables_tma<F16_FI_BYTES>(f16_smem, img, reinterpret_cast<unsigned long long*>(f16_smem + F16_FI_BYTES));
     img = reinterpret_cast<const double*>(f16_smem);
   }
-#if defined(F16_FAST_LDS64)
-  img += tabs.zero;  // always 0; keeps the table gathers 8-byte loads (see fastmath::fd)
-#endif
   // The warps of a CTA leave the table staging together and run the same instruction stream: the three warps that share a
   // scheduler (warp, warp + 4, warp + 8) would sit in the FP64-dense and in the integer / gather parts of a step at the same
   // time.  Starting them a third of a microsecond apart keeps them out of phase: +2 % on a batch without a grid tail (2^20
@@ -116,9 +110,6 @@ step_hifi_fast_chunked_kernel(DevTables tabs, BatchSel sel, double* x_g, long lo
                               const __grid_constant__ ChunkPlan plan, const __grid_constant__ fastmath::LqrDense c_lqr_fast) {
   stage_tables_tma<F16_FI_BYTES>(f16_smem, tabs.hifi_fast, reinterpret_cast<unsigned long long*>(f16_smem + F16_FI_BYTES));
   const double* img = reinterpret_cast<const double*>(f16_smem);
-#if defined(F16_FAST_LDS64)
-  img += tabs.zero;
-#endif
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const long long G = (N + 31) >> 5;
   const int C = (K + chunk - 1) / chunk;
@@ -246,23 +237,15 @@ struct TrimCostFast {
   }
 };
 
-struct TrimGuessFast {
-  double ux[5];
-  int fixed_point_exit;
-};
-
 template <int FI>
 __global__ void __launch_bounds__(256, 1)
 trim_fast_kernel(DevTables tabs, BatchSel sel, const double* __restrict__ h_g, const double* __restrict__ v_g, long long N,
-                 double tol, int maxiter, TrimGuessFast guess, double* __restrict__ x_g, long long ld_x,
+                 double tol, int maxiter, TrimGuess guess, double* __restrict__ x_g, long long ld_x,
                  double* __restrict__ info_g, long long ld_info, int* __restrict__ status) {
   const double* img;
   if (FI) {
     stage_tables_tma<F16_FI_BYTES>(f16_smem, tabs.hifi_fast, reinterpret_cast<unsigned long long*>(f16_smem + F16_FI_BYTES));
     img = reinterpret_cast<const double*>(f16_smem);
-#if defined(F16_FAST_LDS64)
-    img += tabs.zero;
-#endif
   } else {
     double* li = reinterpret_cast<double*>(f16_smem);
     for (int i = threadIdx.x; i < F16_LOFI_STEP_IMG_DOUBLES; i += blockDim.x)
@@ -304,14 +287,14 @@ cudaError_t launch_trim(const LaunchCfg& cfg, const DevTables& tabs, const Batch
                         double tol, int maxiter, const double* ux0, double* x_trim, long long ld_x, double* info, long long ld_info,
                         int* status) {
   if (N <= 0) return cudaSuccess;
-  TrimGuessFast g;
+  TrimGuess g;
   for (int k = 0; k < 5; k++) g.ux[k] = ux0[k];
   g.fixed_point_exit = cfg.trim_fixed_point_exit ? 1 : 0;
   cudaError_t e = cudaSuccess;
-  if (sel_wants(sel, 1))
+  if (wants(sel, 1))
     e = launch_persistent(cfg, trim_fast_kernel<1>, 256, FAST_SMEM_BYTES, N, 256, tabs, sel, h, v, N, tol, maxiter, g, x_trim, ld_x,
                           info, ld_info, status);
-  if (e == cudaSuccess && sel_wants(sel, 0))
+  if (e == cudaSuccess && wants(sel, 0))
     e = launch_persistent(cfg, trim_fast_kernel<0>, 256, F16_LOFI_STEP_IMG_DOUBLES * 8, N, 256, tabs, sel, h, v, N, tol, maxiter, g,
                           x_trim, ld_x, info, ld_info, status);
   return e;
@@ -340,9 +323,7 @@ cudaError_t launch_trim(const LaunchCfg& cfg, const DevTables& tabs, const Batch
 // (a tensor map needs 16-byte strides) fall back to plain loads.
 // ------------------------------------------------------------------------------------------------------
 
-#ifndef XF_TABLE_CHUNK
-#define XF_TABLE_CHUNK 8192
-#endif
+constexpr int XF_TABLE_CHUNK = 8192;  // bytes per bulk copy of the hifi image
 template <int FI, bool NLP, int THREADS>
 struct XfSmem {
   static constexpr int XF_WARPS = THREADS / 32;
@@ -670,15 +651,10 @@ static cudaError_t launch_xdot_fast_one(const LaunchCfg& cfg, const DevTables& t
   bool tma = soa_tensor_map(&mx, x, ld_x, N, NLP ? 17 : 18);
   if (tma && !NLP) tma = soa_tensor_map(&mu, u, ld_u, N, 4);
   // CTA size: what keeps the main loop free of spills (measured at 2^20 aircraft, hifi): Nlplant 384 threads / 168 registers
-  // 61 us, calc_xdot (22 input values instead of 17) 256 threads / 255 registers 68 us against 76 us at 384.  F16_XF_THREADS
-  // overrides for experiments.
-  static const int forced = getenv("F16_XF_THREADS") ? atoi(getenv("F16_XF_THREADS")) : 0;
-  const int threads = forced ? forced : (NLP ? 384 : 256);
-  if (threads == 256)
-    return launch_persistent(cfg, xdot_fast_kernel<FI, NLP, 256>, 256, XfSmem<FI, NLP, 256>::TOTAL, N, 256, tabs, sel, mx, mu, x, ld_x, u,
-                             ld_u, xd, ld_out, N, status, tma ? 1 : 0, redo);
-  return launch_persistent(cfg, xdot_fast_kernel<FI, NLP, 384>, 384, XfSmem<FI, NLP, 384>::TOTAL, N, 384, tabs, sel, mx, mu, x, ld_x, u,
-                           ld_u, xd, ld_out, N, status, tma ? 1 : 0, redo);
+  // 61 us, calc_xdot (22 input values instead of 17) 256 threads / 255 registers 68 us against 76 us at 384
+  constexpr int T = NLP ? 384 : 256;
+  return launch_persistent(cfg, xdot_fast_kernel<FI, NLP, T>, T, XfSmem<FI, NLP, T>::TOTAL, N, T, tabs, sel, mx, mu, x, ld_x, u, ld_u, xd,
+                           ld_out, N, status, tma ? 1 : 0, redo);
 }
 
 // u == nullptr: Nlplant_batch (x is xu [17][N]); else calc_xdot_batch
@@ -687,10 +663,10 @@ cudaError_t launch_xdot_fast(const LaunchCfg& cfg, const DevTables& tabs, const 
                              const double* u, long long ld_u, double* xd, long long ld_out, long long N, int* status, unsigned* redo) {
   if (N <= 0) return cudaSuccess;
   cudaError_t e = cudaSuccess;
-  if (sel_wants(sel, 1))
+  if (wants(sel, 1))
     e = u ? launch_xdot_fast_one<1, false>(cfg, tabs, sel, x, ld_x, u, ld_u, xd, ld_out, N, status, redo)
           : launch_xdot_fast_one<1, true>(cfg, tabs, sel, x, ld_x, nullptr, 0, xd, ld_out, N, status, redo);
-  if (e == cudaSuccess && sel_wants(sel, 0))
+  if (e == cudaSuccess && wants(sel, 0))
     e = u ? launch_xdot_fast_one<0, false>(cfg, tabs, sel, x, ld_x, u, ld_u, xd, ld_out, N, status, redo)
           : launch_xdot_fast_one<0, true>(cfg, tabs, sel, x, ld_x, nullptr, 0, xd, ld_out, N, status, redo);
   return e;
@@ -737,8 +713,7 @@ template <int FI>
 static bool launch_step_tiled(const LaunchCfg& cfg, const DevTables& tabs, const BatchSel& sel, double* x, long long ld_x, const double* u,
                               long long ld_u, long long N, int K, double dt, const LqrLaw* lqr_host, const fastmath::LqrDense& dense,
                               int* status, int* steps_done, cudaError_t* err) {
-  static const bool off = getenv("F16_STEP_TILED") && atoi(getenv("F16_STEP_TILED")) == 0;
-  if (off || !cfg.smem_tables || K < 1 || K >= 8 || N < 4096) return false;
+  if (!cfg.smem_tables || K < 1 || K >= 8 || N < 4096) return false;
   CUtensorMap mx, mu;
   memset(&mx, 0, sizeof mx);
   memset(&mu, 0, sizeof mu);
@@ -754,17 +729,6 @@ static bool launch_step_tiled(const LaunchCfg& cfg, const DevTables& tabs, const
 using StepKern = void (*)(DevTables, BatchSel, double*, long long, const double*, long long, long long, int, double, int*,
                           int*, const fastmath::LqrDense);
 
-template <bool LQR>
-static StepKern pick_step_hifi_fast(bool smem_tables, int& threads) {
-  if (!smem_tables) { threads = 256; return step_hifi_fast_kernel<false, LQR, 256>; }
-  if (threads <= 256) { threads = 256; return step_hifi_fast_kernel<true, LQR, 256>; }
-  if (threads <= 384) { threads = 384; return step_hifi_fast_kernel<true, LQR, 384>; }
-  if (threads <= 512) { threads = 512; return step_hifi_fast_kernel<true, LQR, 512>; }
-  if (threads <= 640) { threads = 640; return step_hifi_fast_kernel<true, LQR, 640>; }
-  threads = 768;
-  return step_hifi_fast_kernel<true, LQR, 768>;
-}
-
 static cudaError_t launch_step_hifi_fast(const LaunchCfg& cfg, const DevTables& tabs, const BatchSel& sel, double* x, long long ld_x,
                                          const double* u, long long ld_u, long long N, int K, double dt, const LqrLaw* lqr_host,
                                          int* status, int* steps_done) {
@@ -774,15 +738,14 @@ static cudaError_t launch_step_hifi_fast(const LaunchCfg& cfg, const DevTables& 
   const bool mpc_cols = lqr_host && dense.colmask == F16_LQR_MPC_COLMASK && dense.row_mask == 0xE;  // the reference's own law: compile-time shape
   cudaError_t te = cudaSuccess;
   if (launch_step_tiled<1>(cfg, tabs, sel, x, ld_x, u, ld_u, N, K, dt, lqr_host, dense, status, steps_done, &te)) return te;
-  int threads = cfg.step_threads;
-  // time-chunked scheduling (no grid tail): the default CTA size, a uniform hifi batch, enough steps to cut into chunks and
+  // time-chunked scheduling (no grid tail): tables staged, a uniform hifi batch, enough steps to cut into chunks and
   // more than one round of warp-tasks; needs the status words (they carry "stopped" between chunks) and the progress flags
   // ... and a tail worth removing: with R = groups / (12 warps x SMs) rounds of warp-tasks the plain kernel idles
   // (ceil(R) - R) / ceil(R) of the launch (2.9 % at 2^20 aircraft, 0.3 % at 2^23, where the plain kernel is the faster one:
   // measured 2.68e10 against 2.60e10 aircraft-steps/s closed loop)
   const long long groups = (N + 31) / 32, slots = 12LL * cfg.sm_count, full = (groups + slots - 1) / slots;
   const bool tail = (full * slots - groups) * 100 > full * slots;  // more than 1 % idle
-  if (cfg.step_chunking && cfg.smem_tables && threads > 256 && threads <= 384 && sel.fi == nullptr && K >= 512 && status &&
+  if (cfg.step_chunking && cfg.smem_tables && sel.fi == nullptr && K >= 512 && status &&
       cfg.step_progress && groups <= cfg.step_progress_cap && groups > slots && tail) {
     const int chunk = (K + 15) / 16 < 64 ? 64 : (K + 15) / 16;
     cudaError_t e = cudaMemsetAsync(cfg.step_progress, 0, (size_t)groups * 4, cfg.stream);
@@ -803,10 +766,15 @@ static cudaError_t launch_step_hifi_fast(const LaunchCfg& cfg, const DevTables& 
     return launch_persistent(cfg, ck, 384, FAST_SMEM_BYTES, N, 384, tabs, sel, x, ld_x, u, ld_u, N, K, chunk, dt, status, steps_done,
                              cfg.step_progress, plan, dense);
   }
-  StepKern k = lqr_host ? pick_step_hifi_fast<true>(cfg.smem_tables, threads) : pick_step_hifi_fast<false>(cfg.smem_tables, threads);
-  if (mpc_cols && cfg.smem_tables && threads == 384) k = step_hifi_fast_kernel<true, true, 384, F16_LQR_MPC_SHAPE>;
-  const int smem = cfg.smem_tables ? FAST_SMEM_BYTES : 0;
-  return launch_persistent(cfg, k, threads, smem, N, threads, tabs, sel, x, ld_x, u, ld_u, N, K, dt, status, steps_done, dense);
+  // 384 threads with the tables staged, 256 with the tables read through L2 (the other CTA sizes measured slower: DESIGN.md)
+  if (!cfg.smem_tables) {
+    StepKern k = lqr_host ? step_hifi_fast_kernel<false, true, 256> : step_hifi_fast_kernel<false, false, 256>;
+    return launch_persistent(cfg, k, 256, 0, N, 256, tabs, sel, x, ld_x, u, ld_u, N, K, dt, status, steps_done, dense);
+  }
+  StepKern k = !lqr_host ? step_hifi_fast_kernel<true, false, 384>
+               : mpc_cols ? step_hifi_fast_kernel<true, true, 384, F16_LQR_MPC_SHAPE>
+                          : step_hifi_fast_kernel<true, true, 384>;
+  return launch_persistent(cfg, k, 384, FAST_SMEM_BYTES, N, 384, tabs, sel, x, ld_x, u, ld_u, N, K, dt, status, steps_done, dense);
 }
 
 static cudaError_t launch_step_lofi_fast(const LaunchCfg& cfg, const DevTables& tabs, const BatchSel& sel, double* x, long long ld_x,
@@ -827,8 +795,8 @@ static cudaError_t launch_step_lofi_fast(const LaunchCfg& cfg, const DevTables& 
 cudaError_t launch_step(const LaunchCfg& cfg, const DevTables& tabs, const BatchSel& sel, double* x, long long ld_x, const double* u,
                         long long ld_u, long long N, int K, double dt, const LqrLaw* lqr_host, int* status, int* steps_done) {
   cudaError_t e = cudaSuccess;
-  if (sel_wants(sel, 1)) e = launch_step_hifi_fast(cfg, tabs, sel, x, ld_x, u, ld_u, N, K, dt, lqr_host, status, steps_done);
-  if (e == cudaSuccess && sel_wants(sel, 0))
+  if (wants(sel, 1)) e = launch_step_hifi_fast(cfg, tabs, sel, x, ld_x, u, ld_u, N, K, dt, lqr_host, status, steps_done);
+  if (e == cudaSuccess && wants(sel, 0))
     e = launch_step_lofi_fast(cfg, tabs, sel, x, ld_x, u, ld_u, N, K, dt, lqr_host, status, steps_done);
   return e;
 }

@@ -55,7 +55,7 @@ extern "C" {
                            *  - Nlplant_batch / calc_xdot_batch from 4096 aircraft, with table staging on: f16_fast.cuh.
                            *    Smaller batches, or staging off: strict;
                            *  - linearise_batch: f16_fast.cuh (two aircraft per warp, csrc/f16_linearise_fast.cu), except under
-                           *    f16_set_linearise_variant(1) or (2), which keep the strict kernels;
+                           *    f16_set_linearise_variant(1) or (2), which keep the strict kernel;
                            *  - the legacy Nlplant and atmos symbols, atmos_batch, f16_hifi_probe, f16_lofi_probe: strict.
                            * f16_fast.cuh stays within the parity bars (<= 1e-12 scaled per derivative, <= 1e-9 after 10 s;
                            * tests/test_gpu_parity.py).  A Jacobian's quotient multiplies last-bit differences of f by 1/eps, so
@@ -135,7 +135,6 @@ int f16_set_clr_mode(int mode);       /* F16_CLR_*; rebuilds the device tables; 
 void f16_set_default_xcg(double xcg); /* for the legacy Nlplant symbol; default 0.25 or $F16_XCG */
 int f16_set_table_staging(int mode);  /* 1 (default): tables staged in shared memory by TMA bulk copy;
                                          0: read through L1/L2 with ld.global.nc (for A/B measurements) */
-int f16_set_step_threads(int threads); /* CTA size of the fused step kernel: 256, 384 (default), 512, 640, 768 or 1024 */
 int f16_set_step_chunking(int on);     /* 1 (default): long runs of the fast hifi step are scheduled in time chunks (work item = 32 aircraft x
                                           K/16 steps) so the persistent grid has no tail; 0: one warp-task = all K steps.  Same bits. */
 int f16_set_step_compaction(int on);    /* 1: a long uniform-fidelity run (K >= 4096 steps, >= 65536 aircraft) is cut into chunks of K / 8 steps
@@ -152,8 +151,8 @@ int f16_set_trim_fixed_point_exit(int on); /* 1 (default): trim_batch leaves a N
                                              maxiter like scipy, env.py:273); the cfg-4 grid at xcg 0.25 takes 36 ms instead of 537. */
 int f16_set_linearise_variant(int variant); /* linearise_batch kernel.  0 (default): in F16_MATH_STRICT the staged strict kernel (CTA per
                                                32 aircraft, columns over warps), in F16_MATH_FAST the two-aircraft-per-warp kernel on
-                                               the fast arithmetic; 1 = strict, warp per aircraft, column per lane; 2 = strict, CTA
-                                               per 32 aircraft, in either math mode.  1 and 2 give the same bits. */
+                                               the fast arithmetic; 1 or 2: the strict kernel in either math mode.  Returns the
+                                               previous value.  $F16_LIN_VARIANT. */
 /* sha256 (hex, 64 chars + NUL) of the canonical table payload in use */
 int f16_tables_sha256(char *out65);
 

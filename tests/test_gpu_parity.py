@@ -518,22 +518,19 @@ def test_step_restartable_and_device_api(f16):
     assert np.array_equal(out, b.x)
 
 
-def test_step_table_staging_variants_agree(f16, mode):
-    """tables staged in shared memory by TMA == tables read through L2; every CTA size gives the same bits
-    (in both math modes: the fast kernel has its own table image and CTA-size instantiations)"""
+def test_step_staged_tables_equal_l2_tables(f16, mode):
+    """tables staged in shared memory by TMA (384 threads per CTA) == tables read through L2 (256 threads per CTA), in both
+    math modes: the fast kernel has its own table image and instantiations"""
     g = load_golden("xcg35")
     x, u = perturbed_trim(20_000, g["x_trim"], seed=6)
     outs = []
-    for staging, threads in ((1, 256), (1, 384), (1, 512), (1, 640), (1, 768), (1, 1024), (0, 256)):
+    for staging in (1, 0):
         f16.lib.f16_set_table_staging(staging)
-        f16.lib.f16_set_step_threads(threads)
         fb = f16.F16Batch(x, u, xcg=0.35)
         fb.step(K=50)
         outs.append(fb.x.copy())
     f16.lib.f16_set_table_staging(1)
-    f16.lib.f16_set_step_threads(384)
-    for o in outs[1:]:
-        assert np.array_equal(o, outs[0])
+    assert np.array_equal(outs[1], outs[0])
 
 
 @pytest.mark.parametrize("with_law", [False, True])
@@ -735,39 +732,63 @@ def test_linearise_matches_env_py_golden(f16, mode, golden):
     assert C.shape == (10, 18) and D.shape == (10, 4) and C.sum() == 10
 
 
-@pytest.fixture(params=[0, 1], ids=["cta32", "warp"])
-def lin_variant(request, f16):
-    """both linearise kernels: CTA per 32 aircraft with shared stages, and warp per aircraft"""
-    prev = f16.lib.f16_set_linearise_variant(request.param)
+@pytest.fixture(params=[(0, 0), (1, 1)], ids=["strict", "fast_variant1"])
+def reference_order_linearise(request, f16):
+    """the reference-order Jacobian kernel, reached by default in F16_MATH_STRICT and through f16_set_linearise_variant(1)
+    in F16_MATH_FAST"""
+    math_mode, variant = request.param
+    prev_mode = f16.lib.f16_set_math_mode(f16.MATH_FAST if math_mode else f16.MATH_STRICT)
+    prev = f16.lib.f16_set_linearise_variant(variant)
     yield request.param
     f16.lib.f16_set_linearise_variant(prev)
+    f16.lib.f16_set_math_mode(prev_mode)
 
 
-def test_linearise_variants_bit_equal(f16):
-    """the staged evaluation (stages shared between columns) and the plain one give the same bits"""
+def test_linearise_strict_equals_host_finite_differences(f16):
+    """The strict linearise_batch (stages of f shared between the columns, calc_xdot_col) gives the bits of finite
+    differences formed on the host from full strict calc_xdot_batch evaluations: the perturbed points built as the kernel
+    builds them (x0 + where(i == c, +-eps, 0.0); the forward base point x0 + 0.0, which turns -0.0 into +0.0), IEEE
+    quotients, a column NaN wherever one of its evaluations (forward: or the base point's) failed, and the status word the
+    OR over every evaluation."""
     g = load_golden("xcg25")
     x, u = perturbed_trim(1000 + 7, g["x_trim"], seed=5, frac=0.04)
-    x[13, 5] = 25.0 - 1e-6
-    fi = np.ones(x.shape[1], dtype=np.uint8)
+    x[13, 5] = 25.0 - 1e-6      # elevator + eps leaves the hifi tables: column 13 of aircraft 5 is NaN
+    n = x.shape[1]
+    fi = np.ones(n, dtype=np.uint8)
     fi[::3] = 0
-    out = {}
-    for variant in (0, 1):
-        prev = f16.lib.f16_set_linearise_variant(variant)
+    eps = 1e-5
+    xu0 = np.vstack([x, u])     # columns 0..17 states, 18..21 inputs
+    idx = np.arange(22)[:, None]
+    prev = f16.lib.f16_set_math_mode(f16.MATH_STRICT)
+    try:
         for scheme in ("forward", "central"):
+            signs = (1.0,) if scheme == "forward" else (1.0, -1.0)
+            pts = [xu0 + np.where(idx == c, s * eps, 0.0) for s in signs for c in range(22)]
+            if scheme == "forward":
+                pts.append(xu0 + 0.0)
+            xu = np.ascontiguousarray(np.hstack(pts))
+            m = len(pts)
+            ev = f16.F16Batch(xu[:18], xu[18:], fi_flag=np.tile(fi, m), xcg=0.25)
+            f = ev._calc_xdot(xu[:18], xu[18:]).reshape(18, m, n)
+            st = ev.last_status.reshape(m, n)
+            # forward: f(x0 + eps e_c) - f(x0 + 0.0); central: f(x0 + eps e_c) - f(x0 - eps e_c)
+            num = f[:, :22] - f[:, 22:]
+            bad = (st[:22] != 0) | (st[22:] != 0)
+            q = np.where(bad[None], np.nan, num / (eps if scheme == "forward" else 2 * eps))   # [row][column][aircraft]
+            status = np.bitwise_or.reduce(st, axis=0)
             fb = f16.F16Batch(x, u, fi_flag=fi, xcg=0.25)
-            A, B, _, _ = fb.linearise(x, u, scheme=scheme)
-            out[variant, scheme] = (A, B, fb.last_status.copy())
-        f16.lib.f16_set_linearise_variant(prev)
-    for scheme in ("forward", "central"):
-        for other in (1,):
-            a, b = out[0, scheme], out[other, scheme]
-            assert np.array_equal(a[2], b[2])
-            assert np.array_equal(a[0], b[0], equal_nan=True) and np.array_equal(a[1], b[1], equal_nan=True)
+            A, B, _, _ = fb.linearise(x, u, scheme=scheme, eps=eps)
+            assert np.array_equal(fb.last_status, status), scheme
+            assert np.array_equal(A, q[:, :18].transpose(2, 0, 1), equal_nan=True), scheme
+            assert np.array_equal(B, q[:, 18:].transpose(2, 0, 1), equal_nan=True), scheme
+            assert np.isnan(A[5, :, 13]).all() and fb.last_status[5] != 0
+    finally:
+        f16.lib.f16_set_math_mode(prev)
 
 
 @pytest.mark.parametrize("scheme", ["forward", "central"])
 @pytest.mark.parametrize("fi", [1, 0])
-def test_linearise_batch_grid(f16, oracle, scheme, fi, lin_variant):
+def test_linearise_batch_grid(f16, oracle, scheme, fi, reference_order_linearise):
     """a 16 x 16 altitude x velocity grid about perturbed trims (cfg 4 is 64 x 64; same code path)"""
     g = load_golden("xcg25")
     n = 256 + 13     # ragged last CTA
@@ -862,7 +883,7 @@ def test_linearise_fast_kernel_edge_semantics_equal_the_strict_kernel(f16):
     assert out[f16.MATH_FAST, "forward", n][2][1] == 1 << 20 and out[f16.MATH_FAST, "forward", n][2][10] == 1 << 22
 
 
-def test_linearise_out_of_envelope_column_is_nan(f16, lin_variant):
+def test_linearise_out_of_envelope_column_is_nan(f16, reference_order_linearise):
     g = load_golden("xcg25")
     x = np.repeat(g["x_trim"][:, None], 3, axis=1)
     u = np.repeat(g["u_trim"][:, None], 3, axis=1)
